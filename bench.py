@@ -8,6 +8,7 @@ tile statistics, greedy assignment and whole-tensor scoring, per tensor.  With N
 its own layer of the tensor list (weak scaling, no data-path collective; result rows are gathered to rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg1|cfg2|cfg3|cfg4|cfg5|cfg2-fp8]
+                    [--dump-outputs DIR]
 
 --config selects another of BASELINE.json's configs (same JSON contract; `config.workload` names it):
   cfg1  `none`, formats bf16/bfp8/bfp4/bfp2/fp0 on [1536,7168] (8 rotating buffers > L2), reconstructions + reference scores
@@ -303,6 +304,71 @@ def maps_vs_reference_goldens(items, *result_sets):
     return ok
 
 
+DUMP_SAMPLE = 1 << 21        # cfg1: reconstruction elements kept per format (3 x 8 MB)
+DUMP_MAP_COLUMNS = 8192      # cfg3: tiles kept of each tensor's 32 threshold maps (8 x 1 MB)
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write DIR/<name>.npy for every array (float32 or float64; at most 44 MB in all, cfg5's maps)."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(d / f"{name}.npy", a)
+
+
+def fixed_sample(n: int, k: int):
+    """Sorted indices of a seeded sample of k of n positions (all of them when n <= k): the same for every run."""
+    import numpy as np
+    return np.arange(n) if n <= k else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def other_outputs(cfg: str, names, K: int, out) -> dict:
+    """What the last timed step of cfg1 / cfg3 / cfg4 computed.
+    cfg1: the bfp8 / bfp4 / bfp2 reconstructions of the step's buffer (bf16 is the input itself, fp0 is zero), a fixed sample
+          of DUMP_SAMPLE elements each (float32).
+    cfg3: per tensor, one row per threshold [threshold, counts bf16/bfp8/bfp4/bfp2, total bytes, pcc, mae, atol] (float64)
+          and the threshold maps at a fixed sample of at most DUMP_MAP_COLUMNS tiles (float32 [32, columns]).
+    cfg4: per tensor, the selected map (float32), its counts and [pcc, mae, atol], and [pcc, mae, atol] of every sample
+          (float64 [1000, 3])."""
+    import numpy as np
+    from quantization_analysis_b200.batch import MIXED
+    res = {}
+    if cfg == "cfg1":
+        j = (K - 1) % 8
+        for fmt, y in zip(("bfp8", "bfp4", "bfp2"), out):
+            y = y.float().cpu().numpy()
+            res[f"buffer{j}.{fmt}.sample"] = y[fixed_sample(y.size, DUMP_SAMPLE)]
+        return res
+    for name, r in zip(names, out):
+        if cfg == "cfg3":
+            rows, maps = r
+            res[f"{name}.rows"] = np.array([[row["threshold"]] + [row["counts"][f] for f in MIXED]
+                                            + [row["total_bytes"], row["pcc"], row["mae"], row["atol"]] for row in rows], dtype=np.float64)
+            maps = maps.cpu().numpy()
+            res[f"{name}.maps_sample"] = maps[:, fixed_sample(maps.shape[1], DUMP_MAP_COLUMNS)].astype(np.float32)
+        else:
+            res[f"{name}.assignment"] = r.assignment.cpu().numpy().astype(np.float32)
+            res[f"{name}.counts"] = np.array([r.counts[f] for f in MIXED], dtype=np.float64)
+            res[f"{name}.metrics"] = np.array([r.metrics_exact[k] for k in ("pcc", "mae", "atol")], dtype=np.float64)
+            res[f"{name}.samples"] = np.array([[s_["pcc"], s_["mae"], s_["atol"]] for s_ in r.meta["samples"]], dtype=np.float64)
+    return res
+
+
+def greedy_outputs(items, results) -> dict:
+    """What a GreedyBatch caller receives for each tensor: the tile map (float32), the tile counts in bf16/bfp8/bfp4/bfp2
+    order and [pcc, mae, atol] (float64)."""
+    import numpy as np
+    from quantization_analysis_b200.batch import MIXED
+    out = {}
+    for (name, _shape, _seed), r in zip(items, results):
+        out[f"{name}.assignment"] = r["assignment"].astype(np.float32)
+        out[f"{name}.counts"] = np.array([r["counts"][f] for f in MIXED], dtype=np.float64)
+        out[f"{name}.metrics"] = np.array([r["metrics"][k] for k in ("pcc", "mae", "atol")], dtype=np.float64)
+    return out
+
+
 def pin_rank_to_cores(local: int, world: int) -> list[int] | None:
     """Give every rank of the node its own slice of the host cores before any pinned buffer is allocated: the launch
     threads and the pinned pages of one rank then do not migrate under the others (round 1: e2e fell to 0.42 efficiency
@@ -470,6 +536,8 @@ def bench_greedy(args, e) -> None:
     clk = ClockSampler(e.local, enabled=(rank == 0))
     clk.__enter__()
     ms_local = timed(batches, K, inflight)
+    if args.dump_outputs:                                        # step k of the timed loop ran on list k % inflight
+        dump_outputs(args.dump_outputs, greedy_outputs(items, batches[(K - 1) % inflight].collect()))
     ms = e.reduce_max(ms_local)
     per_rank_ms = e.gather_floats(ms_local / K)
     value = total_bytes * K / (ms * 1e-3) / 1e9
@@ -740,6 +808,8 @@ def bench_fp8(args, e) -> None:
     clk = ClockSampler(e.local, enabled=(rank == 0))
     clk.__enter__()
     ms = e.reduce_max(timed(K, inflight))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, greedy_outputs(items, batches[(K - 1) % inflight].collect()))
     ms_single = e.reduce_max(timed(K, 1)) / K
     eq_bytes, in_bytes = batch.total_bytes(), batch.input_bytes()
     value = eq_bytes * world * K / (ms * 1e-3) / 1e9
@@ -868,13 +938,13 @@ def bench_other(args, e) -> None:
         scoring = os.environ.get("QA_BENCH_SCORING", "reference")      # "exact": float64 table recombination instead of the
         if cfg == "cfg3":                                               # reference's float32 whole-tensor arithmetic
             def step(k):
-                return [sweep.sweep_tensor(x, engine.MIXED_FORMATS, "pcc", steps=32, lowest=0.9, scoring=scoring)[0][-1]["counts"] for x in xs]
+                return [sweep.sweep_tensor(x, engine.MIXED_FORMATS, "pcc", steps=32, lowest=0.9, scoring=scoring) for x in xs]
         else:
             algo = ca.create_algorithm("mixed-tile-random", {"metric": "pcc", "threshold": 0.99, "iters": 1000, "seed": 42,
                                                               "sample_scoring": scoring})
 
             def step(k):
-                return [algo.run_prepared(engine.prepare_tiles(x), list(engine.MIXED_FORMATS)).counts for x in xs]
+                return [algo.run_prepared(engine.prepare_tiles(x), list(engine.MIXED_FORMATS)) for x in xs]
     for k in range(W):
         step(k)
     e.barrier()
@@ -889,6 +959,10 @@ def bench_other(args, e) -> None:
     clk.__exit__()
     ms = e.reduce_max(a.elapsed_time(b))
     value = e.world * 2.0 * per_step_elems * K / (ms * 1e-3) / 1e9
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, other_outputs(cfg, names, K, out))
+    if cfg != "cfg1":
+        out = [r[0][-1]["counts"] for r in out] if cfg == "cfg3" else [r.counts for r in out]
     # cfg1 end to end through the plug-in: numpy float32 in, five float32 reconstructions out + reference scores
     e2e = {"value": None, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     if cfg == "cfg1":
@@ -931,7 +1005,11 @@ def main() -> None:
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="cfg2", choices=sorted(METRICS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<tensor>.<array>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl b200")
     if args.impl == "reference":
         run_reference_arm(args)
         return

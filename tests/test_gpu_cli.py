@@ -52,6 +52,43 @@ def test_sweep_range_errors_like_reference(workdir):
     assert sweep_cli.main(base + ["--metric", "mae", "--lowest-metric-val", "0.0"]) == 1
 
 
+_DROPIN_GOLDENS = r'''
+import sys
+import numpy as np
+sys.path.insert(0, sys.argv[1])
+import quantization_analysis_b200 as q
+q.install_drop_in()
+from compression_algorithms import create_algorithm          # the names the reference's programs import
+from compression_algorithms.metrics import pearson_corr
+from compression_algorithms.quantizer import Quantizer
+import quantization_formats
+from tests import golden_util as G
+assert "quantization_analysis_b200" in quantization_formats.__file__
+quantizer = Quantizer(backend="emulation")
+for name in G.algo_case_names():
+    x = G.algo_input(name)
+    for key, m, want_a, want_y in G.algo_runs(name):
+        res = create_algorithm(m["algo"], dict(m["params"])).run(xf=x, formats=G.FORMATS, quantizer=quantizer, cache=None)[0]
+        d = np.abs(x - res.y)
+        assert np.array_equal(np.asarray(res.meta["assignment"], dtype=np.int8), want_a), key
+        assert np.array_equal(G.bits(res.y), want_y.reshape(-1)), key
+        assert res.tile_counts == m["counts"] and res.tile_bytes == m["tile_bytes"], key
+        assert pearson_corr(x, res.y) == m["pcc_f32"] and float(np.mean(d)) == m["mae_f32"] and float(np.max(d)) == m["atol_f32"], key
+print("drop_in_ok")
+'''
+
+
+def test_drop_in_modules_reproduce_reference_goldens():
+    """install_drop_in() in a fresh interpreter: the reference's module names (compression_algorithms.*, quantization_formats)
+    resolve to this package, and every recorded reference run (tests/golden/algo_small.*), called the way the reference's
+    programs call it, gives the reference's maps, reconstructions, counts, bytes and float32 scores."""
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, "-c", _DROPIN_GOLDENS, str(U.ROOT)], capture_output=True, text=True, timeout=600, cwd=str(U.ROOT))
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
+    assert "drop_in_ok" in out.stdout
+
+
 def test_unmodified_reference_programs_over_drop_in(workdir):
     """The reference's own `wq` and sweep script, unmodified, import this package through install_drop_in() and must
     write the same trees as when they ran on the reference's NumPy modules."""
