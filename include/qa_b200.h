@@ -204,18 +204,22 @@ int qa_numpy_permutation_par(qa_pcg64* rng, int64_t n, int32_t* out_perm, void* 
                              qa_stream_t stream);
 /* Staging of a greedy run, so that its three independent parts can overlap on different streams:
  *
- *  qa_greedy_prefetch  - the permutations that depend only on (seed, tile count): #1 for the base format (only its
- *      stream position matters), #2 for the first candidate format, and - speculatively - #3 for the second one,
- *      which is the permutation of all n tiles whenever pass 2 accepted every tile (mixed_tile_greedy.py:228-231).
- *      pre_order int32[(nfmt >= 3 ? 2 : 1)][n] = visiting orders of passes 2 (and 3); pre_rng[same count] = stream
- *      states after them.  The greedy checks the candidate count before it uses #3 and draws its own otherwise.
- *      `work` (qa_greedy_par_work_bytes) may be the greedy's own buffer if the prefetch completes before it starts.
- *  qa_greedy_init      - the data-dependent, permutation-independent part: the sequentially rounded initial sums
- *      (mixed_tile_greedy.py:165-170) and the per-tile deltas of every format transition.  init: at least
- *      qa_greedy_init_bytes(ntiles) bytes; fmt_order / metric must match the greedy call that consumes it.
- *  qa_greedy_assign_par_pre - the accept/reject chain; pre_order / pre_rng and init may each be NULL (computed
- *      inline).  Same results as qa_greedy_assign_par in every combination. */
-/* The two halves of one numpy permutation, for callers that pipeline them across streams (a resolve needs the
+ *  permutations - the ones that depend only on (seed, tile count) (mixed_tile_greedy.py:228-231): #1 for the base format
+ *      (only its stream position matters), #2 for the first candidate format, and - speculatively - #3 for the second
+ *      one, which is the permutation of all n tiles whenever pass 2 accepted every tile.  qa_perm_resolve_chain draws #1
+ *      and #2, qa_perm_resolve #3, and qa_perm_apply turns the swap targets of #2 and #3 into visiting orders.  The chain
+ *      takes them as pre_order int32[(nfmt >= 3 ? 2 : 1)][n] (orders of passes 2 and 3) and pre_rng[same count] (stream
+ *      states after #2 and #3); it checks the candidate count before it uses #3 and draws its own otherwise.
+ *  init - the data-dependent, permutation-independent part: the sequentially rounded initial sums
+ *      (mixed_tile_greedy.py:165-170, qa_greedy_init_sums_range) and the per-tile deltas of every format transition
+ *      (qa_greedy_init_deltas).  init: at least qa_greedy_init_bytes(ntiles) bytes; fmt_order / metric must match the
+ *      greedy call that consumes it.
+ *  chain - qa_greedy_assign_passes; pre_order / pre_rng and init may each be NULL.  pre_order == NULL: the chain draws
+ *      every permutation itself.  init == NULL: the call that runs pass 0 computes it into `work` (the delta records and
+ *      the initial sums, ahead of the chain on the same stream).  Same results as qa_greedy_assign_par in every
+ *      combination.
+ *
+ * The two halves of one numpy permutation, for callers that pipeline them across streams (a resolve needs the
  * stream state of the previous one; an apply only needs its own swap targets):
  *  qa_perm_resolve - swap targets jarr int32[n] (entries 1..n-1; NULL = only advance the stream) and the stream state
  *      after the permutation (rng_out may alias rng_in).  One cluster.
@@ -229,25 +233,20 @@ int qa_perm_resolve_chain(const qa_pcg64* rng_in, int64_t n, int count, uint32_t
 int64_t qa_perm_apply_work_bytes(int64_t n);
 int qa_perm_apply(const int32_t* jarr, int64_t n, const int32_t* cand, int32_t* out, void* work,
                   qa_stream_t stream);
-int qa_greedy_prefetch(const qa_pcg64* rng, int64_t n, int nfmt, int32_t* pre_order, qa_pcg64* pre_rng,
-                       void* work, qa_stream_t stream);
 int64_t qa_greedy_init_bytes(int64_t ntiles);
-int qa_greedy_init(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt,
-                   void* init, qa_stream_t stream);
-/* The two halves of qa_greedy_init for callers that run them on different streams: the sums (one cluster, latency
- * bound) and the delta records (a plain grid kernel) write disjoint parts of `init`; the greedy needs both. */
-int qa_greedy_init_sums(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt,
-                        void* init, qa_stream_t stream);
-/* qa_greedy_init_sums over tiles [tile_begin, tile_end) in order: calls must cover [0, ntiles) consecutively on the same
- * `init`; only the call that reaches ntiles needs the whole table (the earlier ones read tiles < tile_end). */
+/* The two halves of `init`, for callers that run them on different streams: the sums (one cluster, latency bound) and
+ * the delta records (a plain grid kernel) write disjoint parts of it; the greedy needs both.  The sums go over tiles
+ * [tile_begin, tile_end) in order: calls must cover [0, ntiles) consecutively on the same `init`; only the call that
+ * reaches ntiles needs the whole table (the earlier ones read tiles < tile_end). */
 int qa_greedy_init_sums_range(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order,
                               int nfmt, void* init, int64_t tile_begin, int64_t tile_end,
                               qa_stream_t stream);
 int qa_greedy_init_deltas(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt,
                           void* init, qa_stream_t stream);
-/* qa_greedy_assign_par_pre restricted to passes [pass_begin, pass_end) of the format order (pass 0 = base format).
- * Consecutive calls covering [0, nfmt) on the same buffers give the results of the single call; the running state
- * travels in `work`.  Lets a caller start the early passes before the speculative third permutation is ready. */
+/* The accept/reject chain over passes [pass_begin, pass_end) of the format order (pass 0 = base format); pre_order /
+ * pre_rng and init as above.  Consecutive calls covering [0, nfmt) on the same buffers give the results of the single
+ * call; the running state travels in `work`.  Lets a caller start the early passes before the speculative third
+ * permutation is ready. */
 int qa_greedy_assign_passes(const double* table, int64_t ntiles, double numel, int metric,
                             double threshold, const int32_t* fmt_order, int nfmt, qa_pcg64* rng,
                             int8_t* assignment, int64_t* counts, double* state, void* work,
@@ -258,11 +257,6 @@ int qa_greedy_assign_passes(const double* table, int64_t ntiles, double numel, i
  * irrelevant, and with this flag its permutation is not drawn at all (*rng is then unspecified).  Maps, counts and
  * sums are unaffected. */
 #define QA_GREEDY_SKIP_FINAL_STREAM 1
-int qa_greedy_assign_par_pre(const double* table, int64_t ntiles, double numel, int metric,
-                             double threshold, const int32_t* fmt_order, int nfmt, qa_pcg64* rng,
-                             int8_t* assignment, int64_t* counts, double* state, void* work,
-                             const int32_t* pre_order, const qa_pcg64* pre_rng, const void* init,
-                             qa_stream_t stream);
 
 /* Upper bound on the thread-block cluster size of the greedy kernels (1, 2, 4, 8, 16; 0 = automatic: large tensors get
  * 16 CTAs for latency).  A caller with many tensors in flight trades per-tensor latency for SM time with a smaller

@@ -39,8 +39,8 @@ def main():
         s = st.cpu().numpy(); s2 = st2.cpu().numpy()
         mhz = 1e-3
         print(f"{name} {shape} ntiles={nt} cluster={int(s[12])} counts={c.tolist()}")
-        print(f"  prefetch kernel {t_pre*1e3:.0f} us | init kernel {t_init*1e3:.0f} us | chain (staged) {t_g*1e3:.0f} us | all inline {t_i*1e3:.0f} us (incl. rng/alloc launches)")
-        for tag, v in (("staged", s), ("inline", s2)):
+        print(f"  prefetch {t_pre*1e3:.0f} us | init kernel {t_init*1e3:.0f} us | chain (staged) {t_g*1e3:.0f} us | single call {t_i*1e3:.0f} us (incl. rng/alloc launches)")
+        for tag, v in (("staged", s), ("single", s2)):
             print(f"  [{tag}] kcycles: init {v[8]*mhz:.0f} (pos-sums {v[13]*mhz:.0f}, signed {v[14]*mhz:.0f}, rounds {int(v[15])}) "
                   f"perm {v[9]*mhz:.0f} (resolve {v[21]*mhz:.0f}, apply {v[22]*mhz:.0f}, sweeps {int(v[23]) % 65536}, rounds {int(v[23]) // 65536}) "
                   f"chain {v[10]*mhz:.0f} (gather {v[18]*mhz:.0f}, commit {v[17]*mhz:.0f}, kernel total {v[16]*mhz:.0f}, chunks {int(v[19])}, min margin {v[20]:.2e}, "

@@ -26,7 +26,9 @@ def stats(st):
 
 
 def init(st):
-    check(L.qa_greedy_init(s["table"].data_ptr(), n, METRIC_CODE["pcc"], b._order, 4, s["init"].data_ptr(), st.cuda_stream), "init")
+    iargs = (s["table"].data_ptr(), n, METRIC_CODE["pcc"], b._order, 4, s["init"].data_ptr())
+    check(L.qa_greedy_init_deltas(*iargs, st.cuda_stream), "init deltas")
+    check(L.qa_greedy_init_sums_range(*iargs, 0, n, st.cuda_stream), "init sums")
 
 
 def resolves(st, k):
@@ -39,11 +41,7 @@ def apply(st, i):
 
 
 def chain(st):
-    s["rng"].copy_(b._rng0, non_blocking=True)
-    check(L.qa_greedy_assign_par_pre(s["table"].data_ptr(), n, float(s["numel"]), METRIC_CODE["pcc"], 0.999, b._order, 4,
-                                     s["rng"].data_ptr(), s["assignment"].data_ptr(), s["counts"].data_ptr(), s["state"].data_ptr(),
-                                     s["work"].data_ptr(), s["pre_order"].data_ptr(), s["rngs"][1].data_ptr(), s["init"].data_ptr(),
-                                     st.cuda_stream), "chain")
+    chain_passes(st, 0, 4)
 
 
 def chain_passes(st, b0, e0):

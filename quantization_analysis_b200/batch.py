@@ -50,14 +50,11 @@ def cached_permutations(device, seed: int, ntiles: int, nfmt: int):
     jarr = torch.empty((3, ntiles), dtype=torch.int32, device=dev)
     pre_order = torch.empty((2, ntiles), dtype=torch.int32, device=dev)
     rngs = torch.stack([rng0, rng0, rng0]).contiguous()
-    awork = torch.empty(L.qa_perm_apply_work_bytes(ntiles), dtype=torch.uint8, device=dev)
-    sp = torch.cuda.current_stream(dev).cuda_stream
-    check(L.qa_perm_resolve_chain(rng0.data_ptr(), ntiles, 2, 0b10, jarr.data_ptr(), rngs.data_ptr(), sp), "qa_perm_resolve_chain")
-    check(L.qa_perm_apply(jarr[1].data_ptr(), ntiles, None, pre_order[0].data_ptr(), awork.data_ptr(), sp), "qa_perm_apply")
-    if nfmt >= 3:
-        check(L.qa_perm_resolve(rngs[1].data_ptr(), ntiles, jarr[2].data_ptr(), rngs[2].data_ptr(), sp), "qa_perm_resolve")
-        check(L.qa_perm_apply(jarr[2].data_ptr(), ntiles, None, pre_order[1].data_ptr(), awork.data_ptr(), sp), "qa_perm_apply")
-    torch.cuda.current_stream(dev).synchronize()
+    awork = torch.empty((2, L.qa_perm_apply_work_bytes(ntiles)), dtype=torch.uint8, device=dev)
+    cur = torch.cuda.current_stream(dev)
+    engine.enqueue_perm_prefetch(rng0, ntiles, nfmt >= 3, (jarr, pre_order, rngs, awork), cur, cur,
+                                 [torch.cuda.Event() for _ in range(3)])
+    cur.synchronize()
     _PERM_CACHE[key] = {"pre_order": pre_order, "rngs": rngs}
     return _PERM_CACHE[key]
 
@@ -260,9 +257,8 @@ class GreedyBatch:
             # streams the tensor.  Resolves chain through the RNG state (#1 -> #2 -> #3, one cluster each); each apply
             # only needs its own swap targets and runs as grid kernels, #2's on a second side stream next to resolve #3.
             side, side2 = side
-            n, three = slot["ntiles"], len(self.tile_formats) >= 3
+            three = len(self.tile_formats) >= 3
             side.wait_stream(stream)
-            sa = side.cuda_stream
             if three:
                 # every tensor restarts the seeded stream: a 40-byte copy node, kept off the stats -> init -> chain path
                 # (side2 is idle until the second resolve is done; the chain joins it before its first launch)
@@ -272,25 +268,12 @@ class GreedyBatch:
             # resolves #1 (stream position only) and #2 in one launch: the cluster keeps its SMs while the tile-stat
             # kernels flood the rest of the GPU.  #3 is a second launch so that #2's apply - all the first chain launch
             # needs - can start as soon as #2 is resolved; #3 has until the later passes start.
-            check(L.qa_perm_resolve_chain(self._rng0.data_ptr(), n, 2, 0b10, slot["jarr"].data_ptr(), slot["rngs"].data_ptr(), sa),
-                  "qa_perm_resolve_chain")
-            mark("resolve", side)
-            if three:
-                slot["ev"].record(side)
-                side2.wait_event(slot["ev"])
-                check(L.qa_perm_apply(slot["jarr"][1].data_ptr(), n, None, slot["pre_order"][0].data_ptr(),
-                                      slot["apply_work"][0].data_ptr(), side2.cuda_stream), "qa_perm_apply")
-                slot["ev_a2"].record(side2)
-                check(L.qa_perm_resolve(slot["rngs"][1].data_ptr(), n, slot["jarr"][2].data_ptr(), slot["rngs"][2].data_ptr(), sa),
-                      "qa_perm_resolve")
-                check(L.qa_perm_apply(slot["jarr"][2].data_ptr(), n, None, slot["pre_order"][1].data_ptr(),
-                                      slot["apply_work"][1].data_ptr(), sa), "qa_perm_apply")
-                slot["ev_a3"].record(side)
-            else:
-                check(L.qa_perm_apply(slot["jarr"][1].data_ptr(), n, None, slot["pre_order"][0].data_ptr(),
-                                      slot["apply_work"][0].data_ptr(), sa), "qa_perm_apply")
-                slot["ev_a2"].record(side)
-        if pre and lead and not cached:
+            resolved = slot["ev"] if self.trace is None else torch.cuda.Event(enable_timing=True)
+            engine.enqueue_perm_prefetch(self._rng0, slot["ntiles"], three,
+                                         (slot["jarr"], slot["pre_order"], slot["rngs"], slot["apply_work"]), side, side2,
+                                         (resolved, slot["ev_a2"], slot["ev_a3"]))
+            if self.trace is not None:
+                self.trace.setdefault(id(slot), {})["resolve"] = resolved
             mark("prefetch", side)
         mode = STATS_FAST if self.metric == "mae" else STATS_FAST_APPROX_ABS
         iargs = (slot["table"].data_ptr(), slot["ntiles"], METRIC_CODE[self.metric], self._order, len(self.tile_formats),
@@ -343,10 +326,10 @@ class GreedyBatch:
                     tiles_w = -(-slot["cols"] // 32)
                     check(L.qa_greedy_init_sums_range(*iargs, split * tiles_w, slot["ntiles"], sp), "qa_greedy_init_sums_range")
                     stream.wait_stream(ss)
-                elif pre_event is not None:
-                    check(L.qa_greedy_init_sums_range(*iargs, 0, slot["ntiles"], sp), "qa_greedy_init_sums_range")
                 else:
-                    check(L.qa_greedy_init(*iargs, sp), "qa_greedy_init")
+                    if pre_event is None:
+                        check(L.qa_greedy_init_deltas(*iargs, sp), "qa_greedy_init_deltas")
+                    check(L.qa_greedy_init_sums_range(*iargs, 0, slot["ntiles"], sp), "qa_greedy_init_sums_range")
                 mark("init")
                 pargs = args + (slot["pre_order"].data_ptr() if pre else None, slot["rngs"][1].data_ptr() if pre else None,
                                 slot["init"].data_ptr())

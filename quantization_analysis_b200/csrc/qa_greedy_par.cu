@@ -27,7 +27,6 @@
 #include <cooperative_groups.h>
 
 #include <cstdio>
-#include <cstdlib>
 
 #include <mutex>
 
@@ -79,11 +78,11 @@ struct ParWork {
     int32_t* bucket;  // [n]
     int32_t* succ;    // [n]
     int32_t* parent;  // [n]
-    double* hdr;      // [32]    initial sums + diagnostics (greedy_init_kernel or the inline init phase)
+    double* hdr;      // [32]    initial sums + diagnostics (greedy_init_kernel)
     double* res;      // [32]    running state handed from one launch of the chain to the next (pass ranges)
     double* delta;    // [3][n][4] per-tile deltas {sy, sy2, sxy, sabs} of the format transitions, tile order
     uint8_t* fixed;   // [n]
-    const int32_t* pre_order;   // optional: permutations #2 (and #3) of n items, drawn ahead by greedy_prefetch_kernel
+    const int32_t* pre_order;   // optional: permutations #2 (and #3) of n items, drawn ahead (qa_perm_resolve[_chain] + qa_perm_apply)
     const qa_pcg64* pre_rng;    //           and the stream states after permutation #2 (and #3)
     int npre;                   // how many permutations were drawn ahead (0, 2 or 3)
 };
@@ -1073,31 +1072,6 @@ __global__ void __launch_bounds__(GT) perm_resolve_chain_kernel(const qa_pcg64* 
     if (c.gtid == 0) stamp(1, true);
 }
 
-// The first permutations of a greedy run do not depend on the data: the base pass permutes all n tiles (only the
-// stream position matters, the order is irrelevant); unless the base state already fails, pass 2 permutes all n
-// tiles again; and when pass 2 accepts every tile (the usual outcome for the first, nearly lossless candidate
-// format) pass 3 permutes all n tiles once more.  This kernel draws them ahead of time so they overlap the
-// tile-stat pass on another stream; the greedy checks the candidate count before it uses the speculative third one.
-__global__ void __launch_bounds__(GT) greedy_prefetch_kernel(const qa_pcg64* rng_in, int n, int npre, int32_t* order_out,
-                                                             qa_pcg64* rng_out, ParWork w) {
-    __shared__ Sh sh;
-    Coop c(sh);
-    Pcg g;
-    g.load(rng_in);
-    c.sync();
-    perm_resolve(c, g, n, nullptr);               // permutation #1: stream position only
-    for (int k = 0; k + 2 <= npre; ++k) {
-        c.sync();                                 // the previous apply has finished reading jarr
-        perm_resolve(c, g, n, w.jarr);
-        perm_apply(c, n, nullptr, order_out + (size_t)k * n, w);
-        if (c.gtid == 0) {
-            rng_out[k].inc_hi = g.inc.hi;
-            rng_out[k].inc_lo = g.inc.lo;
-            g.store(rng_out + k);
-        }
-    }
-}
-
 // Per-thread staging of the chunk's addends in shared memory ([slot][thread] layout: conflict-free), so the
 // walks of a round read them at shared-memory latency instead of re-fetching from L2.
 constexpr int STAGE_SLOTS = 4 * EPS;                 // up to 4 streams x EPS elements per thread
@@ -1249,13 +1223,13 @@ __device__ void faithful_init_sums(Coop& c, const double* const (&col)[NC], int 
 }
 
 // ---------------------------------------------------------------------------------------------
-// init phase: initial sums + per-transition delta tables (data-dependent, permutation-independent)
+// init phase: initial sums and per-transition drift bounds (data-dependent, permutation-independent)
 // ---------------------------------------------------------------------------------------------
 // hdr: [0] sx  [1] sx2  [2..5] sy, sy2, sxy, sabs of the base format  [6] degraded bits  [7] cycles
 //      [8] cycles of the non-negative columns  [9] cycles of the signed columns  [10] scan rounds
 template <bool PCC>
-__device__ void init_phase(Coop& c, const double* __restrict__ table, int nt, const ParOrder& ord, double* hdr, double* delta,
-                           bool build_deltas, int t_begin, int t_end) {
+__device__ void init_phase(Coop& c, const double* __restrict__ table, int nt, const ParOrder& ord, double* hdr, int t_begin,
+                           int t_end) {
     // Tiles [t_begin, t_end) of the sequential sums; a call with t_end < nt only advances the sums of the non-negative
     // columns (kept in hdr[16..19]) so that it can run while the rest of the table is still being produced; the call that
     // reaches nt finishes everything else.
@@ -1329,24 +1303,6 @@ __device__ void init_phase(Coop& c, const double* __restrict__ table, int nt, co
         }
         S[3] = R[0];
     }
-    // delta[tr][t] = stats(fmt[tr+1]) - stats(fmt[tr]) of tile t: one 32-byte record per tile and transition, so the
-    // chain fetches a visited tile with one sector instead of eight
-    if (build_deltas) {
-        for (int t = c.gtid; t < nt; t += c.gth) {
-            double v[QA_NFMT][4];
-#pragma unroll
-            for (int f = 0; f < QA_NFMT; ++f)
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v[f][q] = f < ord.n ? table[(size_t)QA_STAT_FMT(ord.fmt[f], q) * nt + t] : 0.0;
-#pragma unroll
-            for (int tr = 0; tr + 1 < QA_NFMT; ++tr) {
-                if (tr + 1 >= ord.n) break;
-                double2* dst = reinterpret_cast<double2*>(delta + ((size_t)tr * nt + t) * 4);
-                dst[0] = make_double2(__dsub_rn(v[tr + 1][0], v[tr][0]), __dsub_rn(v[tr + 1][1], v[tr][1]));
-                dst[1] = make_double2(__dsub_rn(v[tr + 1][2], v[tr][2]), __dsub_rn(v[tr + 1][3], v[tr][3]));
-            }
-        }
-    }
     if (c.gtid == 0) {
 #pragma unroll
         for (int tr = 0; tr + 1 < QA_NFMT; ++tr) hdr[11 + tr] = dr_sum[tr];
@@ -1359,18 +1315,17 @@ __device__ void init_phase(Coop& c, const double* __restrict__ table, int nt, co
 
 template <bool PCC>
 __global__ void __launch_bounds__(GT) greedy_init_kernel(const double* __restrict__ table, int nt, ParOrder ord, double* hdr,
-                                                         double* delta, int t_begin, int t_end) {
+                                                         int t_begin, int t_end) {
     __shared__ Sh sh;
     Coop c(sh);
     if (c.gtid == 0) stamp(2, false);
-    init_phase<PCC>(c, table, nt, ord, hdr, delta, delta != nullptr, t_begin, t_end);
+    init_phase<PCC>(c, table, nt, ord, hdr, t_begin, t_end);
     if (c.gtid == 0) stamp(3, true);
 }
 
-// delta records of every format transition, one thread per tile (the grid-kernel half of qa_greedy_init)
-__global__ void __launch_bounds__(256) greedy_delta_kernel(const double* __restrict__ table, int nt, ParOrder ord, double* delta) {
-    const int t = blockIdx.x * 256 + threadIdx.x;
-    if (t >= nt) return;
+// delta[tr][t] = stats(fmt[tr+1]) - stats(fmt[tr]) of tile t: one 32-byte record per tile and transition, so the chain
+// fetches a visited tile with one sector instead of eight
+__device__ __forceinline__ void write_deltas(const double* __restrict__ table, int nt, const ParOrder& ord, double* delta, int t) {
     double v[QA_NFMT][4];
 #pragma unroll
     for (int f = 0; f < QA_NFMT; ++f)
@@ -1383,6 +1338,13 @@ __global__ void __launch_bounds__(256) greedy_delta_kernel(const double* __restr
         dst[0] = make_double2(__dsub_rn(v[tr + 1][0], v[tr][0]), __dsub_rn(v[tr + 1][1], v[tr][1]));
         dst[1] = make_double2(__dsub_rn(v[tr + 1][2], v[tr][2]), __dsub_rn(v[tr + 1][3], v[tr][3]));
     }
+}
+
+// delta records of every format transition, one thread per tile
+__global__ void __launch_bounds__(256) greedy_delta_kernel(const double* __restrict__ table, int nt, ParOrder ord, double* delta) {
+    const int t = blockIdx.x * 256 + threadIdx.x;
+    if (t >= nt) return;
+    write_deltas(table, nt, ord, delta, t);
 }
 
 // the same for a descriptor array of tensors: block b finds its tensor by bisection over the block prefix
@@ -1397,20 +1359,7 @@ __global__ void __launch_bounds__(256) greedy_delta_batch_kernel(const qa_batch_
     const int nt = (int)(cdiv(d.rows, TILE) * cdiv(d.cols, TILE));
     const int t = (int)(b - d.block_begin) * 256 + threadIdx.x;
     if (t >= nt) return;
-    const double* table = d.table;
-    double* delta = reinterpret_cast<double*>(reinterpret_cast<char*>(d.init) + hdr_bytes);
-    double v[QA_NFMT][4];
-#pragma unroll
-    for (int f = 0; f < QA_NFMT; ++f)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) v[f][q] = f < ord.n ? table[(size_t)QA_STAT_FMT(ord.fmt[f], q) * nt + t] : 0.0;
-#pragma unroll
-    for (int tr = 0; tr + 1 < QA_NFMT; ++tr) {
-        if (tr + 1 >= ord.n) break;
-        double2* dst = reinterpret_cast<double2*>(delta + ((size_t)tr * nt + t) * 4);
-        dst[0] = make_double2(__dsub_rn(v[tr + 1][0], v[tr][0]), __dsub_rn(v[tr + 1][1], v[tr][1]));
-        dst[1] = make_double2(__dsub_rn(v[tr + 1][2], v[tr][2]), __dsub_rn(v[tr + 1][3], v[tr][3]));
-    }
+    write_deltas(d.table, nt, ord, reinterpret_cast<double*>(reinterpret_cast<char*>(d.init) + hdr_bytes), t);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1429,13 +1378,14 @@ __global__ void __launch_bounds__(256) greedy_delta_batch_kernel(const qa_batch_
 #else
 #define QA_CHAIN_REGCAP __launch_bounds__(GT, 1)
 #endif
-template <bool PCC, bool INIT_INLINE>      // INIT_INLINE = false: the init phase ran ahead (greedy_init_kernel); its code is left out
+template <bool PCC>
 __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ table, int nt, double numel, int metric,
                                                         double thr, ParOrder ord, qa_pcg64* rng, int8_t* assignment,
-                                                        int64_t* counts, double* state, ParWork w, int have_init, int fi_begin,
-                                                        int fi_end, int flags) {
+                                                        int64_t* counts, double* state, ParWork w, int fi_begin, int fi_end,
+                                                        int flags) {
     // Passes [fi_begin, fi_end) of the format order.  A run may be split into several launches (so that a later pass can
-    // wait for a prefetched permutation that an earlier one does not need); the running state travels in w.res.
+    // wait for a prefetched permutation that an earlier one does not need); the running state travels in w.res.  The
+    // initial sums and delta records (w.hdr, w.delta) were written ahead of the chain by greedy_init_kernel and a delta kernel.
     __shared__ Sh sh;
     Coop c(sh);
     const int tid = threadIdx.x;
@@ -1458,11 +1408,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
     c.sync();
     const long long t_start = clock64();
 
-    // ---- (1) initial sums, sequentially rounded in tile order (greedy_init_kernel ran ahead, or inline) ----
-    if (INIT_INLINE && first && !have_init) {
-        init_phase<PCC>(c, table, nt, ord, w.hdr, w.delta, true, 0, nt);
-        c.sync();
-    }
+    // ---- (1) initial sums, sequentially rounded in tile order (greedy_init_kernel) ----
     Consts k;
     k.n = numel; k.thr = thr; k.metric = metric;
     k.sx = w.hdr[0]; k.sx2 = w.hdr[1];
@@ -1474,7 +1420,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
     long long t_mark = clock64(), cyc_perm = 0, cyc_chain = 0;
     long long cy_load = 0, cy_scan = 0, cy_dec = 0, cy_min = 0, cy_commit = 0, cy_gather = 0, tq = 0;
     unsigned n_chunks = 0, n_cutshort = 0;
-    const long long cyc_init = have_init ? (long long)w.hdr[7] : t_mark - t_start;
+    const long long cyc_init = (long long)w.hdr[7];
     const int CHc = c.gth * EPS;
     bool base_failed = false, all_tiles_candidates = true, done = false;
     int accepted_last = nt;
@@ -1554,7 +1500,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
         const bool have_pre = w.pre_order != nullptr && w.npre >= 2 && ord.n >= 2;
         order_ptr = w.order;
         if (have_pre && fi == 0) {
-            // permutations #1 and #2 were drawn ahead of time (greedy_prefetch_kernel); nothing to do for the base pass
+            // permutations #1 and #2 were drawn ahead of time; nothing to do for the base pass
         } else if (have_pre && fi == 1) {
             order_ptr = w.pre_order;          // m == nt here: candidates are 0..nt-1 in order, so perm[k] is the tile
             g.load(w.pre_rng);
@@ -1891,25 +1837,13 @@ static ParWork carve(void* work, int64_t n) {
     return w;
 }
 
-static int pick_cluster_auto(int64_t n);
 static thread_local int g_cluster_cap = 0;   // qa_greedy_cluster_cap: upper bound on the cluster size (0 = none), per calling thread
 
 static int pick_cluster(int64_t n) {
-    const int r = pick_cluster_auto(n);
-    return g_cluster_cap > 0 && r > g_cluster_cap ? g_cluster_cap : r;
-}
-
-static int pick_cluster_auto(int64_t n) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char* e = getenv("QA_GREEDY_CLUSTER");
-        forced = e ? atoi(e) : 0;
-    }
-    if (forced > 0) return forced > MAXR ? MAXR : forced;
     int r = 1;
     while (r < 8 && (int64_t)r * GT * DPT < n) r <<= 1;          // grow until one draw round covers the tensor
     if (n >= 65536) r = 16;                                      // opt-in (non-portable) size for the largest tensors
-    return r;
+    return g_cluster_cap > 0 && r > g_cluster_cap ? g_cluster_cap : r;
 }
 
 template <typename... KArgs, typename... Args>
@@ -2031,16 +1965,6 @@ extern "C" int qa_perm_resolve_chain(const qa_pcg64* rng_in, int64_t n, int coun
                           jarr, rng_out);
 }
 
-extern "C" int qa_greedy_prefetch(const qa_pcg64* rng, int64_t n, int nfmt, int32_t* pre_order, qa_pcg64* pre_rng, void* work,
-                                  qa_stream_t stream) {
-    if (!rng || n <= 0 || n > 0x3FFFFFFF || nfmt < 2 || nfmt > QA_NFMT || !pre_order || !pre_rng || !work) {
-        set_error("qa_greedy_prefetch: bad args");
-        return 1;
-    }
-    return launch_cluster(greedy_prefetch_kernel, pick_cluster(n), (cudaStream_t)stream, rng, (int)n, nfmt >= 3 ? 3 : 2, pre_order,
-                          pre_rng, carve(work, n));
-}
-
 static int fill_order(const int32_t* fmt_order, int nfmt, ParOrder& ord, const char* who) {
     if (!fmt_order || nfmt < 1 || nfmt > QA_NFMT) { set_error("%s: bad format order", who); return 1; }
     ord.n = nfmt;
@@ -2050,48 +1974,42 @@ static int fill_order(const int32_t* fmt_order, int nfmt, ParOrder& ord, const c
     return 0;
 }
 
-static int greedy_init_launch(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt, void* init,
-                              bool sums, bool deltas, bool deltas_in_cluster, qa_stream_t stream, const char* who,
-                              int64_t t_begin = 0, int64_t t_end = -1) {
+// an init buffer (qa_greedy_init_bytes) holds the header and then the delta records
+static double* init_delta(const void* init) {
+    return reinterpret_cast<double*>(static_cast<char*>(const_cast<void*>(init)) + al(8 * HDR_DOUBLES));
+}
+
+// On one stream: the delta records (a grid kernel) if delta != NULL, then the initial sums over tiles [t_begin, t_end) (one
+// cluster) if hdr != NULL
+static int greedy_init_launch(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt, double* hdr,
+                              double* delta, qa_stream_t stream, const char* who, int64_t t_begin = 0, int64_t t_end = -1) {
     if (t_end < 0) t_end = ntiles;
     if (t_begin < 0 || t_begin >= t_end || t_end > ntiles) { set_error("%s: bad tile range", who); return 1; }
-    if (!table || ntiles <= 0 || ntiles > 0x3FFFFFFF || !init) { set_error("%s: bad args", who); return 1; }
+    if (!table || ntiles <= 0 || ntiles > 0x3FFFFFFF || !(hdr || delta)) { set_error("%s: bad args", who); return 1; }
     if (metric != QA_METRIC_PCC && metric != QA_METRIC_MAE) { set_error("%s: metric must be pcc or mae", who); return 1; }
     ParOrder ord;
     if (fill_order(fmt_order, nfmt, ord, who)) return 1;
-    double* hdr = reinterpret_cast<double*>(init);
-    double* delta = reinterpret_cast<double*>(reinterpret_cast<char*>(init) + al(8 * HDR_DOUBLES));
     cudaStream_t s = (cudaStream_t)stream;
-    if (deltas && !deltas_in_cluster) {
+    if (delta) {
         greedy_delta_kernel<<<(unsigned)cdiv(ntiles, 256), 256, 0, s>>>(table, (int)ntiles, ord, delta);
         if (int rc = check_launch(who)) return rc;
     }
-    if (!sums) return 0;
-    double* dcl = deltas_in_cluster ? delta : nullptr;
+    if (!hdr) return 0;
     if (metric == QA_METRIC_PCC)
-        return launch_cluster(greedy_init_kernel<true>, pick_cluster(ntiles), s, table, (int)ntiles, ord, hdr, dcl, (int)t_begin, (int)t_end);
-    return launch_cluster(greedy_init_kernel<false>, pick_cluster(ntiles), s, table, (int)ntiles, ord, hdr, dcl, (int)t_begin, (int)t_end);
-}
-
-extern "C" int qa_greedy_init(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt, void* init,
-                              qa_stream_t stream) {
-    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, init, true, true, false, stream, "qa_greedy_init");
-}
-
-extern "C" int qa_greedy_init_sums(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt, void* init,
-                                   qa_stream_t stream) {
-    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, init, true, false, false, stream, "qa_greedy_init_sums");
+        return launch_cluster(greedy_init_kernel<true>, pick_cluster(ntiles), s, table, (int)ntiles, ord, hdr, (int)t_begin, (int)t_end);
+    return launch_cluster(greedy_init_kernel<false>, pick_cluster(ntiles), s, table, (int)ntiles, ord, hdr, (int)t_begin, (int)t_end);
 }
 
 extern "C" int qa_greedy_init_sums_range(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt,
                                          void* init, int64_t tile_begin, int64_t tile_end, qa_stream_t stream) {
-    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, init, true, false, false, stream, "qa_greedy_init_sums_range",
-                              tile_begin, tile_end);
+    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, static_cast<double*>(init), nullptr, stream,
+                              "qa_greedy_init_sums_range", tile_begin, tile_end);
 }
 
 extern "C" int qa_greedy_init_deltas(const double* table, int64_t ntiles, int metric, const int32_t* fmt_order, int nfmt, void* init,
                                      qa_stream_t stream) {
-    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, init, false, true, false, stream, "qa_greedy_init_deltas");
+    return greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, nullptr, init ? init_delta(init) : nullptr, stream,
+                              "qa_greedy_init_deltas");
 }
 
 extern "C" int qa_greedy_init_deltas_batch(const qa_batch_desc* descs_dev, int n, int64_t total_blocks, const int32_t* fmt_order, int nfmt,
@@ -2118,33 +2036,25 @@ extern "C" int qa_greedy_assign_passes(const double* table, int64_t ntiles, doub
     if (fill_order(fmt_order, nfmt, ord, "qa_greedy_assign_par")) return 1;
     ParWork pw = carve(work, ntiles);
     if (pre_order && pre_rng && nfmt >= 2) { pw.pre_order = pre_order; pw.pre_rng = pre_rng; pw.npre = nfmt >= 3 ? 3 : 2; }
-    int have_init = 0;
     if (init) {
-        pw.hdr = const_cast<double*>(reinterpret_cast<const double*>(init));
-        pw.delta = const_cast<double*>(reinterpret_cast<const double*>(reinterpret_cast<const char*>(init) + al(8 * HDR_DOUBLES)));
-        have_init = 1;
+        pw.hdr = static_cast<double*>(const_cast<void*>(init));
+        pw.delta = init_delta(init);
+    } else if (pass_begin == 0) {
+        // no init buffer: the call that runs pass 0 computes it into `work`, where the later pass ranges find it
+        if (int rc = greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, pw.hdr, pw.delta, stream, "qa_greedy_assign_par")) return rc;
     }
     const int nr = pick_cluster(ntiles);
     cudaStream_t cs = (cudaStream_t)stream;
-#define QA_LAUNCH_CHAIN(P, I)                                                                                                  \
-    launch_cluster(greedy_par_kernel<P, I>, nr, cs, table, (int)ntiles, numel, metric, threshold, ord, rng, assignment, counts, \
-                   state, pw, have_init, pass_begin, pass_end, flags)
-    if (metric == QA_METRIC_PCC) return have_init ? QA_LAUNCH_CHAIN(true, false) : QA_LAUNCH_CHAIN(true, true);
-    return have_init ? QA_LAUNCH_CHAIN(false, false) : QA_LAUNCH_CHAIN(false, true);
-#undef QA_LAUNCH_CHAIN
-}
-
-extern "C" int qa_greedy_assign_par_pre(const double* table, int64_t ntiles, double numel, int metric, double threshold,
-                                        const int32_t* fmt_order, int nfmt, qa_pcg64* rng, int8_t* assignment,
-                                        int64_t* counts, double* state, void* work, const int32_t* pre_order,
-                                        const qa_pcg64* pre_rng, const void* init, qa_stream_t stream) {
-    return qa_greedy_assign_passes(table, ntiles, numel, metric, threshold, fmt_order, nfmt, rng, assignment, counts, state, work,
-                                   pre_order, pre_rng, init, 0, nfmt, 0, stream);
+    if (metric == QA_METRIC_PCC)
+        return launch_cluster(greedy_par_kernel<true>, nr, cs, table, (int)ntiles, numel, metric, threshold, ord, rng, assignment, counts,
+                              state, pw, pass_begin, pass_end, flags);
+    return launch_cluster(greedy_par_kernel<false>, nr, cs, table, (int)ntiles, numel, metric, threshold, ord, rng, assignment, counts,
+                          state, pw, pass_begin, pass_end, flags);
 }
 
 extern "C" int qa_greedy_assign_par(const double* table, int64_t ntiles, double numel, int metric, double threshold,
                                     const int32_t* fmt_order, int nfmt, qa_pcg64* rng, int8_t* assignment,
                                     int64_t* counts, double* state, void* work, qa_stream_t stream) {
-    return qa_greedy_assign_par_pre(table, ntiles, numel, metric, threshold, fmt_order, nfmt, rng, assignment, counts, state,
-                                    work, nullptr, nullptr, nullptr, stream);
+    return qa_greedy_assign_passes(table, ntiles, numel, metric, threshold, fmt_order, nfmt, rng, assignment, counts, state, work,
+                                   nullptr, nullptr, nullptr, 0, nfmt, 0, stream);
 }

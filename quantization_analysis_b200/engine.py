@@ -317,18 +317,43 @@ def numpy_integers(rng: torch.Tensor, k: int, n: int) -> torch.Tensor:
     return out
 
 
-def greedy_prefetch(rng: torch.Tensor, ntiles: int, work: torch.Tensor | None = None, nfmt: int = NFMT):
-    """Draw the data-independent permutations of a greedy run ahead of time (qa_greedy_prefetch).
+def enqueue_perm_prefetch(rng0: torch.Tensor, nt: int, three: bool, bufs, side, side2, events) -> None:
+    """Enqueue the data-independent permutations of a greedy run over nt tiles, drawn from the stream state `rng0` (not
+    modified): resolves #1 (stream position only) and #2 in one cluster launch on `side`, then #2's apply on `side2`
+    next to resolve #3 and #3's apply on `side`.  Without `three` (fewer than three formats) only #2 is applied, on `side`.
+    bufs = (jarr int32[3, nt], pre_order int32[2, nt], rngs [3, 5], awork uint8[2, qa_perm_apply_work_bytes(nt)]): the
+    chain reads pre_order (visiting orders of passes 2 and 3) and rngs[1:] (stream states after permutations #2 and #3).
+    events = (resolved, applied2, applied3), recorded once #1 and #2 are resolved, once pre_order[0] is written and once
+    pre_order[1] is (three only)."""
+    L = _lib.lib()
+    jarr, pre_order, rngs, awork = bufs
+    resolved, applied2, applied3 = events
+    check(L.qa_perm_resolve_chain(_ptr(rng0), nt, 2, 0b10, _ptr(jarr), _ptr(rngs), side.cuda_stream), "qa_perm_resolve_chain")
+    resolved.record(side)
+    s2 = side
+    if three:
+        side2.wait_event(resolved)
+        s2 = side2
+    check(L.qa_perm_apply(_ptr(jarr[1]), nt, None, _ptr(pre_order[0]), _ptr(awork[0]), s2.cuda_stream), "qa_perm_apply")
+    applied2.record(s2)
+    if three:
+        check(L.qa_perm_resolve(_ptr(rngs[1]), nt, _ptr(jarr[2]), _ptr(rngs[2]), side.cuda_stream), "qa_perm_resolve")
+        check(L.qa_perm_apply(_ptr(jarr[2]), nt, None, _ptr(pre_order[1]), _ptr(awork[1]), side.cuda_stream), "qa_perm_apply")
+        applied3.record(side)
+
+
+def greedy_prefetch(rng: torch.Tensor, ntiles: int, nfmt: int = NFMT):
+    """enqueue_perm_prefetch on the current stream, for greedy_assign(prefetched=...).
     -> (pre_order int32[1 or 2][ntiles], pre_rng[1 or 2]).  `rng` is not modified."""
     L = _lib.lib()
     dev = rng.device
-    k = 2 if nfmt >= 3 else 1
-    pre_order = torch.empty((k, ntiles), dtype=torch.int32, device=dev)
-    pre_rng = torch.empty((k,) + tuple(rng.shape), dtype=rng.dtype, device=dev)
-    if work is None:
-        work = torch.empty(L.qa_greedy_par_work_bytes(ntiles), dtype=torch.uint8, device=dev)
-    check(L.qa_greedy_prefetch(_ptr(rng), ntiles, nfmt, _ptr(pre_order), _ptr(pre_rng), _ptr(work), _stream()), "qa_greedy_prefetch")
-    return pre_order, pre_rng
+    three = nfmt >= 3
+    bufs = (torch.empty((3, ntiles), dtype=torch.int32, device=dev), torch.empty((2, ntiles), dtype=torch.int32, device=dev),
+            torch.stack([rng, rng, rng]).contiguous(), torch.empty((2, L.qa_perm_apply_work_bytes(ntiles)), dtype=torch.uint8, device=dev))
+    cur = torch.cuda.current_stream(dev)
+    enqueue_perm_prefetch(rng, ntiles, three, bufs, cur, cur, [torch.cuda.Event() for _ in range(3)])
+    k = 2 if three else 1
+    return bufs[1][:k], bufs[2][1:1 + k]
 
 
 def numpy_permutation_staged(rng: torch.Tensor, n: int) -> torch.Tensor:
@@ -346,12 +371,14 @@ def numpy_permutation_staged(rng: torch.Tensor, n: int) -> torch.Tensor:
 
 
 def greedy_init(table: torch.Tensor, metric: str, fmt_order) -> torch.Tensor:
-    """Initial sums + per-transition delta records of a greedy run (qa_greedy_init); consumed by greedy_assign(init=...)."""
+    """Initial sums + per-transition delta records of a greedy run (qa_greedy_init_deltas, qa_greedy_init_sums_range);
+    consumed by greedy_assign(init=...)."""
     L = _lib.lib()
     nt = table.shape[1]
     init = torch.empty(L.qa_greedy_init_bytes(nt), dtype=torch.uint8, device=table.device)
-    order = _lib.int32_array([FMT_INDEX[f] for f in fmt_order])
-    check(L.qa_greedy_init(_ptr(table), nt, METRIC_CODE[metric], order, len(fmt_order), _ptr(init), _stream()), "qa_greedy_init")
+    iargs = (_ptr(table), nt, METRIC_CODE[metric], _lib.int32_array([FMT_INDEX[f] for f in fmt_order]), len(fmt_order), _ptr(init))
+    check(L.qa_greedy_init_deltas(*iargs, _stream()), "qa_greedy_init_deltas")
+    check(L.qa_greedy_init_sums_range(*iargs, 0, nt, _stream()), "qa_greedy_init_sums_range")
     return init
 
 
@@ -359,7 +386,8 @@ def greedy_assign(table: torch.Tensor, numel: int, metric: str, threshold: float
                   parallel: bool | None = None, prefetched=None, init: torch.Tensor | None = None, split_at: int | None = None):
     """-> (assignment int8[ntiles], counts int64[4], state float64[24]) on device.
     parallel=None: the cluster-parallel kernel for pcc / mae, the one-thread chain for atol.
-    prefetched = greedy_prefetch(...) and init = greedy_init(...) are optional stages computed ahead of time."""
+    prefetched = greedy_prefetch(...) and init = greedy_init(...) are optional stages computed ahead of time; without init the
+    first launch computes it into its work buffer."""
     nt = table.shape[1]
     dev = table.device
     L = _lib.lib()
@@ -392,8 +420,8 @@ _STAGE_STREAMS: dict = {}
 
 def greedy_assign_staged(table: torch.Tensor, numel: int, metric: str, threshold: float, fmt_order, rng: torch.Tensor):
     """greedy_assign for one tensor with the stages overlapped on side streams: the data-independent permutations
-    (qa_perm_resolve_chain / qa_perm_resolve / qa_perm_apply) next to the initial sums and delta records
-    (qa_greedy_init_sums / qa_greedy_init_deltas), then the chain by pass range (qa_greedy_assign_passes).
+    (enqueue_perm_prefetch) next to the initial sums and delta records (qa_greedy_init_sums_range / qa_greedy_init_deltas),
+    then the chain by pass range (qa_greedy_assign_passes).
     Same outputs, bit for bit, as greedy_assign; about half its latency on a large tensor.  `rng` is advanced."""
     if metric not in ("pcc", "mae") or len(fmt_order) < 2:
         return greedy_assign(table, numel, metric, threshold, fmt_order, rng)
@@ -416,24 +444,13 @@ def greedy_assign_staged(table: torch.Tensor, numel: int, metric: str, threshold
     pre_order = torch.empty((2, nt), dtype=torch.int32, device=dev)
     rngs = torch.stack([rng, rng, rng]).contiguous()
     awork = torch.empty((2, L.qa_perm_apply_work_bytes(nt)), dtype=torch.uint8, device=dev)
-    ev2, ev_a2, ev_a3 = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
+    ev_a2, ev_a3 = torch.cuda.Event(), torch.cuda.Event()
     side.wait_stream(cur)
     side2.wait_stream(cur)
-    check(L.qa_perm_resolve_chain(_ptr(rng), nt, 2, 0b10, _ptr(jarr), _ptr(rngs), side.cuda_stream), "qa_perm_resolve_chain")
-    if three:
-        ev2.record(side)
-        side2.wait_event(ev2)
-        check(L.qa_perm_apply(_ptr(jarr[1]), nt, None, _ptr(pre_order[0]), _ptr(awork[0]), side2.cuda_stream), "qa_perm_apply")
-        ev_a2.record(side2)
-        check(L.qa_perm_resolve(_ptr(rngs[1]), nt, _ptr(jarr[2]), _ptr(rngs[2]), side.cuda_stream), "qa_perm_resolve")
-        check(L.qa_perm_apply(_ptr(jarr[2]), nt, None, _ptr(pre_order[1]), _ptr(awork[1]), side.cuda_stream), "qa_perm_apply")
-        ev_a3.record(side)
-    else:
-        check(L.qa_perm_apply(_ptr(jarr[1]), nt, None, _ptr(pre_order[0]), _ptr(awork[0]), side.cuda_stream), "qa_perm_apply")
-        ev_a2.record(side)
+    enqueue_perm_prefetch(rng, nt, three, (jarr, pre_order, rngs, awork), side, side2, (torch.cuda.Event(), ev_a2, ev_a3))
     iargs = (_ptr(table), nt, METRIC_CODE[metric], order, nf, _ptr(init))
     check(L.qa_greedy_init_deltas(*iargs, _stream()), "qa_greedy_init_deltas")
-    check(L.qa_greedy_init_sums(*iargs, _stream()), "qa_greedy_init_sums")
+    check(L.qa_greedy_init_sums_range(*iargs, 0, nt, _stream()), "qa_greedy_init_sums_range")
     pargs = (_ptr(table), nt, float(numel), METRIC_CODE[metric], float(threshold), order, nf, _ptr(rng), _ptr(assignment),
              _ptr(counts), _ptr(state), _ptr(work), _ptr(pre_order), _ptr(rngs[1]), _ptr(init))
     cur.wait_event(ev_a2)

@@ -380,9 +380,11 @@ def test_table_and_init_in_pieces(qa):
 
 
 def test_greedy_staged_equals_inline(qa):
-    """qa_greedy_prefetch / qa_greedy_init + qa_greedy_assign_par_pre give the same map, counts, state and stream
-    position as the kernel that does everything inline, in every combination of stages - including a base state that
-    already fails, a pass 2 that accepts every tile (speculative third permutation used) and one that does not."""
+    """Prefetched permutations (engine.greedy_prefetch: the product's enqueue_perm_prefetch) and a precomputed init buffer
+    (qa_greedy_init_deltas + qa_greedy_init_sums_range) given to qa_greedy_assign_passes give the same map, counts, state
+    and stream position as the call that computes init into its work buffer and draws every permutation itself, in every
+    combination of stages - including a base state that already fails, a pass 2 that accepts every tile (speculative
+    third permutation used) and one that does not."""
     eng = qa["engine"]
     x = G.algo_input("het_256x512")
     p = eng.prepare_tiles(x)
