@@ -85,14 +85,10 @@ class MixedTileGreedyCompression(CompressionAlgorithm):
 
     def run_fp8_blocks(self, w_fp8, scale_inv, formats=None, seed: int | None = None) -> mc.DeviceResult:
         """Extension for real checkpoints: an fp8 e4m3fn tensor + per-block inverse scales as stored on disk
-        (hf_model_utils.py:199-215,271-281).  The table comes from one pass over the bytes (qa_tile_stats_fp8); the result is what
-        `run` gives on the reference's dequantized float32 tensor."""
+        (hf_model_utils.py:199-215,271-281).  The table comes from one pass over the bytes (engine.tile_stats on an Fp8Prepared);
+        the result is what `run` gives on the reference's dequantized float32 tensor."""
         tile_formats = self.tile_formats or self._filter_from_formats(formats or MIXED_TILE_FORMATS)
-        p = engine.Fp8Prepared(w_fp8, scale_inv)
-        table = None
-        if not self.strict:
-            table, _ = engine.tile_stats_fp8(p.w8, p.scale_inv, MIXED_TILE_FORMATS, exact_abs=(self.metric == "mae"))
-        return self.run_prepared(p, tile_formats, table=table, seed=seed)
+        return self.run_prepared(engine.Fp8Prepared(w_fp8, scale_inv), tile_formats, seed=seed)
 
     def _compress(self, xf, quantizer, tile_formats):
         if mc.numel_of(xf) == 0:

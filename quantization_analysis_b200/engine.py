@@ -15,7 +15,7 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, tensor_source
 from ._lib import (METRIC_CODE, NFMT, NSTAT, QA_DT_BF16, QA_DT_F32, STATS_FAST, STATS_FAST_APPROX_ABS, STATS_STRICT,
                    check)
 
@@ -117,6 +117,16 @@ def to_device(x, want_bf16: bool = True) -> tuple[torch.Tensor, int]:
     return t, QA_DT_F32
 
 
+def prepare_loaded(x) -> Prepared:
+    """What tensor_source's loaders return -> Prepared in the mixed-tile geometry: Fp8Prepared for a block-scaled fp8 weight
+    (its bytes go to the device as they are), prepare_tiles for a host array or torch tensor; a Prepared is returned as is."""
+    if isinstance(x, Prepared):
+        return x
+    if isinstance(x, tensor_source.Fp8Blocks):
+        return Fp8Prepared(x.weight, x.scale_inv)
+    return prepare_tiles(x)
+
+
 def prepare_rows(x) -> Prepared:
     """Quantizer geometry: rows of the last axis (1-D: one row)."""
     shape = tuple(x.shape)
@@ -189,7 +199,11 @@ def tile_stats(p: Prepared, formats=MIXED_FORMATS, strict: bool | None = None, e
     """float64 [NSTAT, ntiles] tile-stat table.  strict=None / False: the fast kernels (qa_tile_stats for bf16 input,
     qa_tile_stats_f32 for float32 input that is not bf16-exact); strict=True: NumPy-order sums (validation, certificate
     fallback).  exact_abs=False lets the fast kernels keep sum|x-y| in fp32 group partials (~1e-9 relative): fine when
-    that column only feeds a reported mae or an is-zero test (pcc / atol assignment)."""
+    that column only feeds a reported mae or an is-zero test (pcc / atol assignment).  An Fp8Prepared takes the fused pass
+    over its bytes (tile_stats_fp8; the same table as qa_tile_stats_f32 on its float32 image, which stays unmaterialised)
+    unless strict."""
+    if isinstance(p, Fp8Prepared) and not strict:
+        return tile_stats_fp8(p.w8, p.scale_inv, formats, exact_abs=exact_abs)[0]
     table = torch.zeros((NSTAT, p.ntiles), dtype=torch.float64, device=p.data.device)
     mode = STATS_STRICT if strict else (STATS_FAST if exact_abs else STATS_FAST_APPROX_ABS)
     if p.dtype_code == QA_DT_F32 and not strict:

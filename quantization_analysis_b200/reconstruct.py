@@ -3,8 +3,8 @@
 Mirrors scripts/reconstruct_mixed_tile_assignment.py:40-137 of the reference: read ``assignment.npy`` (int8
 ``[tiles_h, tiles_w]``) and its mapping JSON (``int_to_format``), quantize every 32x32 tile of the tensor in the format the
 map names (qa_apply_assignment: one pass, 4 B/element) and return / save the float32 reconstruction.  The reference loads
-the tensor from Hugging Face; offline this module takes the tensor itself, or a DeepSeek-R1 weight name resolved through
-``synthetic.py``.
+the tensor from the model; this module takes the tensor itself, a tensor name resolved through the ``*.safetensors`` shards
+of ``--checkpoint-dir`` (as wq reads them), a ``.npy`` file, or a DeepSeek-R1 weight name resolved through ``synthetic.py``.
 """
 from __future__ import annotations
 
@@ -15,7 +15,7 @@ from pathlib import Path
 import numpy as np
 import torch
 
-from . import engine, synthetic
+from . import engine, synthetic, tensor_source
 
 _DEVICE_FORMATS = ("bf16", "bfp8", "bfp4", "bfp2")
 
@@ -30,9 +30,10 @@ def load_mapping(path) -> list[str]:
 
 
 def reconstruct_from_assignment(x, assignment: np.ndarray, int_to_format=None) -> np.ndarray:
-    """-> float32 array of x's shape: tile (i, j) quantized in format ``int_to_format[assignment[i, j]]``."""
+    """-> float32 array of x's shape: tile (i, j) quantized in format ``int_to_format[assignment[i, j]]``.  x: a host array or
+    tensor, or what tensor_source's loaders return (tensor_source.Fp8Blocks included)."""
     int_to_format = list(int_to_format) if int_to_format is not None else list(_DEVICE_FORMATS)
-    p = engine.prepare_tiles(x)
+    p = engine.prepare_loaded(x)
     a = np.asarray(assignment, dtype=np.int8)
     expected = (p.tiles_h, p.tiles_w)
     if a.shape != expected:
@@ -49,14 +50,21 @@ def reconstruct_from_assignment(x, assignment: np.ndarray, int_to_format=None) -
 
 
 def main(argv=None) -> int:
-    ap = argparse.ArgumentParser(description="Reconstruct a (synthetic) DeepSeek-R1 tensor from a mixed-tile assignment")
-    ap.add_argument("tensor_name", help="weight name (see synthetic.DEEPSEEK_R1_SHAPES) or a .npy file with the tensor")
+    ap = argparse.ArgumentParser(description="Reconstruct a tensor from a mixed-tile assignment")
+    ap.add_argument("tensor_name", help="tensor name in --checkpoint-dir, a .npy file with the tensor, or (without "
+                                        "--checkpoint-dir) a weight name of synthetic.DEEPSEEK_R1_SHAPES")
     ap.add_argument("--assignment", required=True)
     ap.add_argument("--assignment-mapping", required=True)
     ap.add_argument("--seed", type=int, default=0, help="seed of the synthetic tensor")
     ap.add_argument("--out", default=None)
+    ap.add_argument("--checkpoint-dir", default=None, help="directory of *.safetensors shards holding tensor_name")
     args = ap.parse_args(argv)
-    if args.tensor_name.endswith(".npy"):
+    if args.checkpoint_dir is not None:
+        index = tensor_source.build_tensor_index(str(args.checkpoint_dir), checkpoint_dir=args.checkpoint_dir)
+        if args.tensor_name not in index.tensor_to_file:
+            ap.error(f"{args.tensor_name} is not in the checkpoint {args.checkpoint_dir}")
+        x = index.load(args.tensor_name)
+    elif args.tensor_name.endswith(".npy"):
         x = np.load(args.tensor_name)
     else:
         x = synthetic.randn_bf16_cpu(synthetic.DEEPSEEK_R1_SHAPES[args.tensor_name], args.seed).float().numpy()

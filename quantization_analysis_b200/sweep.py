@@ -63,12 +63,13 @@ def _score_maps(p: engine.Prepared, maps: torch.Tensor, rows_idx) -> dict[int, n
 
 def sweep_tensor(x, tile_formats=MIXED_TILE_FORMATS, metric: str = "pcc", steps: int = 32, lowest: float = 0.9,
                  thresholds=None, scoring: str = "reference"):
-    """-> (rows, maps): rows = list of dicts {threshold (float64), counts, total_bytes, pcc, mae, atol} and the int8 maps
+    """x: a host array or tensor, what tensor_source's loaders return (tensor_source.Fp8Blocks included), or an
+    engine.Prepared.  -> (rows, maps): rows = list of dicts {threshold (float64), counts, total_bytes, pcc, mae, atol} and the int8 maps
     [steps, ntiles] in MIXED_TILE_FORMATS numbering.  scoring="reference": the reference's float32 whole-tensor values
     (every distinct map is materialised and scored); "exact": float64 recombination of the tile-stat table, all maps in one
     launch, no reconstruction (the mathematically exact value of the same formulas)."""
     tile_formats = list(tile_formats)
-    p = engine.prepare_tiles(x)
+    p = engine.prepare_loaded(x)
     scores = engine.tile_scores(p, tile_formats)[_ROW[metric]].contiguous()
     if thresholds is None:
         thresholds = sweep_thresholds(scores, tile_formats, metric, steps, lowest)
@@ -100,7 +101,7 @@ def sweep_tensor(x, tile_formats=MIXED_TILE_FORMATS, metric: str = "pcc", steps:
 
 def baseline_points(x, tile_formats, metric: str, lowest: float) -> list[dict]:
     """Whole-tensor baseline of every candidate format (sweep:688-717), kept if it lies inside the swept range."""
-    p = engine.prepare_tiles(x)
+    p = engine.prepare_loaded(x)
     recon = engine.quant_recon(p, list(tile_formats))
     sc = engine.tensor_scores_f32(p.data, torch.stack([recon[f] for f in tile_formats]), n=p.numel)
     pts = []

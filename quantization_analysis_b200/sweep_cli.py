@@ -2,7 +2,9 @@
 ``details/<tensor>/sweep_config.json`` + ``sweep_results.csv``; the plots (matplotlib) are out of scope.
 
     python -m quantization_analysis_b200.sweep_cli <repo_or_url> <tensor_name> [--no-regex] [--metric pcc|mae|atol]
-           [--lowest-metric-val V] [--steps N] [--formats bf16,bfp8,bfp4,bfp2] [--out-dir DIR]
+           [--lowest-metric-val V] [--steps N] [--formats bf16,bfp8,bfp4,bfp2] [--out-dir DIR] [--checkpoint-dir DIR]
+
+Tensors come from ``tensor_source`` like wq's: the shards of ``--checkpoint-dir`` when given, else the float32 cache.
 """
 from __future__ import annotations
 
@@ -12,8 +14,6 @@ import re
 import sys
 import time
 from pathlib import Path
-
-import numpy as np
 
 from . import sweep, tensor_source
 from .compression_algorithms.tile_utils import MIXED_TILE_FORMATS
@@ -71,6 +71,8 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--lowest-metric-val", type=float, default=0.9)
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--out-dir", default=None)
+    ap.add_argument("--checkpoint-dir", default=None,
+                    help="Directory of *.safetensors shards to read the tensors from (the float32 cache is then not used).")
     return ap
 
 
@@ -79,7 +81,7 @@ def main(argv=None) -> int:
     formats = _parse_formats(args.formats)
     if args.backend == "ttnn":
         raise RuntimeError("TTNN backend requires `ttnn` in the active Python environment.")
-    index = tensor_source.build_tensor_index(args.repo_or_url, args.revision, args.cache_dir)
+    index = tensor_source.build_tensor_index(args.repo_or_url, args.revision, args.cache_dir, checkpoint_dir=args.checkpoint_dir)
     selected = select_tensors(index, args.tensor_name, args.regex)
     if not selected:
         print("error: no tensors matched the filter query")
@@ -94,10 +96,10 @@ def main(argv=None) -> int:
     detail = base / "details"
     detail.mkdir(parents=True, exist_ok=True)
     for name in selected:
-        xf = np.asarray(index.load_fp32(name), dtype=np.float32)
+        x = index.load(name)
         out = detail / name.replace("/", "_").replace(".", "_")
         try:
-            rows, _maps = sweep.sweep_tensor(xf, formats, args.metric, args.steps, args.lowest_metric_val)
+            rows, _maps = sweep.sweep_tensor(x, formats, args.metric, args.steps, args.lowest_metric_val)
         except sweep.SweepRangeError as exc:
             print(f"error: {exc}")
             return 1

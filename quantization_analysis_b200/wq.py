@@ -3,10 +3,13 @@ same ``results/<model>/<algorithm>/<timestamp>/`` tree - with the hot region (wq
 scoring) on the device path.  Scores are the reference's float32 numbers (qa_tensor_scores_f32), so ``table.txt`` matches
 the reference's column for column except TIME(s).
 
-Tensors come from ``tensor_source``: the reference's on-disk float32 tensor cache when it is populated for the repo, or
-the synthetic DeepSeek-R1 shapes for the pseudo-repo ``synthetic`` (no Hugging Face access in this build).
+Tensors come from ``tensor_source``: the ``*.safetensors`` shards of ``--checkpoint-dir`` when it is given (read as stored;
+block-scaled fp8 weights are scored from their bytes), else the reference's on-disk float32 tensor cache when it is
+populated for the repo, or the synthetic DeepSeek-R1 shapes for the pseudo-repo ``synthetic`` (no Hugging Face access in
+this build).
 
-    python -m quantization_analysis_b200.wq <repo_or_url> [filter ...] --compression-config cfg.json [--limit N] [--recompute] [--summary]
+    python -m quantization_analysis_b200.wq <repo_or_url> [filter ...] --compression-config cfg.json [--checkpoint-dir DIR]
+           [--limit N] [--recompute] [--summary]
 """
 from __future__ import annotations
 
@@ -111,12 +114,14 @@ def tensor_meta_str(x_dev: torch.Tensor, shape) -> str:
     return f"shape={tuple(shape)} min={float(flat.min().float()):.3e} mean={mean:.3e} max={float(flat.max().float()):.3e}"
 
 
-def evaluate_tensor(name: str, xf: np.ndarray, algorithms, formats, out_dir: Path | None, cache_ctx: CacheContext | None,
+def evaluate_tensor(name: str, x, algorithms, formats, out_dir: Path | None, cache_ctx: CacheContext | None,
                     save_processed: bool = True):
-    """The hot region of wq:679-742 for one tensor -> ({compression: [Row]}, meta line).  xf: float32 host array."""
+    """The hot region of wq:679-742 for one tensor -> ({compression: [Row]}, meta line).  x: what TensorIndex.load returns (a
+    float32 host array, a host torch tensor as stored, tensor_source.Fp8Blocks) or an engine.Prepared."""
     rows: dict[str, list[Row]] = {}
-    p = engine.prepare_tiles(xf)                                  # one H2D; bf16 on the device when the values allow it
-    meta = tensor_meta_str(p.data if p.kind != "vector" else p.data[: p.numel], xf.shape)
+    p = engine.prepare_loaded(x)                                  # one H2D; bf16 on the device when the values allow it
+    shape = p.shape
+    meta = tensor_meta_str(p.data if p.kind != "vector" else p.data[: p.numel], shape)
     x_flat = p.data
     table = None
     for algo in algorithms:
@@ -125,18 +130,18 @@ def evaluate_tensor(name: str, xf: np.ndarray, algorithms, formats, out_dir: Pat
         if algo.name in ("none", "transpose"):
             from .compression_algorithms.none import quantize_all
             from .compression_algorithms.transpose import quantize_all_transposed
-            xd = (p.data[: p.numel] if p.kind == "vector" else p.data).reshape(xf.shape)
+            xd = (p.data[: p.numel] if p.kind == "vector" else p.data).reshape(shape)
             have = {}
             if cache_ctx is not None:
                 for f in formats:
                     y = cache_ctx.load_array(algo.name, f)
-                    if y is not None and tuple(y.shape) == tuple(xf.shape):
+                    if y is not None and tuple(y.shape) == tuple(shape):
                         have[f] = torch.from_numpy(np.ascontiguousarray(y, dtype=np.float32)).to(xd.device)
             missing = [f for f in formats if f not in have]
             fresh = (quantize_all if algo.name == "none" else quantize_all_transposed)(xd, missing) if missing else {}
             if cache_ctx is not None and save_processed:
                 for f in missing:
-                    cache_ctx.save_array(algo.name, f, fresh[f].float().cpu().numpy().reshape(xf.shape))
+                    cache_ctx.save_array(algo.name, f, fresh[f].float().cpu().numpy().reshape(shape))
             torch.cuda.synchronize()
             elapsed = time.perf_counter() - t0
             for f in formats:
@@ -225,7 +230,8 @@ def _hierarchy_lines(names) -> list[str]:
 
 def build_parser() -> argparse.ArgumentParser:
     ap = argparse.ArgumentParser(prog="wq", description="Weight quantization analyzer (B200 device path).")
-    ap.add_argument("repo_or_url", help="Model repo/URL whose float32 tensor cache is used, or 'synthetic'.")
+    ap.add_argument("repo_or_url", help="Model repo/URL (names the results tree; its float32 tensor cache is the source "
+                                        "without --checkpoint-dir), or 'synthetic'.")
     ap.add_argument("filter_query", nargs="*", help="Optional filter: substring, or dotted torch-style prefix path.")
     ap.add_argument("--revision", default="main", help="Revision (default: main).")
     ap.add_argument("--cache-dir", default="data/hf-cache", help="Shared local cache for float32 tensors (default: data/hf-cache).")
@@ -239,6 +245,9 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--processed-root", default="data/processed", help="Root of the quantized-array cache (default: data/processed).")
     ap.add_argument("--no-save-processed", action="store_true", help="Do not write quantized arrays of none/transpose to disk.")
     ap.add_argument("--synthetic-seed", type=int, default=1000, help="Base seed of the synthetic tensors.")
+    ap.add_argument("--checkpoint-dir", default=None,
+                    help="Directory of *.safetensors shards (a local export or a hub snapshot) to read the tensors from; "
+                         "the float32 cache is then neither read nor written.")
     return ap
 
 
@@ -253,7 +262,8 @@ def run(argv=None) -> int:
     algorithms = [baseline] if selected.name == "none" else [baseline, selected]
     filter_query = " ".join(args.filter_query).strip() or None
     formats = resolve_format_list(config.quantization_formats, SUPPORTED_FORMATS)
-    index = tensor_source.build_tensor_index(args.repo_or_url, args.revision, args.cache_dir, args.synthetic_seed)
+    index = tensor_source.build_tensor_index(args.repo_or_url, args.revision, args.cache_dir, args.synthetic_seed,
+                                             checkpoint_dir=args.checkpoint_dir)
     names = tensor_source.resolve_selected_tensors(index, filter_query)
     if args.limit is not None:
         names = names[: max(0, args.limit)]
@@ -291,11 +301,10 @@ def run(argv=None) -> int:
     aggregate: dict[tuple[str, str], list[Row]] = {}
     table_lines: list[str] = []
     for name in names:
-        cf = index.cache_file(name)
-        print(f"cache: fp32 hit ({cf})" if cf.exists() else "cache: synthetic tensor")
-        xf = np.asarray(index.load_fp32(name), dtype=np.float32)
+        print(index.describe(name))
+        x = index.load(name)
         ctx = CacheContext(root=processed_root, tensor_name=name, backend=args.backend, recompute=args.recompute, run_tag=run_tag)
-        rows_by_comp, meta = evaluate_tensor(name, xf, algorithms, formats, results_dir, ctx, save_processed=not args.no_save_processed)
+        rows_by_comp, meta = evaluate_tensor(name, x, algorithms, formats, results_dir, ctx, save_processed=not args.no_save_processed)
         block = [name, f"  {meta}"]
         for comp in comp_names:
             rows = rows_by_comp.get(comp, [])
