@@ -127,11 +127,15 @@ def check_scale_grid(name: str, shape, grid) -> None:
                              f"ceil(shape / grid); only 2-D F32 block grids are supported")
 
 
-def _header_dtypes(path: Path) -> dict[str, str]:
-    """name -> safetensors dtype string, from the shard's header only."""
+def _header(path: Path) -> dict[str, tuple[str, tuple]]:
+    """name -> (safetensors dtype string, shape), from the shard's header only."""
     from safetensors import safe_open
+    out = {}
     with safe_open(str(path), framework="pt") as f:
-        return {k: f.get_slice(k).get_dtype() for k in f.keys()}
+        for k in f.keys():
+            sl = f.get_slice(k)
+            out[k] = (sl.get_dtype(), tuple(sl.get_shape()))
+    return out
 
 
 def _read_tensor(path: str, name: str) -> torch.Tensor:
@@ -140,14 +144,15 @@ def _read_tensor(path: str, name: str) -> torch.Tensor:
         return f.get_tensor(name)
 
 
-def scan_checkpoint(checkpoint_dir) -> tuple[dict[str, str], dict[str, str]]:
+def scan_checkpoint(checkpoint_dir) -> tuple[dict[str, str], dict[str, str], dict[str, tuple]]:
     """Index of a directory of ``*.safetensors`` shards (hf_model_utils.py:80-111): ``model.safetensors.index.json``'s
-    weight_map when present, else every shard's header.  -> ({name: shard path}, {name: stored dtype})."""
+    weight_map when present, else every shard's header.  -> ({name: shard path}, {name: stored dtype}, {name: shape})."""
     d = Path(checkpoint_dir)
     if not d.is_dir():
         raise FileNotFoundError(f"Checkpoint directory {d} does not exist")
     files: dict[str, str] = {}
     dtypes: dict[str, str] = {}
+    shapes: dict[str, tuple] = {}
     index_file = d / CHECKPOINT_INDEX
     if index_file.is_file():
         weight_map = json.loads(index_file.read_text(encoding="utf-8")).get("weight_map")
@@ -160,22 +165,22 @@ def scan_checkpoint(checkpoint_dir) -> tuple[dict[str, str], dict[str, str]]:
             path = d / shard
             if not path.is_file():
                 raise FileNotFoundError(f"{index_file.name} maps {names[0]} to {shard}, which is not in {d}")
-            header = _header_dtypes(path)
+            header = _header(path)
             for name in names:
                 if name not in header:
                     raise ValueError(f"{index_file.name} maps {name} to {shard}, which does not hold it")
-                files[name], dtypes[name] = str(path), header[name]
+                files[name], (dtypes[name], shapes[name]) = str(path), header[name]
     else:
         shards = sorted(d.glob("*.safetensors"))
         if not shards:
             raise FileNotFoundError(f"No *.safetensors shards and no {CHECKPOINT_INDEX} in {d}")
         for path in shards:
-            for name, dt in _header_dtypes(path).items():
+            for name, (dt, shape) in _header(path).items():
                 if name in files:
                     raise ValueError(f"Tensor {name} is in two shards: {Path(files[name]).name} and {path.name}")
-                files[name], dtypes[name] = str(path), dt
+                files[name], dtypes[name], shapes[name] = str(path), dt, shape
     order = sorted(files)
-    return {n: files[n] for n in order}, {n: dtypes[n] for n in order}
+    return {n: files[n] for n in order}, {n: dtypes[n] for n in order}, {n: shapes[n] for n in order}
 
 
 @dataclass
@@ -188,6 +193,7 @@ class TensorIndex:
     synthetic_seed: int = 1000
     checkpoint_dir: Path | None = None
     dtypes: dict = field(default_factory=dict)              # name -> stored safetensors dtype (checkpoint source only)
+    shapes: dict = field(default_factory=dict)              # name -> stored shape (checkpoint source only)
 
     def fp32_cache_dir(self) -> Path:
         return Path(self.cache_dir) / "tensor-fp32" / safe_repo_revision_key(self.repo_id, self.revision)
@@ -208,6 +214,16 @@ class TensorIndex:
             return f"checkpoint: {Path(self.tensor_to_file[name]).name} {self.dtypes[name]}{blocks}"
         cf = self.cache_file(name)
         return f"cache: fp32 hit ({cf})" if cf.exists() else "cache: synthetic tensor"
+
+    def shape(self, name: str) -> tuple:
+        """The shape `load(name)` returns, from headers only (safetensors header, ``.npy`` header, synthetic table): sizes a
+        tensor list without reading its data."""
+        if self.checkpoint_dir is not None:
+            return self.shapes[name]
+        src = self.tensor_to_file[name]
+        if src == "synthetic":
+            return tuple(synthetic.DEEPSEEK_R1_SHAPES[name])
+        return tuple(np.load(src, mmap_mode="r").shape)
 
     def load(self, name: str):
         """What the analysis reads for `name`: from a checkpoint the host torch tensor as stored, or `Fp8Blocks` for a
@@ -250,7 +266,7 @@ def build_tensor_index(repo_or_url: str, revision: str = "main", cache_dir="data
     idx = TensorIndex(repo_id=repo_id, revision=revision, cache_dir=Path(cache_dir), synthetic_seed=synthetic_seed)
     if checkpoint_dir is not None:
         idx.checkpoint_dir = Path(checkpoint_dir)
-        idx.tensor_to_file, idx.dtypes = scan_checkpoint(checkpoint_dir)
+        idx.tensor_to_file, idx.dtypes, idx.shapes = scan_checkpoint(checkpoint_dir)
         return idx
     d = idx.fp32_cache_dir()
     names = {}

@@ -8,14 +8,19 @@ block-scaled fp8 weights are scored from their bytes), else the reference's on-d
 populated for the repo, or the synthetic DeepSeek-R1 shapes for the pseudo-repo ``synthetic`` (no Hugging Face access in
 this build).
 
+With ``--gpus N`` the matched tensors are split over N GPUs of the node (``multi_gpu``: one worker process per GPU, tensors
+bin-packed by element count); the output is the same as one GPU's except TIME(s).
+
     python -m quantization_analysis_b200.wq <repo_or_url> [filter ...] --compression-config cfg.json [--checkpoint-dir DIR]
-           [--limit N] [--recompute] [--summary]
+           [--limit N] [--recompute] [--summary] [--gpus N]
 """
 from __future__ import annotations
 
 import argparse
+import contextlib
 import csv
 import json
+import math
 import re
 import secrets
 import sys
@@ -27,7 +32,7 @@ from pathlib import Path
 import numpy as np
 import torch
 
-from . import engine, tensor_source
+from . import engine, multi_gpu, tensor_source
 from .compression_algorithms import create_algorithm, load_compression_config
 from .compression_algorithms.cache import CacheContext
 from .compression_algorithms.tile_utils import MIXED_TILE_FORMATS
@@ -204,6 +209,40 @@ def format_block(rows: list[Row], comp: str, comp_w: int) -> list[str]:
     return lines
 
 
+@dataclass
+class TensorJob:
+    """Everything wq's per-tensor step needs besides the tensor's name; built once by `run` (after the seed is resolved) and,
+    under --gpus, pickled to every worker."""
+    index: tensor_source.TensorIndex
+    algorithms: list
+    comp_names: list[str]
+    comp_w: int
+    formats: list[str]
+    results_dir: Path
+    processed_root: Path
+    backend: str
+    recompute: bool
+    run_tag: str
+    save_processed: bool
+
+
+def run_tensor(job: TensorJob, name: str) -> tuple[str, list[str], list[Row]]:
+    """wq's per-tensor step, the same with and without --gpus: load and evaluate one tensor, write its maps and processed arrays.
+    -> (the screen line naming where it was read from, its block of screen / table.txt lines, its rows in block order)."""
+    describe = job.index.describe(name)
+    x = job.index.load(name)
+    ctx = CacheContext(root=job.processed_root, tensor_name=name, backend=job.backend, recompute=job.recompute, run_tag=job.run_tag)
+    rows_by_comp, meta = evaluate_tensor(name, x, job.algorithms, job.formats, job.results_dir, ctx, save_processed=job.save_processed)
+    block, rows = [name, f"  {meta}"], []
+    for comp in job.comp_names:
+        comp_rows = rows_by_comp.get(comp, [])
+        if not comp_rows:
+            continue
+        rows += comp_rows
+        block += format_block(comp_rows, comp, job.comp_w) + [""]
+    return describe, block, rows
+
+
 def _hierarchy_lines(names) -> list[str]:
     """Tree of the dotted tensor names with leaf counts (wq:460-546; screen only, not part of table.txt)."""
     root: dict = {}
@@ -248,11 +287,19 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--checkpoint-dir", default=None,
                     help="Directory of *.safetensors shards (a local export or a hub snapshot) to read the tensors from; "
                          "the float32 cache is then neither read nor written.")
+    ap.add_argument("--gpus", type=int, default=None,
+                    help="Split the matched tensors over N GPUs of this node (one worker process per GPU, tensors balanced by "
+                         "element count); output equals a one-GPU run's except TIME(s).  Default: this process, on the current GPU.")
     return ap
 
 
 def run(argv=None) -> int:
     args = build_parser().parse_args(argv)
+    if args.gpus is not None:
+        err = multi_gpu.gpu_count_error(args.gpus)
+        if err is not None:
+            print(f"error: {err}", file=sys.stderr)
+            return 1
     run_tag = datetime.now().strftime("%Y%m%d-%H%M%S")
     config = load_compression_config(args.compression_config)
     algo_params = dict(config.params)
@@ -298,23 +345,26 @@ def run(argv=None) -> int:
             used["seed_source"] = seed_source
     (results_dir / "compression_config.used.json").write_text(json.dumps(used, indent=2), encoding="utf-8")
     processed_root = Path(args.processed_root) / tensor_source.safe_repo_revision_key(index.repo_id, index.revision)
+    job = TensorJob(index, algorithms, comp_names, comp_w, formats, results_dir, processed_root, args.backend, args.recompute,
+                    run_tag, not args.no_save_processed)
+    if args.gpus is None:
+        results = ((name, run_tensor(job, name)) for name in names)
+    else:
+        sizes = [math.prod(index.shape(name)) for name in names]
+        results = multi_gpu.run_sharded(run_tensor, job, names, sizes, args.gpus)
     aggregate: dict[tuple[str, str], list[Row]] = {}
     table_lines: list[str] = []
-    for name in names:
-        print(index.describe(name))
-        x = index.load(name)
-        ctx = CacheContext(root=processed_root, tensor_name=name, backend=args.backend, recompute=args.recompute, run_tag=run_tag)
-        rows_by_comp, meta = evaluate_tensor(name, x, algorithms, formats, results_dir, ctx, save_processed=not args.no_save_processed)
-        block = [name, f"  {meta}"]
-        for comp in comp_names:
-            rows = rows_by_comp.get(comp, [])
-            if not rows:
-                continue
-            for r in rows:
-                aggregate.setdefault((r.compression, r.fmt), []).append(r)
-            block += format_block(rows, comp, comp_w) + [""]
-        print("\n".join(block))
-        table_lines += block
+    with contextlib.closing(results):
+        try:
+            for _name, (describe, block, rows) in results:
+                print(describe)
+                print("\n".join(block))
+                for r in rows:
+                    aggregate.setdefault((r.compression, r.fmt), []).append(r)
+                table_lines += block
+        except multi_gpu.ShardError as exc:
+            print(f"error: {exc}", file=sys.stderr)
+            return 1
     if args.summary:
         print("Summary (mean across matched tensors)")
         table_lines.append("Summary (mean across matched tensors)")
