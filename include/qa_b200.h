@@ -281,7 +281,8 @@ int qa_collective_bench(double* out, int iters, int cluster, qa_stream_t stream)
  * scores: float32[QA_NFMT][ntiles] of ONE metric; order[norder]: formats by ascending bytes;
  * a tile takes the first format whose float32 score passes (>= for pcc, <= otherwise) the
  * float32 threshold, else order[norder-1].  assignment int8[nthr][ntiles],
- * counts int64[nthr][QA_NFMT]. */
+ * counts int64[nthr][QA_NFMT].  Any nthr >= 1 that fits in int: more than 65535 thresholds are
+ * launched in ranges of 65535 on the same stream. */
 int qa_threshold_assign(const float* scores, int64_t ntiles, const int32_t* order, int norder,
                         int is_pcc, const float* thresholds, int nthr, int8_t* assignment,
                         int64_t* counts, qa_stream_t stream);
@@ -330,7 +331,10 @@ int qa_pair_sums(const float* a, const float* b, int64_t n, double* out, void* w
  *      the node count used by qa_tensor_scores_work_bytes.  The caller copies the plan to the device once per n.
  *  qa_tensor_scores_f32 - x: n elements (bf16 patterns or float32); y: nbatch arrays of n elements, y_stride elements
  *      apart (NULL = all zeros, the fp0 format); plan_dev: the plan on the device, plan_head_host: its first 4 words on
- *      the host.  out float32 [nbatch][4] = {pcc, mae, atol, mean(y)}.  work: qa_tensor_scores_work_bytes(plan[2], nbatch). */
+ *      the host.  out float32 [nbatch][4] = {pcc, mae, atol, mean(y)}.  work: qa_tensor_scores_work_bytes(plan[2], nbatch).
+ *      Any nbatch >= 1 that fits in int (and whose work buffer fits in memory): more than 65535 items are launched in
+ *      ranges of 65535 on the same stream.  x, y and y_stride may have any alignment; 32-byte aligned x, y and
+ *      y_stride * sizeof(y) select the vector loads, and from n >= 16384 on the shared-memory pipeline. */
 int64_t qa_pairwise_plan_words(int64_t n);
 int qa_pairwise_plan_build(int64_t n, int32_t* plan_host);
 int64_t qa_tensor_scores_work_bytes(int64_t plan_nnodes, int nbatch);

@@ -499,9 +499,14 @@ extern "C" int qa_threshold_assign(const float* scores, int64_t ntiles, const in
     cudaStream_t s = (cudaStream_t)stream;
     cudaMemsetAsync(counts, 0, sizeof(int64_t) * QA_NFMT * nthr, s);
     int gx = (int)min((int64_t)148 * 4, cdiv(ntiles, 256));
-    dim3 grid(gx > 0 ? gx : 1, nthr);
-    threshold_kernel<<<grid, 256, 0, s>>>(scores, ntiles, o, is_pcc, thresholds, nthr, assignment,
-                                          reinterpret_cast<unsigned long long*>(counts));
+    // one threshold per gridDim.y index, which CUDA caps at 65535: launch over threshold ranges of at most that many
+    constexpr int max_y = 65535;
+    for (int t0 = 0; t0 < nthr; t0 += max_y) {
+        const int nt = min(nthr - t0, max_y);
+        threshold_kernel<<<dim3(gx > 0 ? gx : 1, nt), 256, 0, s>>>(scores, ntiles, o, is_pcc, thresholds + t0, nt,
+                                                                  assignment + (int64_t)t0 * ntiles,
+                                                                  reinterpret_cast<unsigned long long*>(counts + (int64_t)t0 * QA_NFMT));
+    }
     return check_launch("qa_threshold_assign");
 }
 

@@ -69,8 +69,8 @@ __device__ __forceinline__ float ld_any(const void* p, int dt, int64_t i) {
 __global__ void __launch_bounds__(256) pw_leaf_kernel(const void* __restrict__ x, int xdt, const void* __restrict__ ybase, int ydt,
                                                       int64_t y_stride, int64_t nleaves, int64_t nnodes,
                                                       const int32_t* __restrict__ leaf_start8, const int32_t* __restrict__ leaf_len,
-                                                      float* __restrict__ vals, unsigned* __restrict__ maxbits) {
-    const int b = blockIdx.y;
+                                                      float* __restrict__ vals, unsigned* __restrict__ maxbits, int b0) {
+    const int b = b0 + (int)blockIdx.y;
     const char* yb = reinterpret_cast<const char*>(ybase);
     const void* y = ybase ? (const void*)(yb + (size_t)b * (size_t)y_stride * (ydt == QA_DT_BF16 ? 2 : 4)) : nullptr;
     float* v = vals + (size_t)b * 3 * nnodes;
@@ -146,8 +146,8 @@ template <int XDT, int YDT>
 __global__ void __launch_bounds__(128) pw_leaf_vec_kernel(const void* __restrict__ x, const void* __restrict__ ybase, int64_t y_stride,
                                                           int64_t nleaves, int64_t nnodes, const int32_t* __restrict__ leaf_start8,
                                                           const int32_t* __restrict__ leaf_len, float* __restrict__ vals,
-                                                          unsigned* __restrict__ maxbits) {
-    const int b = blockIdx.y;
+                                                          unsigned* __restrict__ maxbits, int b0) {
+    const int b = b0 + (int)blockIdx.y;
     const void* y = YDT == 2 ? nullptr
                              : (const void*)(reinterpret_cast<const char*>(ybase) + (size_t)b * (size_t)y_stride * (YDT == QA_DT_BF16 ? 2 : 4));
     float* v = vals + (size_t)b * 3 * nnodes;
@@ -211,9 +211,10 @@ __global__ void __launch_bounds__(1024) pw_tree_kernel(int64_t nleaves, int64_t 
 // ---- sdot chains: block = 64 threads = the 64 accumulators of one dot product ------------------------------
 template <int XDT, int YDT>
 __global__ void __launch_bounds__(64) sdot_kernel(const void* __restrict__ x, const void* __restrict__ ybase, int64_t y_stride,
-                                                  int64_t n, int64_t nnodes, const float* __restrict__ vals, float* __restrict__ dots) {
+                                                  int64_t n, int64_t nnodes, const float* __restrict__ vals, float* __restrict__ dots,
+                                                  int b0) {
     const int kind = blockIdx.x;     // 0: (am, am)  1: (bm, bm)  2: (am, bm)
-    const int b = blockIdx.y;
+    const int b = b0 + (int)blockIdx.y;
     if (kind == 0 && b > 0) return;  // x is shared by the batch
     const void* y = ybase ? (const void*)(reinterpret_cast<const char*>(ybase) + (size_t)b * (size_t)y_stride * (YDT == QA_DT_BF16 ? 2 : 4))
                           : nullptr;
@@ -335,11 +336,11 @@ __device__ __forceinline__ float sd_stage(const unsigned char* su, const unsigne
 template <int XDT, int YDT>      // YDT == 2: y is all zeros (never loaded)
 __global__ void __launch_bounds__(64, 1) sdot_pipe_kernel(const void* __restrict__ x, const void* __restrict__ ybase, int64_t y_stride, int64_t n,
                                                        int64_t nnodes, int nstages, const float* __restrict__ vals,
-                                                       float* __restrict__ dots) {
+                                                       float* __restrict__ dots, int b0) {
     extern __shared__ __align__(128) unsigned char sd_smem[];
     __shared__ __align__(8) unsigned long long full[SD_MAX_STAGES];
     const int kind = blockIdx.x;     // 0: (am, am)  1: (bm, bm)  2: (am, bm)
-    const int b = blockIdx.y;
+    const int b = b0 + (int)blockIdx.y;
     if (kind == 0 && b > 0) return;  // x is shared by the batch
     constexpr int XB = XDT == QA_DT_BF16 ? 2 : 4, YB = YDT == QA_DT_BF16 ? 2 : 4;
     constexpr bool HAVE_Y = YDT != 2;
@@ -437,7 +438,7 @@ __global__ void __launch_bounds__(64, 1) sdot_pipe_kernel(const void* __restrict
 
 __global__ void scores_final_kernel(int nbatch, int64_t n, int64_t nnodes, const float* __restrict__ vals, const float* __restrict__ dots,
                                     const unsigned* __restrict__ maxbits, float* __restrict__ out) {
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= nbatch) return;
     const float amax = __uint_as_float(maxbits[b]);
     const float na = __fsqrt_rn(dots[0]), nb = __fsqrt_rn(dots[(size_t)b * 4 + 1]);
@@ -445,10 +446,10 @@ __global__ void scores_final_kernel(int nbatch, int64_t n, int64_t nnodes, const
     float pcc;
     if (denom == 0.f) pcc = (amax == 0.f) ? 1.f : 0.f;
     else pcc = __fdiv_rn(dots[(size_t)b * 4 + 2], denom);
-    out[b * 4 + 0] = pcc;
-    out[b * 4 + 1] = __fdiv_rn(vals[(size_t)b * 3 * nnodes + 2 * nnodes + nnodes - 1], (float)n);
-    out[b * 4 + 2] = amax;
-    out[b * 4 + 3] = __fdiv_rn(vals[(size_t)b * 3 * nnodes + nnodes + nnodes - 1], (float)n);   // mean(b), for reference
+    out[(size_t)b * 4 + 0] = pcc;
+    out[(size_t)b * 4 + 1] = __fdiv_rn(vals[(size_t)b * 3 * nnodes + 2 * nnodes + nnodes - 1], (float)n);
+    out[(size_t)b * 4 + 2] = amax;
+    out[(size_t)b * 4 + 3] = __fdiv_rn(vals[(size_t)b * 3 * nnodes + nnodes + nnodes - 1], (float)n);   // mean(b), for reference
 }
 
 }  // namespace qa
@@ -528,24 +529,30 @@ extern "C" int qa_tensor_scores_f32(const void* x, int x_dtype, const void* y, i
     const size_t ybytes = y_dtype == QA_DT_BF16 ? 2 : 4;
     const bool aligned = reinterpret_cast<uintptr_t>(x) % 32 == 0 &&
                          (!y || (reinterpret_cast<uintptr_t>(y) % 32 == 0 && ((size_t)y_stride * ybytes) % 32 == 0));
+    // The leaf and chain kernels put the batch on gridDim.y, which CUDA caps at 65535: they are launched over batch ranges
+    // [b0, b0 + nb) of at most that many items.  pw_tree_kernel and scores_final_kernel put the batch on gridDim.x.
+    constexpr int max_y = 65535;
+    const int yk = y ? y_dtype : 2;
     if (aligned) {
-        const dim3 gv((unsigned)std::max<int64_t>(1, std::min<int64_t>(cdiv(nl, 128), 148 * 16)), nbatch);
-        const int yk = y ? y_dtype : 2;
-#define QA_LEAF(XD, YD) pw_leaf_vec_kernel<XD, YD><<<gv, 128, 0, s>>>(x, y, y_stride, nl, nnodes, ls, ll, vals, maxbits)
-        if (x_dtype == QA_DT_BF16) { if (yk == QA_DT_BF16) QA_LEAF(QA_DT_BF16, QA_DT_BF16); else if (yk == QA_DT_F32) QA_LEAF(QA_DT_BF16, QA_DT_F32); else QA_LEAF(QA_DT_BF16, 2); }
-        else { if (yk == QA_DT_BF16) QA_LEAF(QA_DT_F32, QA_DT_BF16); else if (yk == QA_DT_F32) QA_LEAF(QA_DT_F32, QA_DT_F32); else QA_LEAF(QA_DT_F32, 2); }
+        const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>(cdiv(nl, 128), 148 * 16));
+        for (int b0 = 0; b0 < nbatch; b0 += max_y) {
+            const dim3 gv(gx, std::min(nbatch - b0, max_y));
+#define QA_LEAF(XD, YD) pw_leaf_vec_kernel<XD, YD><<<gv, 128, 0, s>>>(x, y, y_stride, nl, nnodes, ls, ll, vals, maxbits, b0)
+            if (x_dtype == QA_DT_BF16) { if (yk == QA_DT_BF16) QA_LEAF(QA_DT_BF16, QA_DT_BF16); else if (yk == QA_DT_F32) QA_LEAF(QA_DT_BF16, QA_DT_F32); else QA_LEAF(QA_DT_BF16, 2); }
+            else { if (yk == QA_DT_BF16) QA_LEAF(QA_DT_F32, QA_DT_BF16); else if (yk == QA_DT_F32) QA_LEAF(QA_DT_F32, QA_DT_F32); else QA_LEAF(QA_DT_F32, 2); }
 #undef QA_LEAF
+        }
     } else {
         const int64_t warps_needed = cdiv(nl, 4);
         const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>(cdiv(warps_needed, 8), 148 * 8));
-        pw_leaf_kernel<<<dim3(gx, nbatch), 256, 0, s>>>(x, x_dtype, y, y_dtype, y_stride, nl, nnodes, ls, ll, vals, maxbits);
+        for (int b0 = 0; b0 < nbatch; b0 += max_y)
+            pw_leaf_kernel<<<dim3(gx, std::min(nbatch - b0, max_y)), 256, 0, s>>>(x, x_dtype, y, y_dtype, y_stride, nl, nnodes, ls, ll,
+                                                                                  vals, maxbits, b0);
     }
     if (lv) pw_tree_kernel<<<nbatch, 1024, 0, s>>>(nl, nnodes, lv, loff, lf, rt, vals);
-    const dim3 g(3, nbatch);
     const int ydt = y ? y_dtype : QA_DT_F32;
     if (aligned && n >= 4 * (int64_t)SD_TE) {
         // pipelined chains: shared-memory ring of 4096-element stages
-        const int yk = y ? y_dtype : 2;
         const int stage_bytes = SD_TE * ((x_dtype == QA_DT_BF16 ? 2 : 4) + (yk == 2 ? 0 : (yk == QA_DT_BF16 ? 2 : 4)));
         // one dot product alone wants a deep ring (latency); a batch larger than the GPU wants many CTAs per SM instead - a lone
         // warp per sub-partition issues at half rate - so the ring shrinks to what lets 4 - 7 CTAs share an SM's shared memory
@@ -557,15 +564,21 @@ extern "C" int qa_tensor_scores_f32(const void* x, int x_dtype, const void* y, i
     do {                                                                                                             \
         if (cudaFuncSetAttribute(sdot_pipe_kernel<XD, YD>, cudaFuncAttributeMaxDynamicSharedMemorySize, 196608) != cudaSuccess) \
             return check_launch("qa_tensor_scores_f32 (shared memory attribute)");                                   \
-        sdot_pipe_kernel<XD, YD><<<g, 64, dyn, s>>>(x, y, y_stride, n, nnodes, nst, vals, dots);                      \
+        for (int b0 = 0; b0 < nbatch; b0 += max_y)                                                                   \
+            sdot_pipe_kernel<XD, YD><<<dim3(3, std::min(nbatch - b0, max_y)), 64, dyn, s>>>(x, y, y_stride, n, nnodes, nst, vals, dots, b0); \
     } while (0)
         if (x_dtype == QA_DT_BF16) { if (yk == QA_DT_BF16) QA_SDOT(QA_DT_BF16, QA_DT_BF16); else if (yk == QA_DT_F32) QA_SDOT(QA_DT_BF16, QA_DT_F32); else QA_SDOT(QA_DT_BF16, 2); }
         else { if (yk == QA_DT_BF16) QA_SDOT(QA_DT_F32, QA_DT_BF16); else if (yk == QA_DT_F32) QA_SDOT(QA_DT_F32, QA_DT_F32); else QA_SDOT(QA_DT_F32, 2); }
 #undef QA_SDOT
-    } else if (x_dtype == QA_DT_BF16 && ydt == QA_DT_BF16) sdot_kernel<QA_DT_BF16, QA_DT_BF16><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots);
-    else if (x_dtype == QA_DT_BF16) sdot_kernel<QA_DT_BF16, QA_DT_F32><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots);
-    else if (ydt == QA_DT_BF16) sdot_kernel<QA_DT_F32, QA_DT_BF16><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots);
-    else sdot_kernel<QA_DT_F32, QA_DT_F32><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots);
-    scores_final_kernel<<<(nbatch + 127) / 128, 128, 0, s>>>(nbatch, n, nnodes, vals, dots, maxbits, out);
+    } else {
+        for (int b0 = 0; b0 < nbatch; b0 += max_y) {
+            const dim3 g(3, std::min(nbatch - b0, max_y));
+            if (x_dtype == QA_DT_BF16 && ydt == QA_DT_BF16) sdot_kernel<QA_DT_BF16, QA_DT_BF16><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots, b0);
+            else if (x_dtype == QA_DT_BF16) sdot_kernel<QA_DT_BF16, QA_DT_F32><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots, b0);
+            else if (ydt == QA_DT_BF16) sdot_kernel<QA_DT_F32, QA_DT_BF16><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots, b0);
+            else sdot_kernel<QA_DT_F32, QA_DT_F32><<<g, 64, 0, s>>>(x, y, y_stride, n, nnodes, vals, dots, b0);
+        }
+    }
+    scores_final_kernel<<<(unsigned)cdiv((int64_t)nbatch, 128), 128, 0, s>>>(nbatch, n, nnodes, vals, dots, maxbits, out);
     return check_launch("qa_tensor_scores_f32");
 }
