@@ -92,6 +92,10 @@ int qa_fp8_block_dequant(const void* w_fp8, const float* scale_inv, int64_t rows
  * metrics of wq:684-687 / mixed_tile_random.py:135-141.  vec_tail: 0, or for a 1-D input laid
  * out as rows of 32 (tile_utils.py:96-102) the number of valid elements in the last row (strict
  * mode sums that ragged row as its own view, mixed_tile_greedy.py:111-131).
+ * QA_STATS_STRICT is bit-equal to the reference's NumPy-order sums.  The fast modes (bf16 input) match them bit for bit in
+ * every column whose sum is exactly representable, except sum x^2 (and the bf16 slot's sum y^2 and sum x*y, which are it):
+ * <= 1e-13 relative per tile for any finite input.  Groups whose largest |x| is below 2^-51 or at least 2^64 are summed from
+ * float32 products like the reference's, so denormal-only groups count and overflowing products give the reference's inf.
  * Only the columns of formats in fmt_mask (and SX/SX2) are written. */
 int qa_tile_stats(const void* x, int x_dtype, int64_t rows, int64_t cols, int64_t ld,
                   int64_t vec_tail, uint32_t fmt_mask, int mode, double* table,
@@ -138,7 +142,9 @@ int qa_greedy_init_deltas_batch(const qa_batch_desc* descs_dev, int n, int64_t t
  * and mixed_tile_greedy.py:147-174 (float32 product arrays x*x, x*y, y*y summed in float64).  sum y, sum y^2, sum |x-y| and
  * max |x-y| equal the reference's NumPy-order float64 sums whenever those are exactly representable; sum x, sum x^2 and
  * sum x*y of 24-bit data are order-dependent in the last float64 bits (<= 1e-13 relative per tile) - the greedy's decision-margin
- * certificate (state[20]) covers that, as for the bf16 kernel's sum x^2.  mode: QA_STATS_FAST or QA_STATS_FAST_APPROX_ABS.
+ * certificate (state[20]) covers that, as for the bf16 kernel's sum x^2.  So is the bf16 slot's sum y^2, whose squares are exact
+ * where the reference rounds those below 2^-134 in float32's denormal range.  Groups whose largest |x| is below 2^-51 or at least
+ * 2^63 are summed from float32 products throughout, so squares in the denormal range and overflow to inf follow the reference.  mode: QA_STATS_FAST or QA_STATS_FAST_APPROX_ABS.
  * Tile rows [tile_row_begin, tile_row_end) are produced (tile_row_end < 0: all), so a large table can be made in pieces. */
 int qa_tile_stats_f32(const float* x, int64_t rows, int64_t cols, int64_t ld, uint32_t fmt_mask, int mode, double* table,
                       int64_t tile_row_begin, int64_t tile_row_end, qa_stream_t stream);

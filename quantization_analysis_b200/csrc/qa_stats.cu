@@ -58,6 +58,13 @@ __device__ __noinline__ void group_slow(const uint32_t (&w)[8], uint32_t E, Tile
             a.amax[f] = fmaxf(a.amax[f], r);
         }
     }
+    // 191 <= E < 255: the group's largest |x| is at least 2^64 and its reconstruction in every format has the same sign and
+    // at least the magnitude 2^(E-127), so that float32 x*y is +inf (as are x*x and y*y).  Every other x*y is >= 0, so the
+    // reference's sum x*y is +inf; the difference above would be inf - inf.
+    if (E - 191u < 64u) {
+#pragma unroll
+        for (int f = 0; f < 3; ++f) a.sxy[f] = __longlong_as_double(0x7FF0000000000000LL);
+    }
 }
 
 template <int F>
@@ -139,12 +146,14 @@ __device__ __forceinline__ void group_fast(const uint32_t (&w)[8], TileAcc& a) {
         mabs = max3abs(mabs, xv[i].x, xv[i].y);
     }
     const uint32_t E = __float_as_uint(mabs) >> 23;
-    if (E == 0u) return;                         // every element is zero/denormal: flushed (x ~ 0)
-    // E < 72: squares of the group's elements fall into float32's denormal range, where the reference's float32
-    // products (x*x, y*y, x*y as float32 arrays) round or flush; E == 255: inf/nan.  Both take the generic path,
-    // which forms float32 products like the reference.  (An element below 2^-63 inside a group whose maximum is
-    // above 2^-55 still contributes its exact square here instead of a denormal-rounded one: < 2^-40 relative.)
-    if (E < 72u || E == 255u) {
+    // The generic path forms float32 products like the reference (x*x, y*y, x*y as float32 arrays); it takes
+    //   E < 76: zeros and denormals only (E == 0: each counts in sum x and, unquantized, in sum |x-y| and max |x-y|), or
+    //     squares that round or flush in float32's denormal range by more than the 1e-13 the table promises.  Below
+    //     here an element's fast square is exact where the reference's is rounded to a multiple of 2^-149: off by at
+    //     most 2^-150, 2^-146 per group, against a group sum x^2 of at least 2^(2E-254): <= 2^(108-2E) = 2^-44 at E = 76;
+    //   E >= 191: |x| >= 2^64, where x*x, y*y and x*y overflow to inf in float32 (group_slow records sum x*y = +inf);
+    //   E == 255: inf / nan.
+    if (E < 76u || E >= 191u) {
         // rare: keep the caller's accumulators in registers by handing the slow path its own copy
         TileAcc t;
         acc_zero(t);

@@ -14,7 +14,8 @@
 //     exact-abs mode, float32 group partials otherwise).
 // Every sum equals the reference's NumPy-order float64 sum whenever that sum is exactly representable (the normal case); a tile
 // that spans more octaves than float64 holds can differ in the last bits of sum x, sum x^2, sum |x-y| (<= 1e-13 relative), like
-// the bf16 kernel's sum x^2.  Groups with E < 72 or E = 255 (inf / nan) use the integer recipe and float32 products directly.
+// the bf16 kernel's sum x^2.  Groups with E < 76 or E >= 190 (|x| near or past 2^64, inf / nan) use the integer recipe and
+// float32 products directly.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_fp8.h>
@@ -122,7 +123,10 @@ __device__ __forceinline__ void groupf_fast(const uint32_t (&u)[GROUP], TileAccF
 #pragma unroll
     for (int i = 0; i < GROUP; i += 2) mabs = max3absf(mabs, __uint_as_float(u[i]), __uint_as_float(u[i + 1]));   // a nan surfaces: E = 255
     const uint32_t E = __float_as_uint(mabs) >> 23;
-    if (E < 72u || E == 255u) {
+    // generic path (float32 products like the reference) for E < 76: the bf16 slot's sum y^2 is exact below here where the
+    // reference rounds y*y in float32's denormal range (the bound of qa_stats.cu's group_fast); E >= 190: the bf16 image
+    // of |x| >= 2^64 - 2^55 is 2^64, and y*y (and from E = 191 every product) overflows to inf; E == 255: inf / nan
+    if (E < 76u || E >= 190u) {
         if (E == 0u) {                     // zeros / denormals only: every format flushes them; they still count in sum x
 #pragma unroll
             for (int i = 0; i < GROUP; ++i) {
