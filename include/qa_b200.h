@@ -264,6 +264,22 @@ int qa_greedy_assign_passes(const double* table, int64_t ntiles, double numel, i
  * sums are unaffected. */
 #define QA_GREEDY_SKIP_FINAL_STREAM 1
 
+/* Greedy sweep: the chains of nthr thresholds over ONE table in one launch - what a bytes-versus-metric curve of the greedy
+ * needs.  Every chain is the whole run (passes [0, nfmt)) of qa_greedy_assign_passes with thresholds[k] and gives its
+ * results bit for bit; the table, the init and the prefetched permutations are shared and only read.
+ *  pcc / mae: a grid of nthr clusters (the cluster size qa_greedy_assign_passes would pick, under qa_greedy_cluster_cap);
+ *      clusters beyond what fits on the GPU at once queue.  init == NULL: computed once, ahead of the chains, on `stream`;
+ *      pre_order / pre_rng == NULL: every chain draws its own permutations.
+ *  atol: the one-thread chain of qa_greedy_assign, one block per threshold; pre_order, pre_rng and init are not used.
+ * thresholds: DEVICE double[nthr]; rng: DEVICE, the stream state every chain starts from (not modified).
+ * Outputs: assignment int8[nthr][ntiles], counts int64[nthr][QA_NFMT], state double[nthr][24] (the atol chain writes
+ * state[0..7] only).  work: nthr * qa_greedy_sweep_work_bytes(ntiles, metric) bytes (-1: bad arguments).  flags as above. */
+int64_t qa_greedy_sweep_work_bytes(int64_t ntiles, int metric);
+int qa_greedy_assign_sweep(const double* table, int64_t ntiles, double numel, int metric, const double* thresholds, int nthr,
+                           const int32_t* fmt_order, int nfmt, const qa_pcg64* rng, int8_t* assignment, int64_t* counts,
+                           double* state, void* work, const int32_t* pre_order, const qa_pcg64* pre_rng, const void* init,
+                           int flags, qa_stream_t stream);
+
 /* Upper bound on the thread-block cluster size of the greedy kernels (1, 2, 4, 8, 16; 0 = automatic: large tensors get
  * 16 CTAs for latency).  A caller with many tensors in flight trades per-tensor latency for SM time with a smaller
  * cluster; results do not depend on the cluster size.  The setting belongs to the CALLING THREAD (thread-local): it

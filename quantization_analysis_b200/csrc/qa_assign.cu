@@ -84,10 +84,10 @@ __device__ __forceinline__ bool good(double v, int metric, double thr) {
     return metric == QA_METRIC_PCC ? v >= thr : v <= thr;
 }
 
-__global__ void greedy_seq_kernel(const double* __restrict__ table, int64_t nt, double numel, int metric,
-                                  double thr, OrderArg ord, qa_pcg64* rng,
-                                  int8_t* assignment, int64_t* counts, double* state, GreedyWork w) {
-    if (blockIdx.x || threadIdx.x) return;
+// The stream starts at *rng_in and its final position goes to *rng_out (the same pointer for a single run).
+__device__ __forceinline__ void greedy_seq(const double* __restrict__ table, int64_t nt, double numel, int metric, double thr,
+                                           OrderArg ord, const qa_pcg64* rng_in, qa_pcg64* rng_out, int8_t* assignment,
+                                           int64_t* counts, double* state, GreedyWork w) {
     const int nfmt = ord.n;
     const int base = ord.fmt[0];
     int64_t cnt[QA_NFMT] = {0, 0, 0, 0};
@@ -120,7 +120,7 @@ __global__ void greedy_seq_kernel(const double* __restrict__ table, int64_t nt, 
         }
     }
     Pcg g;
-    g.load(rng);
+    g.load(rng_in);
     for (int fi = 0; fi < nfmt; ++fi) {
         const int fmt = ord.fmt[fi];
         int64_t m = 0;
@@ -189,12 +189,31 @@ __global__ void greedy_seq_kernel(const double* __restrict__ table, int64_t nt, 
             }
         }
     }
-    g.store(rng);
+    g.store(rng_out);
     for (int f = 0; f < QA_NFMT; ++f) counts[f] = cnt[f];
     state[0] = sx; state[1] = sx2; state[2] = sy; state[3] = sy2; state[4] = sxy; state[5] = sabs;
     state[6] = max_abs;
     state[7] = metric == QA_METRIC_PCC ? pcc_value(numel, sx, sx2, sy, sy2, sxy, sabs)
              : metric == QA_METRIC_MAE ? (numel != 0.0 ? __ddiv_rn(sabs, numel) : 0.0) : max_abs;
+}
+
+__global__ void greedy_seq_kernel(const double* __restrict__ table, int64_t nt, double numel, int metric,
+                                  double thr, OrderArg ord, qa_pcg64* rng,
+                                  int8_t* assignment, int64_t* counts, double* state, GreedyWork w) {
+    if (blockIdx.x || threadIdx.x) return;
+    greedy_seq(table, nt, numel, metric, thr, ord, rng, rng, assignment, counts, state, w);
+}
+
+// atol sweep: block k runs the chain with thresholds[k] on its own slice of the work (`stride` bytes per block) and outputs
+__global__ void greedy_seq_sweep_kernel(const double* __restrict__ table, int64_t nt, double numel, const double* __restrict__ thresholds,
+                                        OrderArg ord, const qa_pcg64* rng, qa_pcg64* rng_out, int8_t* assignment, int64_t* counts,
+                                        double* state, GreedyWork w, int64_t stride) {
+    if (threadIdx.x) return;
+    const int64_t k = blockIdx.x, off = k * stride;
+    auto mine = [off](auto* p) { return reinterpret_cast<decltype(p)>(reinterpret_cast<char*>(p) + off); };
+    w.perm = mine(w.perm); w.cand = mine(w.cand); w.fixed = mine(w.fixed);
+    greedy_seq(table, nt, numel, QA_METRIC_ATOL, thresholds[k], ord, rng, mine(rng_out), assignment + k * nt, counts + k * QA_NFMT,
+               state + k * 24, w);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -456,6 +475,15 @@ extern "C" int qa_numpy_integers(qa_pcg64* rng, int k, int64_t n, int8_t* out_va
 
 static inline int64_t align_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 
+static GreedyWork carve_seq(void* work, int64_t ntiles) {
+    GreedyWork w;
+    char* p = reinterpret_cast<char*>(work);
+    w.perm = reinterpret_cast<int32_t*>(p); p += align_up(ntiles * 4, 256);
+    w.cand = reinterpret_cast<int32_t*>(p); p += align_up(ntiles * 4, 256);
+    w.fixed = reinterpret_cast<uint8_t*>(p);
+    return w;
+}
+
 extern "C" int64_t qa_greedy_work_bytes(int64_t ntiles) {
     return align_up(ntiles * 4, 256) * 2 + align_up(ntiles, 256) + 256;
 }
@@ -474,14 +502,20 @@ extern "C" int qa_greedy_assign(const double* table, int64_t ntiles, double nume
     for (int i = 0; i < QA_NFMT; ++i) ord.fmt[i] = i < nfmt ? fmt_order[i] : 0;  // HOST array
     for (int i = 0; i < nfmt; ++i)
         if (ord.fmt[i] < 0 || ord.fmt[i] >= QA_NFMT) { set_error("qa_greedy_assign: bad format index"); return 1; }
-    GreedyWork w;
-    char* p = reinterpret_cast<char*>(work);
-    w.perm = reinterpret_cast<int32_t*>(p); p += align_up(ntiles * 4, 256);
-    w.cand = reinterpret_cast<int32_t*>(p); p += align_up(ntiles * 4, 256);
-    w.fixed = reinterpret_cast<uint8_t*>(p);
     greedy_seq_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(table, ntiles, numel, metric, threshold, ord, rng,
-                                                          assignment, counts, state, w);
+                                                          assignment, counts, state, carve_seq(work, ntiles));
     return check_launch("qa_greedy_assign");
+}
+
+int qa::greedy_seq_sweep_launch(const double* table, int64_t ntiles, double numel, const double* thresholds, int nthr,
+                                const int32_t* fmt_order, int nfmt, const qa_pcg64* rng, qa_pcg64* rng_out, int8_t* assignment,
+                                int64_t* counts, double* state, void* work, int64_t stride, cudaStream_t stream) {
+    OrderArg ord;       // fmt_order: checked by the caller
+    ord.n = nfmt;
+    for (int i = 0; i < QA_NFMT; ++i) ord.fmt[i] = i < nfmt ? fmt_order[i] : 0;
+    greedy_seq_sweep_kernel<<<(unsigned)nthr, 32, 0, stream>>>(table, ntiles, numel, thresholds, ord, rng, rng_out, assignment, counts,
+                                                               state, carve_seq(work, ntiles), stride);
+    return check_launch("qa_greedy_assign_sweep");
 }
 
 extern "C" int qa_threshold_assign(const float* scores, int64_t ntiles, const int32_t* order, int norder,

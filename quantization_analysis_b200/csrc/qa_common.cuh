@@ -13,6 +13,12 @@ constexpr int GROUP = 16;
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);
 
+// qa_greedy_assign_sweep for atol (qa_assign.cu): the one-thread chain, one block per threshold.  Block k's scratch and
+// end-of-stream slot lie k * stride bytes after work / rng_out; every chain starts from *rng.
+int greedy_seq_sweep_launch(const double* table, int64_t ntiles, double numel, const double* thresholds, int nthr,
+                            const int32_t* fmt_order, int nfmt, const qa_pcg64* rng, qa_pcg64* rng_out, int8_t* assignment,
+                            int64_t* counts, double* state, void* work, int64_t stride, cudaStream_t stream);
+
 __host__ __device__ inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 // ---------------------------------------------------------------------------------------

@@ -1378,11 +1378,12 @@ __global__ void __launch_bounds__(256) greedy_delta_batch_kernel(const qa_batch_
 #else
 #define QA_CHAIN_REGCAP __launch_bounds__(GT, 1)
 #endif
+// The chain body, shared by the single-run kernel and the sweep kernel.  The stream starts at *rng_in; its final position goes
+// to *rng_out (the same pointer for a single run; a private slot for a sweep chain, whose starting state is shared).
 template <bool PCC>
-__global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ table, int nt, double numel, int metric,
-                                                        double thr, ParOrder ord, qa_pcg64* rng, int8_t* assignment,
-                                                        int64_t* counts, double* state, ParWork w, int fi_begin, int fi_end,
-                                                        int flags) {
+__device__ __forceinline__ void greedy_chain(const double* __restrict__ table, int nt, double numel, int metric, double thr,
+                                             ParOrder ord, const qa_pcg64* rng_in, qa_pcg64* rng_out, int8_t* assignment,
+                                             int64_t* counts, double* state, ParWork w, int fi_begin, int fi_end, int flags) {
     // Passes [fi_begin, fi_end) of the format order.  A run may be split into several launches (so that a later pass can
     // wait for a prefetched permutation that an earlier one does not need); the running state travels in w.res.  The
     // initial sums and delta records (w.hdr, w.delta) were written ahead of the chain by greedy_init_kernel and a delta kernel.
@@ -1404,7 +1405,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
     }
     if (tid < QA_NFMT) sh.cnt[tid] = 0;
     Pcg g;
-    g.load(rng);
+    g.load(rng_in);
     c.sync();
     const long long t_start = clock64();
 
@@ -1749,7 +1750,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
         if (tid < QA_NFMT && sh.cnt[tid] != 0)
             atomicAdd(reinterpret_cast<unsigned long long*>(&counts[tid]), (unsigned long long)(long long)sh.cnt[tid]);
         if (c.gtid == 0) {
-            g.store(rng);
+            g.store(rng_out);
             double* r = w.res;
             r[0] = S[0]; r[1] = S[1]; r[2] = S[2]; r[3] = S[3];
             r[4] = (double)degraded; r[5] = (double)chain_rounds;
@@ -1769,7 +1770,7 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
     if (tid < QA_NFMT && sh.cnt[tid] != 0)
         atomicAdd(reinterpret_cast<unsigned long long*>(&counts[tid]), (unsigned long long)(long long)sh.cnt[tid]);
     if (c.gtid == 0) {
-        g.store(rng);
+        g.store(rng_out);
         state[0] = k.sx; state[1] = k.sx2; state[2] = S[0]; state[3] = S[1]; state[4] = S[2]; state[5] = S[3];
         state[6] = (double)degraded + 65536.0 * (double)chain_rounds;
         state[7] = is_pcc ? pcc_value_par(k, S[0], S[1], S[2], S[3]) : (numel != 0.0 ? __ddiv_rn(S[3], numel) : 0.0);
@@ -1786,6 +1787,33 @@ __global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ tab
         state[21] = (double)c.cy_resolve; state[22] = (double)c.cy_apply; state[23] = (double)c.n_sweeps + 65536.0 * c.n_rounds;
         stamp(first ? 5 : 7, true);
     }
+}
+
+template <bool PCC>
+__global__ void QA_CHAIN_REGCAP greedy_par_kernel(const double* __restrict__ table, int nt, double numel, int metric,
+                                                        double thr, ParOrder ord, qa_pcg64* rng, int8_t* assignment,
+                                                        int64_t* counts, double* state, ParWork w, int fi_begin, int fi_end,
+                                                        int flags) {
+    greedy_chain<PCC>(table, nt, numel, metric, thr, ord, rng, rng, assignment, counts, state, w, fi_begin, fi_end, flags);
+}
+
+// Sweep: cluster k runs the whole chain (passes [0, nfmt)) with thresholds[k].  Every cluster reads the one table, init
+// (w.hdr / w.delta) and prefetched permutations (w.pre_order / w.pre_rng); its private buffers - the chain's scratch in w,
+// its map, counts, state and the slot its stream ends in - lie `stride` bytes (work) or one row (outputs) per cluster apart,
+// starting from cluster 0's.  The CTA rank inside the cluster comes from the cluster (Coop), never from blockIdx.
+template <bool PCC>
+__global__ void QA_CHAIN_REGCAP greedy_sweep_kernel(const double* __restrict__ table, int nt, double numel, int metric,
+                                                          const double* __restrict__ thresholds, ParOrder ord, const qa_pcg64* rng,
+                                                          qa_pcg64* rng_out, int8_t* assignment, int64_t* counts, double* state,
+                                                          ParWork w, int64_t stride, int flags) {
+    unsigned k;
+    asm("mov.u32 %0, %%clusterid.x;" : "=r"(k));
+    const int64_t off = (int64_t)k * stride;
+    auto mine = [off](auto* p) { return reinterpret_cast<decltype(p)>(reinterpret_cast<char*>(p) + off); };
+    w.order = mine(w.order); w.cand = mine(w.cand); w.jarr = mine(w.jarr); w.off = mine(w.off); w.cursor = mine(w.cursor);
+    w.bucket = mine(w.bucket); w.succ = mine(w.succ); w.parent = mine(w.parent); w.res = mine(w.res); w.fixed = mine(w.fixed);
+    greedy_chain<PCC>(table, nt, numel, metric, thresholds[k], ord, rng, mine(rng_out), assignment + (int64_t)k * nt,
+                      counts + (int64_t)k * QA_NFMT, state + (int64_t)k * 24, w, 0, ord.n, flags);
 }
 
 // micro-benchmark of the collectives (cycles per call), for DESIGN.md / tuning
@@ -1846,8 +1874,10 @@ static int pick_cluster(int64_t n) {
     return g_cluster_cap > 0 && r > g_cluster_cap ? g_cluster_cap : r;
 }
 
+// A grid of `nclusters` clusters of nr CTAs.  A grid with more clusters than can be resident at once queues: the probe below
+// only asks whether one cluster of 16 fits.
 template <typename... KArgs, typename... Args>
-static int launch_cluster_dyn(int dyn, void (*kern)(KArgs...), int nr, cudaStream_t s, Args... args) {
+static int launch_cluster_dyn(int dyn, void (*kern)(KArgs...), int nr, int nclusters, cudaStream_t s, Args... args) {
     {   // attributes are set once per kernel (not a stream operation: keep it out of the per-launch path and of graph
         // captures); the same moment asks the occupancy calculator whether a 16-CTA cluster can be resident at all, so that
         // no launch ever has to fail and be retried (a failed launch would invalidate a stream capture)
@@ -1881,7 +1911,7 @@ static int launch_cluster_dyn(int dyn, void (*kern)(KArgs...), int nr, cudaStrea
         if (idx >= 0 && nr > 8 && !ok16[idx]) nr = 8;
     }
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(nr, 1, 1);
+    cfg.gridDim = dim3((unsigned)(nr * nclusters), 1, 1);
     cfg.blockDim = dim3(GT, 1, 1);
     cfg.dynamicSmemBytes = dyn;
     cfg.stream = s;
@@ -1894,7 +1924,7 @@ static int launch_cluster_dyn(int dyn, void (*kern)(KArgs...), int nr, cudaStrea
     cfg.numAttrs = 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
     if (e != cudaSuccess) {
-        set_error("cluster launch (%d CTAs): %s", nr, cudaGetErrorString(e));
+        set_error("cluster launch (%d x %d CTAs): %s", nclusters, nr, cudaGetErrorString(e));
         return 2;
     }
     return 0;
@@ -1904,11 +1934,15 @@ static int launch_cluster_dyn(int dyn, void (*kern)(KArgs...), int nr, cudaStrea
 // a smaller footprint is easier to place next to a streaming kernel)
 template <typename... KArgs, typename... Args>
 static int launch_cluster(void (*kern)(KArgs...), int nr, cudaStream_t s, Args... args) {
-    return launch_cluster_dyn(STAGE_SLOTS * GT * (int)sizeof(double), kern, nr, s, args...);
+    return launch_cluster_dyn(STAGE_SLOTS * GT * (int)sizeof(double), kern, nr, 1, s, args...);
+}
+template <typename... KArgs, typename... Args>
+static int launch_clusters(void (*kern)(KArgs...), int nr, int nclusters, cudaStream_t s, Args... args) {
+    return launch_cluster_dyn(STAGE_SLOTS * GT * (int)sizeof(double), kern, nr, nclusters, s, args...);
 }
 template <typename... KArgs, typename... Args>
 static int launch_cluster_nostage(void (*kern)(KArgs...), int nr, cudaStream_t s, Args... args) {
-    return launch_cluster_dyn(0, kern, nr, s, args...);
+    return launch_cluster_dyn(0, kern, nr, 1, s, args...);
 }
 
 }  // namespace qa
@@ -2057,4 +2091,49 @@ extern "C" int qa_greedy_assign_par(const double* table, int64_t ntiles, double 
                                     int64_t* counts, double* state, void* work, qa_stream_t stream) {
     return qa_greedy_assign_passes(table, ntiles, numel, metric, threshold, fmt_order, nfmt, rng, assignment, counts, state, work,
                                    nullptr, nullptr, nullptr, 0, nfmt, 0, stream);
+}
+
+// per threshold: the chain's scratch (the single-run layout of the metric's kernel), then the slot its stream ends in
+static int64_t sweep_chain_bytes(int64_t ntiles, int metric) {
+    return al(metric == QA_METRIC_ATOL ? qa_greedy_work_bytes(ntiles) : qa_greedy_par_work_bytes(ntiles));
+}
+
+extern "C" int64_t qa_greedy_sweep_work_bytes(int64_t ntiles, int metric) {
+    if (ntiles <= 0 || ntiles > 0x3FFFFFFF || metric < QA_METRIC_PCC || metric > QA_METRIC_ATOL) return -1;
+    return sweep_chain_bytes(ntiles, metric) + al(sizeof(qa_pcg64));
+}
+
+extern "C" int qa_greedy_assign_sweep(const double* table, int64_t ntiles, double numel, int metric, const double* thresholds,
+                                      int nthr, const int32_t* fmt_order, int nfmt, const qa_pcg64* rng, int8_t* assignment,
+                                      int64_t* counts, double* state, void* work, const int32_t* pre_order, const qa_pcg64* pre_rng,
+                                      const void* init, int flags, qa_stream_t stream) {
+    const char* who = "qa_greedy_assign_sweep";
+    if (!table || ntiles <= 0 || ntiles > 0x3FFFFFFF || !thresholds || nthr < 1 || !rng || !assignment || !counts || !state || !work) {
+        set_error("%s: bad args", who);
+        return 1;
+    }
+    if (metric < QA_METRIC_PCC || metric > QA_METRIC_ATOL) { set_error("%s: bad metric", who); return 1; }
+    ParOrder ord;
+    if (fill_order(fmt_order, nfmt, ord, who)) return 1;
+    const int64_t stride = qa_greedy_sweep_work_bytes(ntiles, metric);
+    char* rng_slot = static_cast<char*>(work) + sweep_chain_bytes(ntiles, metric);    // cluster / block 0's
+    cudaStream_t cs = (cudaStream_t)stream;
+    if (metric == QA_METRIC_ATOL)       // the one-thread chain, as for a single threshold: block k runs thresholds[k]
+        return greedy_seq_sweep_launch(table, ntiles, numel, thresholds, nthr, fmt_order, nfmt, rng,
+                                       reinterpret_cast<qa_pcg64*>(rng_slot), assignment, counts, state, work, stride, cs);
+    const int nr = pick_cluster(ntiles);
+    if ((int64_t)nthr * MAXR > 0x7FFFFFFF) { set_error("%s: too many thresholds", who); return 1; }
+    ParWork pw = carve(work, ntiles);
+    if (pre_order && pre_rng && nfmt >= 2) { pw.pre_order = pre_order; pw.pre_rng = pre_rng; pw.npre = nfmt >= 3 ? 3 : 2; }
+    if (init) {
+        pw.hdr = static_cast<double*>(const_cast<void*>(init));
+        pw.delta = init_delta(init);
+    } else if (int rc = greedy_init_launch(table, ntiles, metric, fmt_order, nfmt, pw.hdr, pw.delta, stream, who)) {
+        return rc;       // computed once, into the first chain's work, where every chain reads it
+    }
+    if (metric == QA_METRIC_PCC)
+        return launch_clusters(greedy_sweep_kernel<true>, nr, nthr, cs, table, (int)ntiles, numel, metric, thresholds, ord, rng,
+                               reinterpret_cast<qa_pcg64*>(rng_slot), assignment, counts, state, pw, stride, flags);
+    return launch_clusters(greedy_sweep_kernel<false>, nr, nthr, cs, table, (int)ntiles, numel, metric, thresholds, ord, rng,
+                           reinterpret_cast<qa_pcg64*>(rng_slot), assignment, counts, state, pw, stride, flags);
 }

@@ -429,6 +429,32 @@ def greedy_assign(table: torch.Tensor, numel: int, metric: str, threshold: float
     return assignment, counts, state
 
 
+def greedy_sweep(table: torch.Tensor, numel: int, metric: str, thresholds, fmt_order, rng: torch.Tensor, prefetched=None,
+                 init: torch.Tensor | None = None):
+    """The greedy chains of every threshold over one table in one launch (qa_greedy_assign_sweep): row k is what
+    greedy_assign gives for thresholds[k] from the stream state `rng` (not modified).  prefetched = greedy_prefetch(...) or
+    the permutation cache, init = greedy_init(...): shared by every chain (pcc / mae; atol runs the one-thread chain and
+    needs neither).  -> (maps int8 [K, ntiles], counts int64 [K, 4], states float64 [K, 24]) on the device."""
+    nt = table.shape[1]
+    dev = table.device
+    L = _lib.lib()
+    thr = torch.tensor(np.asarray(list(thresholds), dtype=np.float64).reshape(-1), device=dev)
+    k = thr.numel()
+    maps = torch.empty((k, nt), dtype=torch.int8, device=dev)
+    counts = torch.zeros((k, NFMT), dtype=torch.int64, device=dev)
+    states = torch.zeros((k, 24), dtype=torch.float64, device=dev)
+    per = L.qa_greedy_sweep_work_bytes(nt, METRIC_CODE[metric])
+    work = torch.empty(max(k, 1) * max(per, 0), dtype=torch.uint8, device=dev)
+    pre_order, pre_rng = prefetched if prefetched is not None else (None, None)
+    if pre_order is not None and len(fmt_order) >= 3 and pre_order.shape[0] < 2:
+        raise ValueError("prefetched permutations were drawn for fewer formats than fmt_order has")
+    order = _lib.int32_array([FMT_INDEX[f] for f in fmt_order])
+    check(L.qa_greedy_assign_sweep(_ptr(table), nt, float(numel), METRIC_CODE[metric], _ptr(thr), k, order, len(fmt_order), _ptr(rng),
+                                   _ptr(maps), _ptr(counts), _ptr(states), _ptr(work), _ptr(pre_order), _ptr(pre_rng), _ptr(init), 0,
+                                   _stream()), "qa_greedy_assign_sweep")
+    return maps, counts, states
+
+
 _STAGE_STREAMS: dict = {}
 
 

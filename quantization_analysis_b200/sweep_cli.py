@@ -3,6 +3,12 @@
 
     python -m quantization_analysis_b200.sweep_cli <repo_or_url> <tensor_name> [--no-regex] [--metric pcc|mae|atol]
            [--lowest-metric-val V] [--steps N] [--formats bf16,bfp8,bfp4,bfp2] [--out-dir DIR] [--checkpoint-dir DIR] [--gpus N]
+           [--algorithm mixed-tile-threshold|mixed-tile-greedy] [--seed S] [--highest-metric-val V]
+
+``--algorithm mixed-tile-greedy`` sweeps the greedy instead (sweep.greedy_sweep_tensor: one table and one launch for all
+thresholds per tensor), from ``--highest-metric-val`` (default: the first format's whole-tensor score) down to
+``--lowest-metric-val``; the first of ``--formats`` is its base format.  ``--seed`` is the greedy's (0, the default, draws
+one), drawn once for the run and recorded in every ``sweep_config.json``.  Files go under ``mixed_tile_greedy_sweep/``.
 
 Tensors come from ``tensor_source`` like wq's: the shards of ``--checkpoint-dir`` when given, else the float32 cache.  With
 ``--gpus N`` the matched tensors are split over N GPUs of the node like wq's (``multi_gpu``); the files are the same.
@@ -14,6 +20,7 @@ import contextlib
 import fnmatch
 import math
 import re
+import secrets
 import sys
 import time
 from dataclasses import dataclass
@@ -21,6 +28,8 @@ from pathlib import Path
 
 from . import multi_gpu, sweep, tensor_source
 from .compression_algorithms.tile_utils import MIXED_TILE_FORMATS
+
+ALGORITHMS = ("mixed-tile-threshold", "mixed-tile-greedy")
 
 
 def _parse_formats(value: str) -> list[str]:
@@ -72,18 +81,28 @@ class SweepJob:
     metric: str
     lowest: float
     steps: int
+    algorithm: str = "mixed-tile-threshold"
+    seed: int = 0                         # greedy: the resolved seed (never 0 here)
+    highest: float | None = None          # greedy: --highest-metric-val
 
 
 def sweep_one(job: SweepJob, name: str) -> str | None:
     """Sweep one tensor and write its ``details/<tensor>/`` files.  -> None, or the message of its SweepRangeError (nothing
     is written for that tensor)."""
     x = job.index.load(name)
+    greedy = job.algorithm == "mixed-tile-greedy"
     try:
-        rows, _maps = sweep.sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest)
+        if greedy:
+            rows, _maps = sweep.greedy_sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest, highest=job.highest, seed=job.seed)
+        else:
+            rows, _maps = sweep.sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest)
     except sweep.SweepRangeError as exc:
         return str(exc)
     out = job.detail / name.replace("/", "_").replace(".", "_")
-    sweep.write_sweep_config(out, job.repo_or_url, name, job.revision, job.backend, job.formats, job.metric, job.lowest, job.steps)
+    # highest_metric_val: the first threshold swept (the base format's score unless --highest-metric-val gave it)
+    extra = {"algorithm": job.algorithm, "seed": job.seed, "highest_metric_val": rows[0]["threshold"]} if greedy else None
+    sweep.write_sweep_config(out, job.repo_or_url, name, job.revision, job.backend, job.formats, job.metric, job.lowest, job.steps,
+                             greedy=extra)
     sweep.write_sweep_csv(out, rows, job.formats)
     return None
 
@@ -110,11 +129,41 @@ def build_parser() -> argparse.ArgumentParser:
                          "element count); the files equal a one-GPU run's.  When --lowest-metric-val is out of range for a tensor, "
                          "the error of the first such tensor in name order is printed and the exit code is 1, as without the "
                          "flag, but other GPUs may already have written tensors that come after it in name order.")
+    ap.add_argument("--algorithm", default="mixed-tile-threshold",
+                    help=f"Algorithm to sweep: {' or '.join(ALGORITHMS)} (default mixed-tile-threshold).")
+    ap.add_argument("--seed", type=int, default=None,
+                    help="mixed-tile-greedy only: the greedy's seed; 0 (the default) draws one, recorded in sweep_config.json.")
+    ap.add_argument("--highest-metric-val", type=float, default=None,
+                    help="mixed-tile-greedy only: first (tightest) threshold; default: the first format's whole-tensor score.")
     return ap
+
+
+def greedy_args_error(args) -> str | None:
+    """The message for an --algorithm / --seed / --highest-metric-val combination that cannot run, else None."""
+    if args.algorithm not in ALGORITHMS:
+        return f"--algorithm must be one of {', '.join(ALGORITHMS)}, not {args.algorithm!r}"
+    if args.algorithm != "mixed-tile-greedy":
+        for flag, v in (("--seed", args.seed), ("--highest-metric-val", args.highest_metric_val)):
+            if v is not None:
+                return f"{flag} applies to --algorithm mixed-tile-greedy only"
+        return None
+    if args.seed is not None and not 0 <= args.seed < 2 ** 63:
+        return "--seed must be 0 (random) or a positive integer"
+    if args.highest_metric_val is not None and not math.isfinite(args.highest_metric_val):
+        return "--highest-metric-val must be a finite number"
+    return None
 
 
 def main(argv=None) -> int:
     args = build_parser().parse_args(argv)
+    err = greedy_args_error(args)
+    if err is not None:
+        print(f"error: {err}", file=sys.stderr)
+        return 1
+    greedy = args.algorithm == "mixed-tile-greedy"
+    seed = 0
+    if greedy:      # resolved once here, so that every tensor on every GPU uses the recorded seed
+        seed = args.seed if args.seed else secrets.randbits(31)
     if args.gpus is not None:
         err = multi_gpu.gpu_count_error(args.gpus)
         if err is not None:
@@ -133,12 +182,13 @@ def main(argv=None) -> int:
         for n in selected:
             print(f"  {n}")
         return 0
-    base = Path(args.out_dir) if args.out_dir else (Path("results") / index.repo_id.replace("/", "__") / "mixed_tile_threshold_sweep"
+    kind = "mixed_tile_greedy_sweep" if greedy else "mixed_tile_threshold_sweep"
+    base = Path(args.out_dir) if args.out_dir else (Path("results") / index.repo_id.replace("/", "__") / kind
                                                     / time.strftime("%Y%m%d-%H%M%S"))
     detail = base / "details"
     detail.mkdir(parents=True, exist_ok=True)
     job = SweepJob(index, detail, args.repo_or_url, args.revision, args.backend, formats, args.metric, args.lowest_metric_val,
-                   args.steps)
+                   args.steps, args.algorithm, seed, args.highest_metric_val)
     if args.gpus is None:
         results = ((name, sweep_one(job, name)) for name in selected)
     else:
