@@ -364,6 +364,14 @@ int qa_tensor_scores_f32(const void* x, int x_dtype, const void* y, int y_dtype,
                          const int32_t* plan_dev, const int32_t* plan_head_host, float* out, void* work,
                          qa_stream_t stream);
 
+/* out[cols][rows] (contiguous) = x[rows][cols] (leading dimension ld) for elem_bytes 1, 2 or 4; any other value is
+ * rejected.  The device layout of a linear weight: the checkpoint stores W [out, in], the Tenstorrent device holds
+ * W^T [in, out], and its BFP groups and 32x32 tiles are taken there.  The mixed-tile algorithms run in that layout by
+ * transposing once and then using every row-major kernel above unchanged (bf16 / float32 weights, fp8 e4m3fn bytes with
+ * their float32 scale grid - dequant(w^T, s^T) == dequant(w, s)^T - and the reconstruction back).  x and out must not
+ * overlap.  Vector accesses when x, out, ld and rows allow them. */
+int qa_transpose_2d(const void* x, int elem_bytes, int64_t rows, int64_t cols, int64_t ld, void* out, qa_stream_t stream);
+
 /* fp32 -> bf16 bit patterns plus a count of elements that are NOT bf16-exact (low 16 bits != 0).
  * Host helper for the numpy-in API (SURVEY.md H7).  inexact_count: uint64 on device (accumulated). */
 int qa_f32_to_bf16_checked(const float* x, int64_t n, void* out_bf16, unsigned long long* inexact_count,

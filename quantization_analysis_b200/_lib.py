@@ -26,7 +26,7 @@ EXPORTS = [
     "qa_f32_to_bf16_checked", "qa_scalar_proxy", "qa_fp8_block_dequant", "qa_greedy_par_work_bytes", "qa_greedy_assign_par", "qa_numpy_permutation_par", "qa_collective_bench", "qa_debug_times", "qa_greedy_cluster_cap", "qa_greedy_assign_passes", "qa_greedy_init_sums_range", "qa_greedy_init_deltas", "qa_tile_stats_rows", "qa_greedy_init_bytes", "qa_perm_resolve", "qa_perm_resolve_chain", "qa_perm_apply", "qa_perm_apply_work_bytes", "qa_pair_sums", "qa_pair_sums_work_bytes",
     "qa_pairwise_plan_words", "qa_pairwise_plan_build", "qa_tensor_scores_work_bytes", "qa_tensor_scores_f32",
     "qa_tile_stats_f32", "qa_tile_stats_fp8", "qa_tile_stats_items", "qa_tile_stats_batch", "qa_greedy_init_deltas_batch",
-    "qa_greedy_sweep_work_bytes", "qa_greedy_assign_sweep",
+    "qa_greedy_sweep_work_bytes", "qa_greedy_assign_sweep", "qa_transpose_2d",
 ]
 
 
@@ -125,6 +125,7 @@ def lib():
     L.qa_tensor_scores_work_bytes.argtypes = [i64, i32]
     L.qa_tensor_scores_work_bytes.restype = i64
     L.qa_tensor_scores_f32.argtypes = [vp, i32, vp, i32, i64, i32, i64, vp, vp, vp, vp, vp]
+    L.qa_transpose_2d.argtypes = [vp, i32, i64, i64, i64, vp, vp]
     for name in EXPORTS:
         fn = getattr(L, name)
         if name not in ("qa_last_error", "qa_greedy_work_bytes", "qa_greedy_par_work_bytes", "qa_greedy_init_bytes", "qa_perm_apply_work_bytes", "qa_version",

@@ -44,7 +44,9 @@ def filter_formats(formats, algo_name: str) -> list[str]:
 
 @dataclass
 class DeviceResult:
-    """What one algorithm run leaves on the device (nothing is copied to the host unless asked)."""
+    """What one algorithm run leaves on the device (nothing is copied to the host unless asked).  transposed: the run was
+    in the device layout - `prepared` holds x.T (engine.prepare_transposed) and the map is over its tiles - while y_device()
+    and `metrics` are in x's layout."""
     compression: str
     prepared: engine.Prepared
     assignment: torch.Tensor | None        # int8 [ntiles] (device) for mixed results
@@ -53,26 +55,45 @@ class DeviceResult:
     metrics_exact: dict                    # float64 recombination of pcc / mae / atol from the tile-stat table
     tile_formats: list[str]
     meta: dict = field(default_factory=dict)
+    transposed: bool = False
     _y: torch.Tensor | None = None
     _metrics: dict | None = None
 
     @property
+    def shape(self) -> tuple:
+        """Shape of x (and of y)."""
+        p = self.prepared
+        return tuple(reversed(p.shape)) if self.transposed else p.shape
+
+    @property
     def metrics(self) -> dict:
         """pcc / mae / atol of the result as the reference reports them (wq:684-687): float32, NumPy's summation orders
-        (qa_tensor_scores_f32 over x and the materialised reconstruction)."""
+        (qa_tensor_scores_f32 over x and the materialised reconstruction, both in x's layout)."""
         if self._metrics is None:
             p = self.prepared
-            s = engine.tensor_scores_f32(p.data, self.y_device(), n=p.numel)[0]
+            s = engine.tensor_scores_f32(self.x_device(), self.y_device(), n=p.numel)[0]
             self._metrics = {"pcc": float(s[0]), "mae": float(s[1]), "atol": float(s[2])}
         return self._metrics
 
+    def x_device(self) -> torch.Tensor:
+        """x on the device in its own layout (flat; a transposed run transposes its copy back)."""
+        p = self.prepared
+        if not self.transposed:
+            return p.data
+        return engine.transpose_2d(p.data.reshape(p.rows, p.cols)).reshape(-1)
+
     def y_device(self) -> torch.Tensor:
-        """bf16 reconstruction on the device (materialised on first use)."""
+        """bf16 reconstruction on the device (materialised on first use), flat, in x's layout."""
         if self._y is None:
-            self._y = engine.apply_assignment(self.prepared, self.assignment)
+            y = engine.apply_assignment(self.prepared, self.assignment)
+            if self.transposed:
+                p = self.prepared
+                y = engine.transpose_2d(y.reshape(p.rows, p.cols)).reshape(-1)
+            self._y = y
         return self._y
 
     def assignment_numpy(self) -> np.ndarray:
+        """The map [tiles_h, tiles_w] over the tiles of the layout the run used (x.T's when transposed)."""
         p = self.prepared
         return self.assignment.cpu().numpy().astype(np.int8).reshape(p.tiles_h, p.tiles_w)
 
@@ -96,14 +117,36 @@ def numel_of(x) -> int:
 
 
 def finish(dr: DeviceResult, xf, extra_meta: dict | None = None):
-    """DeviceResult -> the reference's (y, counts, assignment) triple in the caller's array type."""
+    """DeviceResult -> the reference's (y, counts, assignment) triple in the caller's array type; y has x's shape."""
     y_dev = dr.y_device()
-    if is_torch(xf):
+    if dr.transposed:
+        y = y_dev.reshape(dr.shape)
+        if not is_torch(xf):
+            y = y.to(torch.float32).cpu().numpy()
+    elif is_torch(xf):
         p = dr.prepared
         y = y_dev[: p.numel].reshape(p.shape) if p.kind == "vector" else y_dev.reshape(p.shape)
     else:
         y = engine.result_to_numpy(dr.prepared, y_dev)
     return y, dr.counts, dr.assignment_numpy()
+
+
+def parse_transpose(params: dict) -> bool:
+    """params["transpose"] (default False): run in the device layout, over the tiles of x.T.  Only a bool is accepted."""
+    v = params.get("transpose", False)
+    if not isinstance(v, bool):
+        raise ValueError(f"transpose must be true or false, not {v!r}")
+    return v
+
+
+def prepare(xf, transpose: bool) -> engine.Prepared:
+    """x in the layout an algorithm runs in: x.T's tiles when `transpose` (engine.prepare_transposed), else x's."""
+    return engine.prepare_transposed(xf) if transpose else engine.prepare_tiles(xf)
+
+
+def is_transposed(p: engine.Prepared, transpose: bool) -> bool:
+    """Whether a run with the flag over `p` is in a layout other than x's (0-D and 1-D inputs: x.T is x)."""
+    return bool(transpose) and p.kind == "nd"
 
 
 def total_bytes(counts: dict) -> float:

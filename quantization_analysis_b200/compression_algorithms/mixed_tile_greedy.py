@@ -34,6 +34,8 @@ class MixedTileGreedyCompression(CompressionAlgorithm):
         self.certify = bool(self.params.get("certify", True))
         self.margin_bound = float(self.params.get("margin_bound", 2e-13))
         self.tile_formats = mc.parse_formats(raw) if raw is not None else None
+        # extension: run in the device layout, over the tiles of x.T (BFP groups down the columns of the stored W)
+        self.transpose = mc.parse_transpose(self.params)
         if self.metric not in mc.VALID_METRICS:
             raise ValueError(f"Unsupported metric: {self.metric}")
 
@@ -51,7 +53,8 @@ class MixedTileGreedyCompression(CompressionAlgorithm):
         return mc.filter_formats(formats, "mixed-tile-greedy")
 
     def run_prepared(self, p: engine.Prepared, tile_formats, table=None, seed: int | None = None) -> mc.DeviceResult:
-        """Device-resident run; `table` may be shared between algorithms on the same tensor."""
+        """Device-resident run; `table` may be shared between algorithms on the same tensor.  `p` is in the algorithm's
+        layout already (engine.prepare_transposed when the transpose param is set)."""
         if table is None:
             table = engine.tile_stats(p, MIXED_TILE_FORMATS, strict=True if self.strict else None,
                                       exact_abs=(self.metric == "mae"))
@@ -81,19 +84,22 @@ class MixedTileGreedyCompression(CompressionAlgorithm):
         sums = engine.assignment_sums(table, assignment)
         metrics = engine.metrics_from_sums(sums.cpu().numpy(), p.numel)
         return mc.DeviceResult(self.name, p, assignment, counts, mc.total_bytes(counts), metrics, list(tile_formats),
-                               meta={"seed": seed, "state": state, "table": table, "certificate": cert})
+                               meta={"seed": seed, "state": state, "table": table, "certificate": cert},
+                               transposed=mc.is_transposed(p, self.transpose))
 
     def run_fp8_blocks(self, w_fp8, scale_inv, formats=None, seed: int | None = None) -> mc.DeviceResult:
         """Extension for real checkpoints: an fp8 e4m3fn tensor + per-block inverse scales as stored on disk
         (hf_model_utils.py:199-215,271-281).  The table comes from one pass over the bytes (engine.tile_stats on an Fp8Prepared);
-        the result is what `run` gives on the reference's dequantized float32 tensor."""
+        the result is what `run` gives on the reference's dequantized float32 tensor (with the transpose param: the bytes and
+        the scale grid are transposed on the device, the table still comes from the bytes)."""
         tile_formats = self.tile_formats or self._filter_from_formats(formats or MIXED_TILE_FORMATS)
-        return self.run_prepared(engine.Fp8Prepared(w_fp8, scale_inv), tile_formats, seed=seed)
+        p = engine.Fp8Prepared(w_fp8, scale_inv)
+        return self.run_prepared(engine.prepare_transposed(p) if self.transpose else p, tile_formats, seed=seed)
 
     def _compress(self, xf, quantizer, tile_formats):
         if mc.numel_of(xf) == 0:
             return mc.empty_result(xf)
-        dr = self.run_prepared(engine.prepare_tiles(xf), tile_formats)
+        dr = self.run_prepared(mc.prepare(xf, self.transpose), tile_formats)
         return mc.finish(dr, xf)
 
     def run(self, xf, formats, quantizer=None, cache=None):

@@ -30,6 +30,7 @@ class MixedTileRandomCompression(CompressionAlgorithm):
         self.seed = int(self.params.get("seed", 0))
         self.formats = mc.parse_formats(self.params.get("formats"))
         self.sample_scoring = str(self.params.get("sample_scoring", "reference"))
+        self.transpose = mc.parse_transpose(self.params)          # extension: the device layout (tiles of x.T)
         if self.metric not in mc.VALID_METRICS:
             raise ValueError(f"Unsupported metric: {self.metric}")
         if self.iters < 1:
@@ -77,10 +78,12 @@ class MixedTileRandomCompression(CompressionAlgorithm):
         assignment = choices[best_id].contiguous()
         counts = {f: int(cnt[best_id, i]) for i, f in enumerate(MIXED_TILE_FORMATS)}
         metrics = {"pcc": float(met[best_id, 0]), "mae": float(met[best_id, 1]), "atol": float(met[best_id, 2])}
+        transposed = mc.is_transposed(p, self.transpose)
         dr = mc.DeviceResult(self.name, p, assignment, counts, mc.total_bytes(counts), metrics, fmt_list,
-                             meta={"samples": samples, "best_id": best_id})
-        if self.sample_scoring != "exact":
+                             meta={"samples": samples, "best_id": best_id}, transposed=transposed)
+        if self.sample_scoring != "exact" and not transposed:
             dr._metrics = dict(metrics)            # already the reference's float32 values of the chosen sample
+        # transposed: the samples are scored over x.T's flatten order; dr.metrics scores the chosen one in x's layout
         return dr
 
     @staticmethod
@@ -105,7 +108,7 @@ class MixedTileRandomCompression(CompressionAlgorithm):
         if mc.numel_of(xf) == 0:
             y, counts, assignment = mc.empty_result(xf)
             return y, counts, assignment, []
-        dr = self.run_prepared(engine.prepare_tiles(xf), tile_formats)
+        dr = self.run_prepared(mc.prepare(xf, self.transpose), tile_formats)
         y, counts, assignment = mc.finish(dr, xf)
         return y, counts, assignment, dr.meta["samples"]
 

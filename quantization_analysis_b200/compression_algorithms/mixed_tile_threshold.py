@@ -28,6 +28,7 @@ class MixedTileThresholdCompression(CompressionAlgorithm):
         self.threshold = float(self.params.get("threshold", 0.999))
         raw = self.params.get("formats", self.params.get("tile_formats"))
         self.tile_formats = mc.parse_formats(raw) if raw is not None else None
+        self.transpose = mc.parse_transpose(self.params)          # extension: the device layout (tiles of x.T)
         if self.metric not in mc.VALID_METRICS:
             raise ValueError(f"Unsupported metric: {self.metric}")
 
@@ -57,12 +58,12 @@ class MixedTileThresholdCompression(CompressionAlgorithm):
         if table is not None:
             metrics = engine.metrics_from_sums(engine.assignment_sums(table, assignment[0]).cpu().numpy(), p.numel)
         return mc.DeviceResult(self.name, p, assignment[0], counts, mc.total_bytes(counts), metrics, list(tile_formats),
-                               meta={"scores": scores})
+                               meta={"scores": scores}, transposed=mc.is_transposed(p, self.transpose))
 
     def _compress(self, xf, quantizer, tile_formats):
         if mc.numel_of(xf) == 0:
             return mc.empty_result(xf)
-        dr = self.run_prepared(engine.prepare_tiles(xf), tile_formats)
+        dr = self.run_prepared(mc.prepare(xf, self.transpose), tile_formats)
         return mc.finish(dr, xf)
 
     def run(self, xf, formats, quantizer=None, cache=None):

@@ -127,6 +127,43 @@ def prepare_loaded(x) -> Prepared:
     return prepare_tiles(x)
 
 
+_ELEM_BYTES = {torch.uint8: 1, torch.bfloat16: 2, torch.float32: 4}
+
+
+def transpose_2d(t: torch.Tensor) -> torch.Tensor:
+    """Contiguous device copy of t.T for a 2-D device tensor of 1-, 2- or 4-byte elements (qa_transpose_2d)."""
+    if t.dim() != 2 or t.dtype not in _ELEM_BYTES:
+        raise ValueError(f"transpose_2d expects a 2-D uint8 / bfloat16 / float32 tensor, got {t.dtype} {tuple(t.shape)}")
+    if t.stride(1) != 1:
+        t = t.contiguous()
+    rows, cols = int(t.shape[0]), int(t.shape[1])
+    out = torch.empty((cols, rows), dtype=t.dtype, device=t.device)
+    check(_lib.lib().qa_transpose_2d(_ptr(t), _ELEM_BYTES[t.dtype], rows, cols, max(int(t.stride(0)), cols), _ptr(out), _stream()),
+          "qa_transpose_2d")
+    return out
+
+
+def prepare_transposed(x) -> Prepared:
+    """The device layout: a linear weight W [out, in] is held on the device as W^T [in, out], and the BFP groups and the
+    32x32 tiles are taken there.  -> prepare_loaded(x.T) for a 2-D x (the tile grid is [ceil(cols/32), ceil(rows/32)]):
+    one H2D copy (bf16 when the values are bf16-exact, as prepare_tiles), then qa_transpose_2d on the device.  An fp8
+    weight (tensor_source.Fp8Blocks or Fp8Prepared) stays fp8: its bytes and its scale grid are transposed, and
+    dequant(w^T, s^T) == dequant(w, s)^T element for element.  A Prepared already on the device is transposed there.
+    0-D and 1-D inputs: x.T is x, so this is prepare_loaded(x).  3 or more dimensions: ValueError."""
+    shape = tuple(x.shape)
+    if len(shape) > 2:
+        raise ValueError(f"the transposed (device) layout needs a 0-, 1- or 2-D tensor, got shape {shape}")
+    if len(shape) < 2:
+        return prepare_loaded(x)
+    if isinstance(x, tensor_source.Fp8Blocks):
+        x = Fp8Prepared(x.weight, x.scale_inv)
+    if isinstance(x, Fp8Prepared):
+        return Fp8Prepared(transpose_2d(x.w8), transpose_2d(x.scale_inv))
+    p = x if isinstance(x, Prepared) else prepare_tiles(x)
+    data = p.data.reshape(p.rows, p.cols)
+    return Prepared(transpose_2d(data).reshape(-1), p.dtype_code, p.cols, p.rows, p.numel, (p.cols, p.rows), "nd")
+
+
 def prepare_rows(x) -> Prepared:
     """Quantizer geometry: rows of the last axis (1-D: one row)."""
     shape = tuple(x.shape)

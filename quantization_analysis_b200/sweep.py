@@ -62,15 +62,20 @@ def _score_maps(p: engine.Prepared, maps: torch.Tensor, rows_idx) -> dict[int, n
     return out
 
 
+def _prepare(x, transpose: bool) -> engine.Prepared:
+    return engine.prepare_transposed(x) if transpose else engine.prepare_loaded(x)
+
+
 def sweep_tensor(x, tile_formats=MIXED_TILE_FORMATS, metric: str = "pcc", steps: int = 32, lowest: float = 0.9,
-                 thresholds=None, scoring: str = "reference"):
+                 thresholds=None, scoring: str = "reference", transpose: bool = False):
     """x: a host array or tensor, what tensor_source's loaders return (tensor_source.Fp8Blocks included), or an
-    engine.Prepared.  -> (rows, maps): rows = list of dicts {threshold (float64), counts, total_bytes, pcc, mae, atol} and the int8 maps
+    engine.Prepared.  transpose=True: the sweep over the tiles of x.T (the device layout; engine.prepare_transposed) - every
+    row, map and score is what the unflagged sweep gives on x.T.  -> (rows, maps): rows = list of dicts {threshold (float64), counts, total_bytes, pcc, mae, atol} and the int8 maps
     [steps, ntiles] in MIXED_TILE_FORMATS numbering.  scoring="reference": the reference's float32 whole-tensor values
     (every distinct map is materialised and scored); "exact": float64 recombination of the tile-stat table, all maps in one
     launch, no reconstruction (the mathematically exact value of the same formulas)."""
     tile_formats = list(tile_formats)
-    p = engine.prepare_loaded(x)
+    p = _prepare(x, transpose)
     scores = engine.tile_scores(p, tile_formats)[_ROW[metric]].contiguous()
     if thresholds is None:
         thresholds = sweep_thresholds(scores, tile_formats, metric, steps, lowest)
@@ -119,12 +124,12 @@ def greedy_thresholds(highest: float, metric: str, steps: int, lowest: float) ->
 
 def greedy_sweep_tensor(x, tile_formats=MIXED_TILE_FORMATS, metric: str = "pcc", steps: int = 32, lowest: float = 0.9,
                         highest: float | None = None, seed: int = 0, thresholds=None, scoring: str = "reference",
-                        certify: bool = True, margin_bound: float = 2e-13):
+                        certify: bool = True, margin_bound: float = 2e-13, transpose: bool = False):
     """mixed-tile-greedy over a range of thresholds: one tile-stat table, one init, one set of permutations and one launch
     for all the chains (engine.greedy_sweep).  Row k equals MixedTileGreedyCompression({"threshold": thresholds[k],
     "seed": seed, ...}).run_prepared on the same tensor: map, counts, state, certificate and metrics.
 
-    x: as sweep_tensor.  tile_formats: the greedy's order, the first is the base format.  Thresholds: float64
+    x, transpose: as sweep_tensor (transpose=True gives the unflagged sweep of x.T, the default `highest` included).  tile_formats: the greedy's order, the first is the base format.  Thresholds: float64
     ``np.linspace(highest, lowest, steps)`` unless given; `highest` defaults to the base format's whole-tensor float32 score
     (wq's `none` row).  seed 0 draws one at random (as the greedy does); every row records the seed used.  Certificate: a
     pcc / mae chain whose decision margin (state[20]) is below `margin_bound` is redone alone from NumPy-order tile sums with
@@ -141,7 +146,7 @@ def greedy_sweep_tensor(x, tile_formats=MIXED_TILE_FORMATS, metric: str = "pcc",
         raise ValueError(f"Unsupported metric: {metric}")
     if seed == 0:
         seed = secrets.randbits(31)           # mixed_tile_greedy.py:222-224
-    p = engine.prepare_loaded(x)
+    p = _prepare(x, transpose)
     if thresholds is None:
         if highest is None:
             highest = base_format_score(p, tile_formats[0], metric)
@@ -225,10 +230,14 @@ def write_sweep_csv(out_dir, rows, formats=MIXED_TILE_FORMATS):
     return out / "sweep_results.csv"
 
 
-def write_sweep_config(out_dir, repo_or_url, tensor_name, revision, backend, formats, metric, lowest, steps, greedy=None):
-    """``sweep_config.json`` (sweep:675-686).  greedy: {"algorithm", "seed", "highest_metric_val"} of a greedy sweep, appended."""
+def write_sweep_config(out_dir, repo_or_url, tensor_name, revision, backend, formats, metric, lowest, steps, greedy=None,
+                       transpose: bool = False):
+    """``sweep_config.json`` (sweep:675-686).  greedy: {"algorithm", "seed", "highest_metric_val"} of a greedy sweep, appended;
+    a sweep over the tiles of x.T appends "transpose": true (nothing when unset, so those files are unchanged)."""
     out = Path(out_dir)
     out.mkdir(parents=True, exist_ok=True)
     payload = {"repo_or_url": repo_or_url, "tensor_name": tensor_name, "revision": revision, "backend": backend,
                "formats": list(formats), "metric": metric, "lowest_metric_val": lowest, "steps": steps, **(greedy or {})}
+    if transpose:
+        payload["transpose"] = True
     (out / "sweep_config.json").write_text(json.dumps(payload, indent=2), encoding="utf-8")

@@ -3,12 +3,16 @@
 
     python -m quantization_analysis_b200.sweep_cli <repo_or_url> <tensor_name> [--no-regex] [--metric pcc|mae|atol]
            [--lowest-metric-val V] [--steps N] [--formats bf16,bfp8,bfp4,bfp2] [--out-dir DIR] [--checkpoint-dir DIR] [--gpus N]
-           [--algorithm mixed-tile-threshold|mixed-tile-greedy] [--seed S] [--highest-metric-val V]
+           [--algorithm mixed-tile-threshold|mixed-tile-greedy] [--seed S] [--highest-metric-val V] [--transpose]
 
 ``--algorithm mixed-tile-greedy`` sweeps the greedy instead (sweep.greedy_sweep_tensor: one table and one launch for all
 thresholds per tensor), from ``--highest-metric-val`` (default: the first format's whole-tensor score) down to
 ``--lowest-metric-val``; the first of ``--formats`` is its base format.  ``--seed`` is the greedy's (0, the default, draws
 one), drawn once for the run and recorded in every ``sweep_config.json``.  Files go under ``mixed_tile_greedy_sweep/``.
+
+``--transpose`` sweeps either algorithm in the device layout: over the tiles of W^T, where the device takes its BFP groups
+and 32x32 tiles (sweep.sweep_tensor / greedy_sweep_tensor with transpose=True); ``sweep_config.json`` then records
+``"transpose": true``.
 
 Tensors come from ``tensor_source`` like wq's: the shards of ``--checkpoint-dir`` when given, else the float32 cache.  With
 ``--gpus N`` the matched tensors are split over N GPUs of the node like wq's (``multi_gpu``); the files are the same.
@@ -84,6 +88,7 @@ class SweepJob:
     algorithm: str = "mixed-tile-threshold"
     seed: int = 0                         # greedy: the resolved seed (never 0 here)
     highest: float | None = None          # greedy: --highest-metric-val
+    transpose: bool = False               # --transpose: over the tiles of x.T
 
 
 def sweep_one(job: SweepJob, name: str) -> str | None:
@@ -93,16 +98,17 @@ def sweep_one(job: SweepJob, name: str) -> str | None:
     greedy = job.algorithm == "mixed-tile-greedy"
     try:
         if greedy:
-            rows, _maps = sweep.greedy_sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest, highest=job.highest, seed=job.seed)
+            rows, _maps = sweep.greedy_sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest, highest=job.highest, seed=job.seed,
+                                                    transpose=job.transpose)
         else:
-            rows, _maps = sweep.sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest)
+            rows, _maps = sweep.sweep_tensor(x, job.formats, job.metric, job.steps, job.lowest, transpose=job.transpose)
     except sweep.SweepRangeError as exc:
         return str(exc)
     out = job.detail / name.replace("/", "_").replace(".", "_")
     # highest_metric_val: the first threshold swept (the base format's score unless --highest-metric-val gave it)
     extra = {"algorithm": job.algorithm, "seed": job.seed, "highest_metric_val": rows[0]["threshold"]} if greedy else None
     sweep.write_sweep_config(out, job.repo_or_url, name, job.revision, job.backend, job.formats, job.metric, job.lowest, job.steps,
-                             greedy=extra)
+                             greedy=extra, transpose=job.transpose)
     sweep.write_sweep_csv(out, rows, job.formats)
     return None
 
@@ -135,6 +141,9 @@ def build_parser() -> argparse.ArgumentParser:
                     help="mixed-tile-greedy only: the greedy's seed; 0 (the default) draws one, recorded in sweep_config.json.")
     ap.add_argument("--highest-metric-val", type=float, default=None,
                     help="mixed-tile-greedy only: first (tightest) threshold; default: the first format's whole-tensor score.")
+    ap.add_argument("--transpose", action="store_true",
+                    help="Sweep over the tiles of the transposed tensor (the device layout W^T, where the BFP groups and "
+                         "32x32 tiles are taken); recorded in sweep_config.json.")
     return ap
 
 
@@ -188,7 +197,7 @@ def main(argv=None) -> int:
     detail = base / "details"
     detail.mkdir(parents=True, exist_ok=True)
     job = SweepJob(index, detail, args.repo_or_url, args.revision, args.backend, formats, args.metric, args.lowest_metric_val,
-                   args.steps, args.algorithm, seed, args.highest_metric_val)
+                   args.steps, args.algorithm, seed, args.highest_metric_val, args.transpose)
     if args.gpus is None:
         results = ((name, sweep_one(job, name)) for name in selected)
     else:

@@ -67,20 +67,24 @@ def resolve_seed(config, algo_params: dict):
     return used, source
 
 
-def _mapping(assignment: np.ndarray) -> dict:
-    return {"tile_hw": 32, "format_to_int": {f: i for i, f in enumerate(MIXED_TILE_FORMATS)},
-            "int_to_format": MIXED_TILE_FORMATS, "assignment_shape": list(assignment.shape)}
+def _mapping(assignment: np.ndarray, transposed: bool = False) -> dict:
+    """The mapping JSON; a map over the tiles of x.T (the device layout) says so with "layout": "transposed"."""
+    m = {"tile_hw": 32, "format_to_int": {f: i for i, f in enumerate(MIXED_TILE_FORMATS)},
+         "int_to_format": MIXED_TILE_FORMATS, "assignment_shape": list(assignment.shape)}
+    if transposed:
+        m["layout"] = "transposed"
+    return m
 
 
-def write_assignment(out_dir: Path, algo_dir: str, tensor_name: str, assignment: np.ndarray) -> None:
+def write_assignment(out_dir: Path, algo_dir: str, tensor_name: str, assignment: np.ndarray, transposed: bool = False) -> None:
     """assignment.npy + assignment_mapping.json (wq:295-316)."""
     d = out_dir / algo_dir / _slug(tensor_name)
     d.mkdir(parents=True, exist_ok=True)
     np.save(d / "assignment.npy", assignment.astype(np.int8))
-    (d / "assignment_mapping.json").write_text(json.dumps(_mapping(assignment), indent=2))
+    (d / "assignment_mapping.json").write_text(json.dumps(_mapping(assignment, transposed), indent=2))
 
 
-def write_random_outputs(out_dir: Path, tensor_name: str, samples, tile_formats, assignment) -> None:
+def write_random_outputs(out_dir: Path, tensor_name: str, samples, tile_formats, assignment, transposed: bool = False) -> None:
     """<slug>.csv + <slug>_assignment.npy + mapping (wq:151-194)."""
     if not samples:
         return
@@ -95,7 +99,7 @@ def write_random_outputs(out_dir: Path, tensor_name: str, samples, tile_formats,
                          s["pcc"], s["mae"], s["atol"]])
     if assignment is not None:
         np.save(d / f"{slug}_assignment.npy", assignment.astype(np.int8))
-        (d / f"{slug}_assignment_mapping.json").write_text(json.dumps(_mapping(assignment), indent=2))
+        (d / f"{slug}_assignment_mapping.json").write_text(json.dumps(_mapping(assignment, transposed), indent=2))
 
 
 @dataclass
@@ -157,9 +161,11 @@ def evaluate_tensor(name: str, x, algorithms, formats, out_dir: Path | None, cac
                                                           if f in FORMAT_BYTES_PER_ELEM else 0.0))
             continue
         tile_formats = getattr(algo, "tile_formats", None) or getattr(algo, "formats", None) or algo._filter_from_formats(formats)
+        # "transpose": true - the mixed algorithm runs over x.T (the device layout) with its own copy and table
+        pm = engine.prepare_transposed(p) if getattr(algo, "transpose", False) else p
         if table is None and getattr(algo, "strict", False) is False and algo.name != "mixed-tile-threshold":
-            table = engine.tile_stats(p, engine.MIXED_FORMATS)
-        dr = algo.run_prepared(p, tile_formats, table=table)
+            table = engine.tile_stats(pm, engine.MIXED_FORMATS)
+        dr = algo.run_prepared(pm, tile_formats, table=table)
         dr.y_device()                                            # the reference's run() returns y: part of TIME(s)
         torch.cuda.synchronize()
         elapsed = time.perf_counter() - t0
@@ -169,9 +175,9 @@ def evaluate_tensor(name: str, x, algorithms, formats, out_dir: Path | None, cac
         if out_dir is not None:
             a = dr.assignment_numpy()
             if algo.name == "mixed-tile-random":
-                write_random_outputs(out_dir, name, dr.meta["samples"], dr.tile_formats, a)
+                write_random_outputs(out_dir, name, dr.meta["samples"], dr.tile_formats, a, dr.transposed)
             else:
-                write_assignment(out_dir, algo.name.replace("-", "_"), name, a)
+                write_assignment(out_dir, algo.name.replace("-", "_"), name, a, dr.transposed)
     return rows, meta
 
 
