@@ -287,17 +287,6 @@ int qa_greedy_assign_sweep(const double* table, int64_t ntiles, double numel, in
  * see each other's value.  Returns the previous value. */
 int qa_greedy_cluster_cap(int max_cluster);
 
-/* Diagnostic timeline: device timestamps (ns) {first start, last end} of the cluster kernels since the last reset -
- * resolve chain, init sums, chain launch containing pass 0, later chain launch - one row of 8 per cluster-size class
- * (log2 of the cluster size, 0..4).  out8_host: HOST array of 40 (may be NULL); reset != 0 re-arms the slots.  A debugging aid,
- * the one synchronous entry point (cudaMemcpy{From,To}Symbol), and only live in a library built with -DQA_STAMP_TIMES: the
- * shipped build compiles the in-kernel timestamps out and this call returns 3. */
-int qa_debug_times(unsigned long long* out8_host, int reset);
-
-/* Diagnostic: cycles per call of the cluster collectives used by qa_greedy_assign_par
- * (out double[8] on device: scan+flag exchange, 3-way min, cluster.sync, __syncthreads, pair scan). */
-int qa_collective_bench(double* out, int iters, int cluster, qa_stream_t stream);
-
 /* Per-tile threshold assignment for nthr thresholds at once.
  * Replaces mixed_tile_threshold.py:111-123 and scripts/sweep_mixed_tile_threshold.py:145-155.
  * scores: float32[QA_NFMT][ntiles] of ONE metric; order[norder]: formats by ascending bytes;

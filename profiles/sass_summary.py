@@ -50,7 +50,7 @@ for (mangled, c), name in zip(kern.items(), demangle):
                + (f" <!-- {wide} x LDG.256 -->" if wide else ""))
 out += ["", "Markers: packed fp32 (`FFMA2` / `FADD2` / `FMUL2`), `FMNMX3`, `FMNMX.XORSIGN` and 256-bit `LDG.E...256` loads in the streaming kernels;",
         "`SYNCS` (mbarrier) + distributed-shared-memory stores and `UCGABAR_*` in the cluster kernels; TMA bulk copies (`UBLKCP.S.G`, completing on",
-        "`SYNCS.ARRIVE.TRANS64` mbarriers) in `sdot_pipe_kernel` and the opt-in `stats_tma_kernel`; `F2FP` = the hardware e4m3x2 -> f16x2 and f32 -> bf16x2",
+        "`SYNCS.ARRIVE.TRANS64` mbarriers) in `sdot_pipe_kernel`; `F2FP` = the hardware e4m3x2 -> f16x2 and f32 -> bf16x2",
         "conversions of `stats_f32_kernel`; no tensor-core instructions (the path is not a contraction)."]
 (ROOT / "profiles" / "r2_sass_summary.md").write_text("\n".join(out) + "\n")
 print("\n".join(out[:12]))

@@ -23,7 +23,7 @@ EXPORTS = [
     "qa_version", "qa_last_error", "qa_quant_recon", "qa_quant_recon_cols", "qa_tile_stats", "qa_tile_scores_f32", "qa_tile_scores_pair_f32",
     "qa_numpy_permutation", "qa_numpy_integers", "qa_greedy_work_bytes", "qa_greedy_assign",
     "qa_threshold_assign", "qa_random_samples", "qa_apply_assignment", "qa_assignment_sums", "qa_assignment_sums_batch",
-    "qa_f32_to_bf16_checked", "qa_scalar_proxy", "qa_fp8_block_dequant", "qa_greedy_par_work_bytes", "qa_greedy_assign_par", "qa_numpy_permutation_par", "qa_collective_bench", "qa_debug_times", "qa_greedy_cluster_cap", "qa_greedy_assign_passes", "qa_greedy_init_sums_range", "qa_greedy_init_deltas", "qa_tile_stats_rows", "qa_greedy_init_bytes", "qa_perm_resolve", "qa_perm_resolve_chain", "qa_perm_apply", "qa_perm_apply_work_bytes", "qa_pair_sums", "qa_pair_sums_work_bytes",
+    "qa_f32_to_bf16_checked", "qa_scalar_proxy", "qa_fp8_block_dequant", "qa_greedy_par_work_bytes", "qa_greedy_assign_par", "qa_numpy_permutation_par", "qa_greedy_cluster_cap", "qa_greedy_assign_passes", "qa_greedy_init_sums_range", "qa_greedy_init_deltas", "qa_tile_stats_rows", "qa_greedy_init_bytes", "qa_perm_resolve", "qa_perm_resolve_chain", "qa_perm_apply", "qa_perm_apply_work_bytes", "qa_pair_sums", "qa_pair_sums_work_bytes",
     "qa_pairwise_plan_words", "qa_pairwise_plan_build", "qa_tensor_scores_work_bytes", "qa_tensor_scores_f32",
     "qa_tile_stats_f32", "qa_tile_stats_fp8", "qa_tile_stats_items", "qa_tile_stats_batch", "qa_greedy_init_deltas_batch",
     "qa_greedy_sweep_work_bytes", "qa_greedy_assign_sweep", "qa_transpose_2d",
@@ -85,8 +85,6 @@ def lib():
     L.qa_greedy_par_work_bytes.restype = i64
     L.qa_greedy_assign_par.argtypes = [vp, i64, f64, i32, f64, C.POINTER(C.c_int32), i32, vp, vp, vp, vp, vp, vp]
     L.qa_numpy_permutation_par.argtypes = [vp, i64, vp, vp, vp]
-    L.qa_collective_bench.argtypes = [vp, i32, i32, vp]
-    L.qa_debug_times.argtypes = [vp, i32]
     L.qa_greedy_cluster_cap.argtypes = [i32]
     L.qa_pair_sums.argtypes = [vp, vp, i64, vp, vp, vp]
     L.qa_pair_sums_work_bytes.argtypes = []

@@ -26,8 +26,6 @@
 //    steps that last wrote the position it reads.
 #include <cooperative_groups.h>
 
-#include <cstdio>
-
 #include <mutex>
 
 #include "qa_common.cuh"
@@ -43,26 +41,6 @@ constexpr int DPT = 8;            // draws per thread per round (4 LCG outputs)
 constexpr int EPS = 8;           // elements each thread streams through per chunk (scan works on thread totals)
 constexpr int SEQ_TAIL = 96;      // last Fisher-Yates steps are drawn by one thread
 constexpr long long M_LO = 1ll << 52, M_HI = 1ll << 53;
-
-// Diagnostic timeline: first-start / last-end device timestamps (ns, %globaltimer) of the cluster kernels of this file,
-// read back with qa_debug_times.  Slots: 0/1 resolve chain, 2/3 init sums, 4/5 chain launch with pass 0, 6/7 later launch.
-// One row of 8 per cluster-size class (log2 of the cluster size, 0..4), so tensors of different sizes can be told apart.
-// Diagnostic only: compiled in with -DQA_STAMP_TIMES (profiles/step_variants.py); the shipped library does no global
-// atomics of its own in these kernels and qa_debug_times reports "not compiled in".
-__device__ unsigned long long qa_times[5 * 8];
-__device__ __forceinline__ void stamp(int slot, bool is_end) {
-#ifndef QA_STAMP_TIMES
-    (void)slot; (void)is_end;
-    return;
-#endif
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    unsigned nr;
-    asm volatile("mov.u32 %0, %%cluster_nctaid.x;" : "=r"(nr));
-    const int cls = 31 - __clz((int)(nr | 1u));
-    if (is_end) atomicMax(&qa_times[cls * 8 + slot], t);
-    else atomicMin(&qa_times[cls * 8 + slot], t);
-}
 
 struct ParOrder {
     int32_t fmt[QA_NFMT];
@@ -87,11 +65,6 @@ struct ParWork {
     int npre;                   // how many permutations were drawn ahead (0, 2 or 3)
 };
 constexpr int HDR_DOUBLES = 32;
-#ifdef QA_DBG_CHAIN
-#define QA_PHASE_SYNC() __syncthreads()
-#else
-#define QA_PHASE_SYNC()
-#endif
 
 struct P2 {          // increment of m if the incoming m is even / odd
     long long d0, d1;
@@ -767,15 +740,8 @@ __device__ void perm_resolve(Coop& c, Pcg& g, int m, int32_t* jarr) {     // jar
     unsigned long long rk = 0ull, pnext = g.has32 ? 1ull : 2ull;
     int i_cur = m - 1;
     long long t0 = clock64();
-#ifdef QA_DBG_PERM
-    long long d_gen = 0, d_sw = 0, d_wr = 0, td;
-    int d_sweeps = 0, d_rounds = 0;
-#endif
     while (i_cur > SEQ_TAIL) {
         ++c.n_rounds;
-#ifdef QA_DBG_PERM
-        __syncthreads(); td = clock64(); ++d_rounds;
-#endif
         const int L = i_cur - SEQ_TAIL;                      // accepts still wanted from the parallel part
         const unsigned long long kb = pnext >> 1;
         if (kb != rk) {
@@ -801,9 +767,6 @@ __device__ void perm_resolve(Coop& c, Pcg& g, int m, int32_t* jarr) {     // jar
         // every sweep fixes at least one more thread (typically all of them within ~10 sweeps)
         // start from the expected accept count at the current acceptance rate (any start converges: the prefix of
         // thread 0 is exact from the first exchange on, and every sweep fixes at least one more thread)
-#ifdef QA_DBG_PERM
-        __syncthreads(); d_gen += clock64() - td; td = clock64();
-#endif
         int c_in, total = 0, a_prev = -1;
         {
             // expected accepts among the valid draws before this thread's first one: within a mask bracket the rate is
@@ -832,9 +795,6 @@ __device__ void perm_resolve(Coop& c, Pcg& g, int m, int32_t* jarr) {     // jar
             c_in = c_new;
             a = local_accepts(raw, validmask, c_in, i_cur, L);
         }
-#ifdef QA_DBG_PERM
-        __syncthreads(); d_sw += clock64() - td; td = clock64();
-#endif
         // write j for the steps this thread resolved; find the draw that supplied the L-th accept
         int done_off = 0x7FFFFFFF;
         {
@@ -858,14 +818,7 @@ __device__ void perm_resolve(Coop& c, Pcg& g, int m, int32_t* jarr) {     // jar
             pnext = 2ull * (kb + 4ull * (unsigned long long)c.gth);      // every draw of the round was consumed
         }
         i_cur -= total;
-#ifdef QA_DBG_PERM
-        __syncthreads(); d_wr += clock64() - td;
-#endif
     }
-#ifdef QA_DBG_PERM
-    __syncthreads();
-    const long long t_tail0 = clock64();
-#endif
     // tail (the last <= SEQ_TAIL steps) and stream hand-back, by warp 0 of every CTA (redundantly, identically): the
     // lanes generate the next 256 draws in parallel (one LCG jump per lane), lane 0 consumes them in order.
     if (tid < 32) {
@@ -932,10 +885,6 @@ __device__ void perm_resolve(Coop& c, Pcg& g, int m, int32_t* jarr) {     // jar
     g.has32 = (uint32_t)c.sh.i32[3 * NW + 2];
     g.buf32 = (uint32_t)c.sh.i32[3 * NW + 3];
     c.sync();
-#ifdef QA_DBG_PERM
-    if (c.gtid == 0) printf("resolve m=%d rounds %d gen %lld sweeps %lld write+min %lld tail %lld total %lld\n", m, d_rounds, d_gen, d_sw, d_wr,
-                            clock64() - t_tail0, clock64() - t0);
-#endif
     c.cy_resolve += clock64() - t0;
 }
 
@@ -946,18 +895,10 @@ __device__ void perm_apply(Coop& c, int m, const int32_t* cand, int32_t* out, co
         return;
     }
     const long long t0 = clock64();
-#ifdef QA_DBG_PERM
-    long long tp[8]; int np_ = 0;
-#define QA_TP() tp[np_++] = clock64()
-#else
-#define QA_TP()
-#endif
     for (int p = c.gtid; p < m; p += c.gth) w.cursor[p] = 0;
     c.sync();
-    QA_TP();
     for (int i = 1 + c.gtid; i < m; i += c.gth) atomicAdd(&w.cursor[w.jarr[i]], 1);
     c.sync();
-    QA_TP();
     {   // exclusive scan of the per-position counts -> off[], contiguous range per thread
         const int per = (m + c.gth - 1) / c.gth;
         const int b = min(m, c.gtid * per), e = min(m, b + per);
@@ -974,13 +915,11 @@ __device__ void perm_apply(Coop& c, int m, const int32_t* cand, int32_t* out, co
         if (c.gtid == 0) w.off[m] = total;
     }
     c.sync();
-    QA_TP();
     for (int i = 1 + c.gtid; i < m; i += c.gth) {
         const int slot = atomicAdd(&w.cursor[w.jarr[i]], 1);
         w.bucket[slot] = i;
     }
     c.sync();
-    QA_TP();
     for (int p = c.gtid; p < m; p += c.gth) {
         const int b = w.off[p], e = w.off[p + 1];
         for (int a = b + 1; a < e; ++a) {          // insertion sort (buckets hold ~1 entry)
@@ -998,7 +937,6 @@ __device__ void perm_apply(Coop& c, int m, const int32_t* cand, int32_t* out, co
         w.parent[p] = par;       // first later-executed step that writes position p
     }
     c.sync();
-    QA_TP();
     for (int i = c.gtid; i < m; i += c.gth) {
         // a[0] ends as the content of position 0 after all steps; a[i] (i >= 1) is what step i read
         const int start = i == 0 ? w.parent[0] : w.succ[i];
@@ -1012,11 +950,6 @@ __device__ void perm_apply(Coop& c, int m, const int32_t* cand, int32_t* out, co
         out[i] = cand ? cand[val] : val;
     }
     c.sync();
-    QA_TP();
-#ifdef QA_DBG_PERM
-    if (c.gtid == 0) printf("apply m=%d zero %lld count %lld scan %lld fill %lld sort %lld follow %lld\n", m, tp[0] - t0, tp[1] - tp[0],
-                            tp[2] - tp[1], tp[3] - tp[2], tp[4] - tp[3], tp[5] - tp[4]);
-#endif
     c.cy_apply += clock64() - t0;
 }
 
@@ -1059,7 +992,6 @@ __global__ void __launch_bounds__(GT) perm_resolve_chain_kernel(const qa_pcg64* 
     Coop c(sh);
     Pcg g;
     g.load(rng_in);
-    if (c.gtid == 0) stamp(0, false);
     c.sync();
     for (int k = 0; k < count; ++k) {
         perm_resolve(c, g, n, ((write_mask >> k) & 1u) ? jarr + (size_t)k * n : nullptr);
@@ -1069,7 +1001,6 @@ __global__ void __launch_bounds__(GT) perm_resolve_chain_kernel(const qa_pcg64* 
             g.store(rng_out + k);
         }
     }
-    if (c.gtid == 0) stamp(1, true);
 }
 
 // Per-thread staging of the chunk's addends in shared memory ([slot][thread] layout: conflict-free), so the
@@ -1318,9 +1249,7 @@ __global__ void __launch_bounds__(GT) greedy_init_kernel(const double* __restric
                                                          int t_begin, int t_end) {
     __shared__ Sh sh;
     Coop c(sh);
-    if (c.gtid == 0) stamp(2, false);
     init_phase<PCC>(c, table, nt, ord, hdr, t_begin, t_end);
-    if (c.gtid == 0) stamp(3, true);
 }
 
 // delta[tr][t] = stats(fmt[tr+1]) - stats(fmt[tr]) of tile t: one 32-byte record per tile and transition, so the chain
@@ -1369,15 +1298,8 @@ __global__ void __launch_bounds__(256) greedy_delta_batch_kernel(const qa_batch_
 // two tile-stat CTAs of the next tensor lists fit beside it.  The cluster kernels issue on ~17 % of the cycles, the tile-stat
 // kernel is pipe-bound, so sharing the SMs pays once enough lists are in flight: cfg2 step 0.286 -> 0.269 ms with 12 lists
 // (profiles/r2_chain_regcap2.txt, r2_chain_regcap3.txt; 96 / 112 registers give the same, 168 nothing), at the price of a
-// 13 % longer chain for a tensor processed alone (0.326 -> 0.369 ms).  -DQA_CHAIN_MAXNREG=0 restores the uncapped kernel.
-#ifndef QA_CHAIN_MAXNREG
-#define QA_CHAIN_MAXNREG 128
-#endif
-#if QA_CHAIN_MAXNREG > 0
-#define QA_CHAIN_REGCAP __maxnreg__(QA_CHAIN_MAXNREG)
-#else
-#define QA_CHAIN_REGCAP __launch_bounds__(GT, 1)
-#endif
+// 13 % longer chain for a tensor processed alone (0.326 -> 0.369 ms).  DESIGN.md §3.5 has the measurements.
+#define QA_CHAIN_REGCAP __maxnreg__(128)
 // The chain body, shared by the single-run kernel and the sweep kernel.  The stream starts at *rng_in; its final position goes
 // to *rng_out (the same pointer for a single run; a private slot for a sweep chain, whose starting state is shared).
 template <bool PCC>
@@ -1392,7 +1314,6 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
     const int tid = threadIdx.x;
     const int base = ord.fmt[0];
     const bool first = fi_begin == 0, last = fi_end >= ord.n;
-    if (c.gtid == 0) stamp(first ? 4 : 6, false);
     constexpr bool is_pcc = PCC;
     // running sums carried with the reference's exact rounding sequence: sy, sy2, sxy (pcc) | sabs (mae).
     // In pcc mode sum|x-y| only enters the degenerate den == 0 branch (mixed_tile_greedy.py:187-188): it is
@@ -1419,7 +1340,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
     unsigned chain_rounds = 0;
     const int32_t* order_ptr = w.order;
     long long t_mark = clock64(), cyc_perm = 0, cyc_chain = 0;
-    long long cy_load = 0, cy_scan = 0, cy_dec = 0, cy_min = 0, cy_commit = 0, cy_gather = 0, tq = 0;
+    long long cy_load = 0, cy_scan = 0, cy_dec = 0, cy_commit = 0, cy_gather = 0, tq = 0;
     unsigned n_chunks = 0, n_cutshort = 0;
     const long long cyc_init = (long long)w.hdr[7];
     const int CHc = c.gth * EPS;
@@ -1602,7 +1523,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
                     else staged(0, j) = db[j].y;
                 }
             }
-            QA_PHASE_SYNC(); cy_load += clock64() - tq;
+            cy_load += clock64() - tq;
             for (int round = 0; round < 64; ++round) {
                 ++chain_rounds;
                 tq = clock64();
@@ -1626,7 +1547,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
 #pragma unroll
                     for (int s = 0; s < NS; ++s) pre0[s] = P2{0, 0};
                 }
-                QA_PHASE_SYNC(); cy_scan += clock64() - tq; tq = clock64();
+                cy_scan += clock64() - tq; tq = clock64();
                 // walk 2: exact state before every element -> decision; first wrong flag; first binade exit
                 int mism = 0x7FFFFFFF, cut = 0x7FFFFFFF;
                 D = 0;
@@ -1663,13 +1584,12 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
                         }
                     }
                 }
-                QA_PHASE_SYNC(); cy_dec += clock64() - tq; tq = clock64();
+                cy_dec += clock64() - tq; tq = clock64();
                 // third slot: 0 if any element would carry an accept flag in the next round (F below mism, D from it on)
                 const int nval = max(0, min(cnt, valid - lo));
                 const int next_any = ((D | F) & (nval > 0 ? (0xFFFFFFFFu >> (32 - nval)) : 0u)) ? 0 : 0x7FFFFFFF;
                 int next_any_io = next_any;
                 c_min3(c, mism, cut, next_any_io);
-                QA_PHASE_SYNC(); cy_min += clock64() - tq;
                 cut = min(cut, valid - 1);
                 if (mism > cut) { valid = cut + 1; break; }       // flags are consistent up to the cut
                 if (round == 63) { valid = mism + 1; pathological = true; }   // commit up to the first wrong flag
@@ -1738,7 +1658,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
             ++n_chunks;
             if (valid < len) ++n_cutshort;
             pos += valid;
-            QA_PHASE_SYNC(); cy_commit += clock64() - tq;
+            cy_commit += clock64() - tq;
         }
         if (fi + 1 < ord.n) accepted_last = (int)c_reduce_d<false>(c, (double)my_accepts);     // exact: counts < 2^53
         cyc_chain += clock64() - t_mark;
@@ -1757,7 +1677,6 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
             r[6] = base_failed ? 1.0 : 0.0; r[7] = all_tiles_candidates ? 1.0 : 0.0; r[8] = (double)accepted_last;
             r[9] = (double)cyc_perm; r[10] = (double)cyc_chain; r[11] = done ? 1.0 : 0.0;
             r[12] = (double)n_chunks; r[13] = (double)n_cutshort; r[14] = min_margin;
-            stamp(first ? 5 : 7, true);
         }
         return;
     }
@@ -1781,11 +1700,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
         state[16] = (double)(clock64() - t_start); state[17] = (double)cy_commit; state[18] = (double)cy_gather;
         state[19] = (double)n_chunks; state[20] = min_margin;     // [20]: lower bound of min |value - thr| / thr over all decisions
         state[13] = w.hdr[8]; state[14] = w.hdr[9]; state[15] = w.hdr[10];
-#ifdef QA_DBG_CHAIN
-        printf("chain nt=%d load %lld walk1+scan %lld decide %lld min3 %lld commit %lld gather %lld | chunks %u rounds %u total %lld\n", nt, cy_load, cy_scan, cy_dec, cy_min, cy_commit, cy_gather, n_chunks, chain_rounds, (long long)(clock64() - t_start));
-#endif
         state[21] = (double)c.cy_resolve; state[22] = (double)c.cy_apply; state[23] = (double)c.n_sweeps + 65536.0 * c.n_rounds;
-        stamp(first ? 5 : 7, true);
     }
 }
 
@@ -1814,31 +1729,6 @@ __global__ void QA_CHAIN_REGCAP greedy_sweep_kernel(const double* __restrict__ t
     w.bucket = mine(w.bucket); w.succ = mine(w.succ); w.parent = mine(w.parent); w.res = mine(w.res); w.fixed = mine(w.fixed);
     greedy_chain<PCC>(table, nt, numel, metric, thresholds[k], ord, rng, mine(rng_out), assignment + (int64_t)k * nt,
                       counts + (int64_t)k * QA_NFMT, state + (int64_t)k * 24, w, 0, ord.n, flags);
-}
-
-// micro-benchmark of the collectives (cycles per call), for DESIGN.md / tuning
-__global__ void __launch_bounds__(GT) collective_bench_kernel(double* out, int iters) {
-    __shared__ Sh sh;
-    Coop c(sh);
-    int v = threadIdx.x & 3, tot = 0;
-    bool any;
-    long long t0 = clock64();
-    for (int i = 0; i < iters; ++i) v = c_scan_excl_any(c, v & 3, tot, (v & 1) != 0, any) & 7;
-    long long t1 = clock64();
-    int a = v, b = v + 1, d = v + 2;
-    for (int i = 0; i < iters; ++i) { c_min3(c, a, b, d); a += threadIdx.x & 1; }
-    long long t2 = clock64();
-    for (int i = 0; i < iters; ++i) c.sync();
-    long long t3 = clock64();
-    for (int i = 0; i < iters; ++i) __syncthreads();
-    long long t4 = clock64();
-    P2 tt[3] = {{v, v}, {1, 2}, {3, 3}}, pp[3];
-    for (int i = 0; i < iters; ++i) { scan_totals<3>(c, tt, pp); tt[0].d0 = pp[0].d0 & 3; }
-    long long t5 = clock64();
-    if (c.gtid == 0) {
-        out[0] = (double)(t1 - t0) / iters; out[1] = (double)(t2 - t1) / iters; out[2] = (double)(t3 - t2) / iters;
-        out[3] = (double)(t4 - t3) / iters; out[4] = (double)(t5 - t4) / iters; out[5] = (double)(a + tot + pp[1].d0);
-    }
 }
 
 static inline int64_t al(int64_t v) { return (v + 255) / 256 * 256; }
@@ -1949,29 +1839,10 @@ static int launch_cluster_nostage(void (*kern)(KArgs...), int nr, cudaStream_t s
 
 using namespace qa;
 
-extern "C" int qa_debug_times(unsigned long long* out8_host, int reset) {
-#ifndef QA_STAMP_TIMES
-    (void)out8_host; (void)reset;
-    set_error("qa_debug_times: timestamps are not compiled in (build with -DQA_STAMP_TIMES)");
-    return 3;
-#endif
-    if (out8_host && cudaMemcpyFromSymbol(out8_host, qa_times, sizeof(unsigned long long) * 40) != cudaSuccess) return check_launch("qa_debug_times");
-    if (reset) {
-        unsigned long long init[40];
-        for (int i = 0; i < 40; ++i) init[i] = (i & 1) ? 0ull : ~0ull;
-        if (cudaMemcpyToSymbol(qa_times, init, sizeof(init)) != cudaSuccess) return check_launch("qa_debug_times");
-    }
-    return 0;
-}
-
 extern "C" int qa_greedy_cluster_cap(int max_cluster) {
     const int prev = g_cluster_cap;
     g_cluster_cap = max_cluster < 0 ? 0 : (max_cluster > MAXR ? MAXR : max_cluster);
     return prev;
-}
-
-extern "C" int qa_collective_bench(double* out, int iters, int cluster, qa_stream_t stream) {
-    return launch_cluster(collective_bench_kernel, cluster, (cudaStream_t)stream, out, iters);
 }
 
 extern "C" int64_t qa_greedy_par_work_bytes(int64_t n) { return al(4 * (n + 1)) * 8 + al(n) + 2 * al(8 * HDR_DOUBLES) + al(96 * n) + 512; }

@@ -74,17 +74,10 @@ template <> struct Fmt<1> { static constexpr float M = 402653184.f, L = 224.f; }
 template <> struct Fmt<2> { static constexpr float M = 1610612736.f, L = 128.f; };   // bfp2: step 128
 
 // sm_100 packed-float2 arithmetic (FADD2 / FMUL2 / FFMA2: two fp32 lanes per issue slot)
-#ifdef QA_STATS_SCALAR      // experiment (profiles/r2_stats_variants.txt): scalar FADD / FFMA instead of the packed forms
-__device__ __forceinline__ float2 add2(float2 a, float2 b) { return make_float2(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y)); }
-__device__ __forceinline__ float2 sub2(float2 a, float2 b) { return make_float2(__fsub_rn(a.x, b.x), __fsub_rn(a.y, b.y)); }
-__device__ __forceinline__ float2 mul2(float2 a, float2 b) { return make_float2(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y)); }
-__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return make_float2(__fmaf_rn(a.x, b.x, c.x), __fmaf_rn(a.y, b.y, c.y)); }
-#else
 __device__ __forceinline__ float2 add2(float2 a, float2 b) { return __fadd2_rn(a, b); }
 __device__ __forceinline__ float2 sub2(float2 a, float2 b) { return __fadd2_rn(a, make_float2(-b.x, -b.y)); }
 __device__ __forceinline__ float2 mul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
 __device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
-#endif
 // clamp(y, -L, L) in one instruction: min(|y|, L) with the sign of y (FMNMX.XORSIGN)
 __device__ __forceinline__ float clamp_sym(float y, float L) {
     float r;
@@ -100,21 +93,12 @@ __device__ __forceinline__ float max3abs(float m, float a, float b) {
 struct GroupAcc {   // in-group float32 partials, two lanes (even / odd element) each
     float2 sy, sy2, sry, sab;
     float mx;
-    double dab;         // QA_SAB_FP64: sum |r| accumulated on the FP64 pipe (exact)
 };
-#ifndef QA_SAB_FP64
-#define QA_SAB_FP64 0
-#endif
 
 template <int F, bool EXACT_ABS>
 __device__ __forceinline__ void fmt_step(const float2 X, const float2 aX, GroupAcc& g) {
     const float2 Mv = make_float2(Fmt<F>::M, Fmt<F>::M);
-#ifdef QA_STATS_SCALAR_ROUND      // experiment: the rounding as scalar FADDs (they overlap the ALU clamps, the packed forms do not)
-    float2 y = make_float2(__fadd_rn(__fadd_rn(X.x, Fmt<F>::M), -Fmt<F>::M), __fadd_rn(__fadd_rn(X.y, Fmt<F>::M), -Fmt<F>::M));
-    (void)Mv;
-#else
     float2 y = sub2(add2(X, Mv), Mv);                  // round to the format's step, ties to even
-#endif
     y.x = clamp_sym(y.x, Fmt<F>::L);                   // mantissa clamp (no exponent bump)
     y.y = clamp_sym(y.y, Fmt<F>::L);
     const float2 r = sub2(X, y);
@@ -125,9 +109,6 @@ __device__ __forceinline__ void fmt_step(const float2 X, const float2 aX, GroupA
         // |X| - |r|: 0 for elements every format flushes, a short dyadic otherwise (exact in fp32)
         g.sab.x += aX.x - fabsf(r.x);
         g.sab.y += aX.y - fabsf(r.y);
-    } else if (QA_SAB_FP64) {
-        g.dab += fabs((double)r.x);
-        g.dab += fabs((double)r.y);
     } else {
         g.sab.x += fabsf(r.x);
         g.sab.y += fabsf(r.y);
@@ -177,7 +158,6 @@ __device__ __forceinline__ void group_fast(const uint32_t (&w)[8], TileAcc& a) {
     for (int f = 0; f < 3; ++f) {
         g[f].sy = g[f].sy2 = g[f].sry = g[f].sab = make_float2(0.f, 0.f);
         g[f].mx = 0.f;
-        g[f].dab = 0.0;
     }
     double gx = 0.0, gx2 = 0.0, gax = 0.0;
 #pragma unroll
@@ -207,7 +187,6 @@ __device__ __forceinline__ void group_fast(const uint32_t (&w)[8], TileAcc& a) {
         a.sy2[f] = fma((double)(g[f].sy2.x + g[f].sy2.y), s2, a.sy2[f]);
         a.sxy[f] = fma((double)(g[f].sry.x + g[f].sry.y), s2, a.sxy[f]);   // holds sum r*y; + sum y^2 at tile end
         if (EXACT_ABS) a.sab[f] += fma(-(double)(g[f].sab.x + g[f].sab.y), s1, gax);
-        else if (QA_SAB_FP64) a.sab[f] = fma(g[f].dab, s1, a.sab[f]);
         else a.sab[f] = fma((double)(g[f].sab.x + g[f].sab.y), s1, a.sab[f]);
         a.amax[f] = fmaxf(a.amax[f], g[f].mx * s1f);
     }
@@ -236,13 +215,8 @@ __device__ __forceinline__ void load_row_group(const uint16_t* __restrict__ x, i
 
 constexpr int FAST_WARPS = 4;               // warps per CTA; one CTA = one 32-row x 512-column item
 constexpr int FAST_RPW = TILE / FAST_WARPS; // rows per warp
-#ifndef FAST_UNROLL_N
-#define FAST_UNROLL_N 4
-#endif
-constexpr int FAST_UNROLL = FAST_UNROLL_N;
-#ifndef FAST_MIN_BLOCKS
-#define FAST_MIN_BLOCKS 4
-#endif
+constexpr int FAST_UNROLL = 4;
+constexpr int FAST_MIN_BLOCKS = 4;
 
 // One CTA per (tile row, 512-column chunk); warp w walks rows 8w..8w+7 of the stripe, the four
 // partial accumulator sets are summed in warp order through shared memory (fixed order => the
@@ -262,32 +236,8 @@ __device__ __forceinline__ void stats_fast_item(double (&part)[FAST_WARPS - 1][1
     TileAcc a;
     acc_zero(a);
     if (col0 < cols) {
-#ifdef QA_STATS_PREFETCH          // experiment: rows in batches of QA_STATS_PREFETCH, the next batch requested before this one is processed
-        constexpr int PB = QA_STATS_PREFETCH, NB = FAST_RPW / PB;
-        uint32_t buf[2][PB][8];
-        auto load_batch = [&](int b, uint32_t (&dst)[PB][8]) {
-#pragma unroll
-            for (int k = 0; k < PB; ++k) {
-                if (b * PB + k < nrows) load_row_group<VEC>(x, row0 + b * PB + k, col0, cols, ld, dst[k]);
-                else {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) dst[k][i] = 0u;
-                }
-            }
-        };
-        load_batch(0, buf[0]);
-#pragma unroll
-        for (int b = 0; b < NB; ++b) {
-            if (b + 1 < NB) load_batch(b + 1, buf[(b + 1) & 1]);
-#pragma unroll
-            for (int k = 0; k < PB; ++k) group_fast<EXACT_ABS>(buf[b & 1][k], a);
-        }
-        int r = nrows;
-        uint32_t cur[1][8];
-#else
         uint32_t cur[FAST_UNROLL][8];
         int r = 0;
-#endif
         for (; r + FAST_UNROLL <= nrows; r += FAST_UNROLL) {
 #pragma unroll
             for (int k = 0; k < FAST_UNROLL; ++k) load_row_group<VEC>(x, row0 + r + k, col0, cols, ld, cur[k]);
@@ -386,147 +336,6 @@ __global__ void __launch_bounds__(FAST_WARPS * 32, FAST_MIN_BLOCKS) stats_fast_b
     const bool vec = (d.cols % GROUP == 0) && (d.ld % GROUP == 0) && (reinterpret_cast<uintptr_t>(d.x) % 32 == 0);
     if (vec) stats_fast_item<true, EXACT_ABS>(part, partmx, x, d.rows, d.cols, d.ld, tiles_w, chunks, b - d.item_begin, tiles_h * tiles_w, fmt_mask, d.table);
     else stats_fast_item<false, EXACT_ABS>(part, partmx, x, d.rows, d.cols, d.ld, tiles_w, chunks, b - d.item_begin, tiles_h * tiles_w, fmt_mask, d.table);
-}
-
-// ------------------------------------------------------------------------------------------
-// FAST, TMA-staged (experiment of round 2, selected with QA_STATS_TMA=1): a persistent CTA walks (tile row, 512-column chunk)
-// items; thread 0 streams 16-row x 512-column half-items (16 bulk copies of 1 KB, one mbarrier per stage) into a two-stage
-// shared-memory ring, each warp pulls its four rows into registers (LDS.128), frees the stage and runs the same group
-// arithmetic.  The row loads leave the warps' scoreboards (12 % of the warp-time of stats_fast_kernel waits on them).
-// ------------------------------------------------------------------------------------------
-constexpr int TS_ROWS = 16, TS_NST = 2, TS_STAGE = TS_ROWS * 512 * 2;
-__device__ __forceinline__ unsigned ts_s32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ts_wait(unsigned bar, unsigned parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "TS_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra TS_DONE;\n\t"
-        "bra TS_WAIT;\n\t"
-        "TS_DONE:\n\t}" ::"r"(bar), "r"(parity) : "memory");
-}
-
-template <bool EXACT_ABS>
-__global__ void __launch_bounds__(FAST_WARPS * 32, FAST_MIN_BLOCKS) stats_tma_kernel(
-    const uint16_t* __restrict__ x, int64_t ld, int64_t tiles_w, int64_t chunks, int64_t item0, int64_t nitems, int64_t ntiles,
-    uint32_t fmt_mask, double* __restrict__ table) {
-    __shared__ __align__(128) unsigned char ring[TS_NST][TS_STAGE];
-    __shared__ __align__(8) unsigned long long full[TS_NST], empty[TS_NST];
-    __shared__ double part[FAST_WARPS - 1][14][32];
-    __shared__ float partmx[FAST_WARPS - 1][3][32];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    if (threadIdx.x == 0) {
-        for (int s_ = 0; s_ < TS_NST; ++s_) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(ts_s32(&full[s_])) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(ts_s32(&empty[s_])), "r"(FAST_WARPS) : "memory");
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncthreads();
-    if ((int64_t)blockIdx.x >= nitems) return;
-    const int64_t my_items = (nitems - blockIdx.x + gridDim.x - 1) / gridDim.x;
-    const int64_t nh = 2 * my_items;                       // half-items of this CTA, in order
-    auto issue = [&](int64_t h) {                          // thread 0: stage h % TS_NST <- half-item h
-        const int64_t item = item0 + blockIdx.x + (h >> 1) * gridDim.x;
-        const int64_t tr = item / chunks, ck = item - tr * chunks;
-        const uint16_t* src = x + (tr * TILE + (h & 1) * TS_ROWS) * ld + ck * 512;
-        const int s_ = (int)(h % TS_NST);
-        const unsigned bar = ts_s32(&full[s_]);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((unsigned)TS_STAGE) : "memory");
-#pragma unroll 4
-        for (int r = 0; r < TS_ROWS; ++r)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             ts_s32(&ring[s_][r * 1024])),
-                         "l"(src + (int64_t)r * ld), "r"(1024u), "r"(bar)
-                         : "memory");
-    };
-    if (threadIdx.x == 0)
-        for (int64_t h = 0; h < nh && h < TS_NST; ++h) issue(h);
-    TileAcc a;
-    acc_zero(a);
-    for (int64_t h = 0; h < nh; ++h) {
-        const int s_ = (int)(h % TS_NST);
-        const unsigned parity = (unsigned)((h / TS_NST) & 1);
-        ts_wait(ts_s32(&full[s_]), parity);
-        uint32_t cur[TS_ROWS / FAST_WARPS][8];
-        const unsigned char* base = &ring[s_][(w * (TS_ROWS / FAST_WARPS)) * 1024 + lane * 32];
-#pragma unroll
-        for (int k = 0; k < TS_ROWS / FAST_WARPS; ++k) {
-            const uint4 lo = *reinterpret_cast<const uint4*>(base + k * 1024), hi = *reinterpret_cast<const uint4*>(base + k * 1024 + 16);
-            cur[k][0] = lo.x; cur[k][1] = lo.y; cur[k][2] = lo.z; cur[k][3] = lo.w;
-            cur[k][4] = hi.x; cur[k][5] = hi.y; cur[k][6] = hi.z; cur[k][7] = hi.w;
-        }
-        __syncwarp();
-        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(ts_s32(&empty[s_])) : "memory");
-        if (threadIdx.x == 0 && h + TS_NST < nh) {         // every warp has its rows in registers: refill the stage
-            ts_wait(ts_s32(&empty[s_]), parity);
-            issue(h + TS_NST);
-        }
-#pragma unroll
-        for (int k = 0; k < TS_ROWS / FAST_WARPS; ++k) group_fast<EXACT_ABS>(cur[k], a);
-        if (!(h & 1)) continue;
-        // end of an item: the four warps' partial sets are summed in warp order (as in stats_fast_kernel)
-        const int64_t item = item0 + blockIdx.x + (h >> 1) * gridDim.x;
-        const int64_t tr = item / chunks, ck = item - tr * chunks;
-#pragma unroll
-        for (int f = 0; f < 3; ++f) a.sxy[f] += a.sy2[f];
-        if (w > 0) {
-            double (*p)[32] = part[w - 1];
-            p[0][lane] = a.sx; p[1][lane] = a.sx2;
-#pragma unroll
-            for (int f = 0; f < 3; ++f) {
-                p[2 + f][lane] = a.sy[f]; p[5 + f][lane] = a.sy2[f]; p[8 + f][lane] = a.sxy[f]; p[11 + f][lane] = a.sab[f];
-                partmx[w - 1][f][lane] = a.amax[f];
-            }
-        }
-        __syncthreads();
-        if (w == 0) {
-#pragma unroll
-            for (int q = 0; q < FAST_WARPS - 1; ++q) {
-                a.sx += part[q][0][lane]; a.sx2 += part[q][1][lane];
-#pragma unroll
-                for (int f = 0; f < 3; ++f) {
-                    a.sy[f] += part[q][2 + f][lane]; a.sy2[f] += part[q][5 + f][lane];
-                    a.sxy[f] += part[q][8 + f][lane]; a.sab[f] += part[q][11 + f][lane];
-                    a.amax[f] = fmaxf(a.amax[f], partmx[q][f][lane]);
-                }
-            }
-            a.sx += shfl_xor_d(a.sx, 1);
-            a.sx2 += shfl_xor_d(a.sx2, 1);
-#pragma unroll
-            for (int f = 0; f < 3; ++f) {
-                a.sy[f] += shfl_xor_d(a.sy[f], 1); a.sy2[f] += shfl_xor_d(a.sy2[f], 1);
-                a.sxy[f] += shfl_xor_d(a.sxy[f], 1); a.sab[f] += shfl_xor_d(a.sab[f], 1);
-                a.amax[f] = fmaxf(a.amax[f], __shfl_xor_sync(0xFFFFFFFFu, a.amax[f], 1));
-            }
-            const int64_t tc = ck * 16 + (lane >> 1);
-            if ((lane & 1) == 0 && tc < tiles_w) {
-                const int64_t t = tr * tiles_w + tc;
-                table[QA_STAT_SX * ntiles + t] = a.sx;
-                table[QA_STAT_SX2 * ntiles + t] = a.sx2;
-                if (fmt_mask & 1u) {
-                    table[QA_STAT_FMT(0, 0) * ntiles + t] = a.sx;
-                    table[QA_STAT_FMT(0, 1) * ntiles + t] = a.sx2;
-                    table[QA_STAT_FMT(0, 2) * ntiles + t] = a.sx2;
-                    table[QA_STAT_FMT(0, 3) * ntiles + t] = 0.0;
-                    table[QA_STAT_FMT(0, 4) * ntiles + t] = 0.0;
-                }
-#pragma unroll
-                for (int f = 0; f < 3; ++f) {
-                    if (fmt_mask & (2u << f)) {
-                        table[QA_STAT_FMT(f + 1, 0) * ntiles + t] = a.sy[f];
-                        table[QA_STAT_FMT(f + 1, 1) * ntiles + t] = a.sy2[f];
-                        table[QA_STAT_FMT(f + 1, 2) * ntiles + t] = a.sxy[f];
-                        table[QA_STAT_FMT(f + 1, 3) * ntiles + t] = a.sab[f];
-                        table[QA_STAT_FMT(f + 1, 4) * ntiles + t] = (double)a.amax[f];
-                    }
-                }
-            }
-        }
-        __syncthreads();                                   // part[] is free again
-        acc_zero(a);
-    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -716,13 +525,6 @@ static int tile_stats_fast(const void* x, int64_t rows, int64_t cols, int64_t ld
     const bool vec = (cols % GROUP == 0) && (ld % GROUP == 0) && (reinterpret_cast<uintptr_t>(x) % 32 == 0);
     const uint16_t* xp = reinterpret_cast<const uint16_t*>(x);
     const bool exact_abs = (mode == QA_STATS_FAST);
-    static const int use_tma = getenv("QA_STATS_TMA") ? atoi(getenv("QA_STATS_TMA")) : 0;
-    if (use_tma && vec && cols % 512 == 0 && rows % TILE == 0) {
-        const unsigned g = (unsigned)std::min<int64_t>(grid, 148 * use_tma);
-        if (exact_abs) stats_tma_kernel<true><<<g, FAST_WARPS * 32, 0, s>>>(xp, ld, tiles_w, chunks, item0, grid, ntiles, fmt_mask, table);
-        else stats_tma_kernel<false><<<g, FAST_WARPS * 32, 0, s>>>(xp, ld, tiles_w, chunks, item0, grid, ntiles, fmt_mask, table);
-        return check_launch("qa_tile_stats(fast, tma)");
-    }
     if (vec && exact_abs) stats_fast_kernel<true, true><<<(unsigned)grid, FAST_WARPS * 32, 0, s>>>(xp, rows, cols, ld, tiles_w, chunks, item0, ntiles, fmt_mask, table);
     else if (vec) stats_fast_kernel<true, false><<<(unsigned)grid, FAST_WARPS * 32, 0, s>>>(xp, rows, cols, ld, tiles_w, chunks, item0, ntiles, fmt_mask, table);
     else if (exact_abs) stats_fast_kernel<false, true><<<(unsigned)grid, FAST_WARPS * 32, 0, s>>>(xp, rows, cols, ld, tiles_w, chunks, item0, ntiles, fmt_mask, table);

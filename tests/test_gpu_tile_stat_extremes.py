@@ -16,11 +16,6 @@ row, as bf16-exact data (the bf16 kernels) and with 24-bit significands (the flo
 pattern spans few enough octaves that every tile sum the rules hold bit-equal is exactly representable.  No input is inf
 or NaN.
 """
-import os
-import subprocess
-import sys
-from pathlib import Path
-
 import numpy as np
 import pytest
 import torch
@@ -29,7 +24,6 @@ from oracle import qa_oracle as orc
 
 pytestmark = pytest.mark.gpu
 
-ROOT = Path(__file__).resolve().parent.parent
 MIXED = list(orc.MIXED_FORMATS)
 KEYS = ("sy", "sy2", "sxy", "sabs", "amax")
 SHAPES = {"vec": (64, 1024), "ragged": (45, 77), "1d": (3000,)}
@@ -279,41 +273,6 @@ def test_bf16_batch_kernel(qa):
     eng.tile_stats_batch(descs, n, items, MIXED, exact_abs=True)
     for (pattern, shape), t, want in zip(BF16_CASES, tables, wants):
         _check_bf16_fast(_table(t), want, (pattern, shape, "batch"))
-
-
-_TMA_SCRIPT = r"""
-import sys
-import numpy as np
-from quantization_analysis_b200 import engine
-z = np.load(sys.argv[1])
-out = {}
-for k in z.files:
-    p = engine.prepare_tiles(z[k])
-    assert p.dtype_code == 0
-    out[k + "__exact"] = engine.tile_stats(p, exact_abs=True).cpu().numpy()
-    out[k + "__approx"] = engine.tile_stats(p, exact_abs=False).cpu().numpy()
-np.savez(sys.argv[2], **out)
-"""
-
-
-def test_bf16_tma_kernel(qa, tmp_path):
-    """stats_tma_kernel (QA_STATS_TMA=1, read once per process: a subprocess) on every 64 x 1024 bf16 case: the default
-    kernel's bits in both |x-y| modes."""
-    eng = qa["eng"]
-    xs = {p: _case(p, "vec", False)[0] for p in BF16_PATTERNS}
-    np.savez(tmp_path / "in.npz", **xs)
-    env = dict(os.environ, QA_STATS_TMA="1", PYTHONPATH=os.pathsep.join([str(ROOT)] + [os.environ.get("PYTHONPATH", "")]))
-    flags = ["-s"] if sys.flags.no_user_site else []
-    r = subprocess.run([sys.executable, *flags, "-c", _TMA_SCRIPT, str(tmp_path / "in.npz"), str(tmp_path / "out.npz")],
-                       cwd=ROOT, env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-4000:]
-    got = np.load(tmp_path / "out.npz")
-    for pat, x in xs.items():
-        p = eng.prepare_tiles(x)
-        for mode, exact in (("exact", True), ("approx", False)):
-            ref = eng.tile_stats(p, exact_abs=exact).cpu().numpy()
-            assert np.array_equal(got[f"{pat}__{mode}"].view(np.uint64), ref.view(np.uint64)), (pat, mode)
-        _check_bf16_fast(_table(torch.from_numpy(got[f"{pat}__exact"])), _case(pat, "vec", False)[1], (pat, "tma"))
 
 
 # --------------------------------------------------------------------------------------------------------------------------
