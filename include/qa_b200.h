@@ -160,7 +160,9 @@ int qa_tile_stats_fp8(const void* w_fp8, const float* scale_inv, int64_t rows, i
 /* NumPy-float32-faithful per-tile scores on zero-padded 32x32 tiles.
  * Replaces tile_utils.py:46-57 (tile_metrics) incl. metrics.py:6-16 (pearson_corr) with the
  * float32 summation orders of NumPy 2.3.5 / OpenBLAS 0.3.30 SkylakeX (SURVEY.md App. B).
- * scores[(metric * QA_NFMT + f) * ntiles + tile], float32, for all three metrics. */
+ * scores[(metric * QA_NFMT + f) * ntiles + tile], float32, for all three metrics.  inf / nan elements propagate as in
+ * NumPy: a tile that holds one has nan mae and atol in every format whose reconstruction there is inf or nan, the bf16
+ * slot of a bf16 input included (inf - inf); atol is the maximum of the |x - y| bit patterns, so a nan is never dropped. */
 int qa_tile_scores_f32(const void* x, int x_dtype, int64_t rows, int64_t cols, int64_t ld,
                        uint32_t fmt_mask, float* scores, qa_stream_t stream);
 
@@ -303,7 +305,9 @@ int qa_threshold_assign(const float* scores, int64_t ntiles, const int32_t* orde
  * fmt_indices[nfmt]: candidate formats.  sample_metrics double[iters][3] = pcc, mae, atol;
  * sample_counts int64[iters][QA_NFMT].  choices: int8[iters][ntiles] (format index per tile)
  * must be pre-filled when `choices_ready` != 0 (k not a power of two), else it is produced
- * here by jumping the PCG64 stream; *rng is advanced past iters*ntiles draws. */
+ * here by jumping the PCG64 stream; *rng is advanced past iters*ntiles draws.  A nan in the table propagates: atol is the
+ * maximum of the max_abs column on its bit patterns (nan above +inf, like np.max), and a nan centred sum of squares keeps
+ * pcc nan as Python's max(v, 0.0) does. */
 int qa_random_samples(const double* table, int64_t ntiles, double numel,
                       const int32_t* fmt_indices, int nfmt, int iters, qa_pcg64* rng,
                       int8_t* choices, int choices_ready, double* sample_metrics,
@@ -317,7 +321,9 @@ int qa_apply_assignment(const void* x, int x_dtype, int64_t rows, int64_t cols, 
 
 /* Whole-tensor sums for a given assignment (or a single format when assignment == NULL and
  * fmt >= 0), reduced from the table in a fixed order: out double[8] =
- * {sx, sx2, sy, sy2, sxy, sabs, max_abs, 0}.  Feeds wq:684-687-style scoring. */
+ * {sx, sx2, sy, sy2, sxy, sabs, max_abs, 0}.  Feeds wq:684-687-style scoring.  max_abs is the maximum on the bit
+ * patterns of the non-negative doubles, so a nan in the table's max_abs column gives a nan max_abs (np.max); the sums
+ * propagate nan and inf by IEEE rules. */
 int qa_assignment_sums(const double* table, int64_t ntiles, const int8_t* assignment, int fmt,
                        double* out, qa_stream_t stream);
 /* qa_assignment_sums for nmaps assignment maps at once (one block per map): maps int8 [nmaps][ntiles] -> out double
@@ -327,7 +333,8 @@ int qa_assignment_sums_batch(const double* table, int64_t ntiles, const int8_t* 
 
 /* Sums over two arbitrary float32 arrays for compression_algorithms/metrics.py:6-27 (pearson_corr, mae, atol) and
  * the whole-tensor scoring of wq:684-687: out double[8] = {sum a, sum a^2, sum b, sum b^2, sum a*b, sum |a-b|,
- * max |a-b|, 0} in float64 with a fixed reduction tree (b == NULL means b = 0: the fp0 format).
+ * max |a-b|, 0} in float64 with a fixed reduction tree (b == NULL means b = 0: the fp0 format); max |a-b| is taken on the
+ * bit patterns, so a nan difference gives nan.
  * work: qa_pair_sums_work_bytes() bytes. */
 int64_t qa_pair_sums_work_bytes(void);
 int qa_pair_sums(const float* a, const float* b, int64_t n, double* out, void* work, qa_stream_t stream);

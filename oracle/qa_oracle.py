@@ -234,14 +234,17 @@ def np_pairwise_sum(a: np.ndarray) -> np.ndarray:
 
 
 def _fma_f32(a: np.ndarray, b: np.ndarray, c: np.ndarray) -> np.ndarray:
-    """Correctly rounded float32 fma(a, b, c), vectorised (round-to-odd in f64)."""
+    """Correctly rounded float32 fma(a, b, c), vectorised (round-to-odd in f64).
+
+    The product of two float32 values is exact in float64 and cannot overflow it, so a non-finite float64 sum s means an
+    inf or NaN operand: s is then the IEEE result (inf * 0 and inf - inf are NaN) and is returned as it is."""
     p = a.astype(np.float64) * b.astype(np.float64)          # exact (48 bits)
     cc = c.astype(np.float64)
     s = p + cc
     bb = s - p
     err = (p - (s - bb)) + (cc - bb)                          # TwoSum error term
     bits = s.view(np.uint64) if s.ndim else np.array(s).view(np.uint64)
-    inexact = err != 0.0
+    inexact = (err != 0.0) & np.isfinite(s)
     even = (bits & np.uint64(1)) == 0
     # round-to-odd: if inexact and the f64 result is even, step one ulp towards the true value
     toward_up = (err > 0.0) == (s > 0.0)
@@ -515,7 +518,8 @@ def tile_stat_table(x: np.ndarray, formats=MIXED_FORMATS) -> dict:
             for rs, cs in views[t]:
                 v = arr3[t][rs, cs]
                 lm = float(np.max(v)) if v.size else 0.0
-                m = max(m, lm)
+                if lm > m or lm != lm:          # np.max over the views: a nan wins (Python's max(0.0, nan) is 0.0)
+                    m = lm
             res[t] = m
         return res
 

@@ -114,8 +114,10 @@ __device__ __forceinline__ void greedy_seq(const double* __restrict__ table, int
         } else if (metric == QA_METRIC_MAE) {
             sabs = __dadd_rn(sabs, bsab[t]);
         } else {
+            // np.max of the column: a nan wins and stays (max_cnt no longer matters: nothing compares above a nan, so
+            // every later decision fails like the reference's)
             const double v = bmax[t];
-            if (t == 0 || v > max_abs) { max_abs = v; max_cnt = 1; }
+            if (t == 0 || v > max_abs || v != v) { max_abs = v; max_cnt = 1; }
             else if (v == max_abs) ++max_cnt;
         }
     }
@@ -173,7 +175,7 @@ __device__ __forceinline__ void greedy_seq(const double* __restrict__ table, int
                     bool first = true;
                     for (int64_t q = 0; q < nt; ++q) {
                         const double v = q == t ? new_max : table[QA_STAT_FMT(assignment[q], 4) * nt + q];
-                        if (first || v > c_max) { c_max = v; c_cnt = 1; first = false; }
+                        if (first || v > c_max || v != v) { c_max = v; c_cnt = 1; first = false; }
                         else if (v == c_max) ++c_cnt;
                     }
                 }
@@ -248,6 +250,12 @@ __global__ void __launch_bounds__(256) threshold_kernel(const float* __restrict_
 // ------------------------------------------------------------------------------------------
 constexpr int RB = 256;
 
+// max of two non-negative doubles (values of |x - y|) on their bit patterns: they order like unsigned integers, and a nan
+// (np.max propagates it) orders above +inf.  fmax would drop the nan.
+__device__ __forceinline__ double absmax(double a, double b) {
+    return __longlong_as_double((long long)max((unsigned long long)__double_as_longlong(a), (unsigned long long)__double_as_longlong(b)));
+}
+
 __device__ __forceinline__ double block_sum(double v, double* sm) {
     // fixed-shape tree: deterministic for a given (ntiles, RB)
 #pragma unroll
@@ -310,19 +318,19 @@ __global__ void __launch_bounds__(RB) random_samples_kernel(const double* __rest
         sy2 += table[QA_STAT_FMT(c, 1) * nt + t];
         sxy += table[QA_STAT_FMT(c, 2) * nt + t];
         sab += table[QA_STAT_FMT(c, 3) * nt + t];
-        amax = fmax(amax, table[QA_STAT_FMT(c, 4) * nt + t]);
+        amax = absmax(amax, table[QA_STAT_FMT(c, 4) * nt + t]);
     }
     sx = block_sum(sx, sm); sx2 = block_sum(sx2, sm);
     sy = block_sum(sy, sm); sy2 = block_sum(sy2, sm); sxy = block_sum(sxy, sm); sab = block_sum(sab, sm);
 #pragma unroll
     for (int o = 16; o; o >>= 1)
-        amax = fmax(amax, __hiloint2double(__shfl_xor_sync(0xFFFFFFFFu, __double2hiint(amax), o),
-                                           __shfl_xor_sync(0xFFFFFFFFu, __double2loint(amax), o)));
+        amax = absmax(amax, __hiloint2double(__shfl_xor_sync(0xFFFFFFFFu, __double2hiint(amax), o),
+                                             __shfl_xor_sync(0xFFFFFFFFu, __double2loint(amax), o)));
     __syncthreads();
     if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = amax;
     __syncthreads();
     amax = 0.0;
-    for (int i = 0; i < RB / 32; ++i) amax = fmax(amax, sm[i]);
+    for (int i = 0; i < RB / 32; ++i) amax = absmax(amax, sm[i]);
 #pragma unroll
     for (int f = 0; f < QA_NFMT; ++f) {
         const unsigned int c = __reduce_add_sync(0xFFFFFFFFu, cnt[f]);
@@ -330,7 +338,10 @@ __global__ void __launch_bounds__(RB) random_samples_kernel(const double* __rest
     }
     if (threadIdx.x == 0) {
         double pcc;
-        const double am2 = fmax(sx2 - sx * sx / numel, 0.0), bm2 = fmax(sy2 - sy * sy / numel, 0.0);
+        // max(v, 0.0) as Python evaluates it: a nan stays nan (fmax would give 0.0, hence a finite pcc)
+        double am2 = sx2 - sx * sx / numel, bm2 = sy2 - sy * sy / numel;
+        if (am2 < 0.0) am2 = 0.0;
+        if (bm2 < 0.0) bm2 = 0.0;
         const double den = sqrt(am2 * bm2);
         if (den == 0.0) pcc = amax == 0.0 ? 1.0 : 0.0;
         else pcc = (sxy - sx * sy / numel) / den;
@@ -375,7 +386,7 @@ __global__ void __launch_bounds__(SB) assignment_sums_kernel(const double* __res
             v[3] += table[QA_STAT_FMT(c, 1) * nt + t];
             v[4] += table[QA_STAT_FMT(c, 2) * nt + t];
             v[5] += table[QA_STAT_FMT(c, 3) * nt + t];
-            v[6] = fmax(v[6], table[QA_STAT_FMT(c, 4) * nt + t]);
+            v[6] = absmax(v[6], table[QA_STAT_FMT(c, 4) * nt + t]);
         } else {  // "none": y == x
             v[2] += table[QA_STAT_SX * nt + t];
             v[3] += table[QA_STAT_SX2 * nt + t];
@@ -388,14 +399,14 @@ __global__ void __launch_bounds__(SB) assignment_sums_kernel(const double* __res
         for (int o = 16; o; o >>= 1) {
             const double other = __hiloint2double(__shfl_xor_sync(0xFFFFFFFFu, __double2hiint(v[i]), o),
                                                   __shfl_xor_sync(0xFFFFFFFFu, __double2loint(v[i]), o));
-            v[i] = i == 6 ? fmax(v[i], other) : v[i] + other;
+            v[i] = i == 6 ? absmax(v[i], other) : v[i] + other;
         }
         if ((threadIdx.x & 31) == 0) sm[i][threadIdx.x >> 5] = v[i];
     }
     __syncthreads();
     if (threadIdx.x < 7) {
         double r = 0.0;
-        for (int w = 0; w < SB / 32; ++w) r = threadIdx.x == 6 ? fmax(r, sm[threadIdx.x][w]) : r + sm[threadIdx.x][w];
+        for (int w = 0; w < SB / 32; ++w) r = threadIdx.x == 6 ? absmax(r, sm[threadIdx.x][w]) : r + sm[threadIdx.x][w];
         out[threadIdx.x] = r;
     }
     if (threadIdx.x == 7) out[7] = 0.0;
@@ -411,26 +422,28 @@ __global__ void __launch_bounds__(PS_THREADS) pair_sums_kernel(const float* __re
     double v[7] = {0, 0, 0, 0, 0, 0, 0};
     const int64_t per = cdiv(n, (int64_t)gridDim.x * blockDim.x);
     const int64_t i0 = min(n, ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * per), i1 = min(n, i0 + per);
+    uint32_t mxb = 0u;                           // max |a - b| on float32 bit patterns (see absmax)
     for (int64_t i = i0; i < i1; ++i) {         // fixed element ranges and a fixed tree: deterministic
         const double x = (double)a[i], y = b ? (double)b[i] : 0.0;
-        const double d = fabs((double)__fsub_rn(a[i], b ? b[i] : 0.f));     // float32 difference, as the reference forms it
-        v[0] += x; v[1] = fma(x, x, v[1]); v[2] += y; v[3] = fma(y, y, v[3]); v[4] = fma(x, y, v[4]); v[5] += d;
-        v[6] = fmax(v[6], d);
+        const float df = fabsf(__fsub_rn(a[i], b ? b[i] : 0.f));     // float32 difference, as the reference forms it
+        v[0] += x; v[1] = fma(x, x, v[1]); v[2] += y; v[3] = fma(y, y, v[3]); v[4] = fma(x, y, v[4]); v[5] += (double)df;
+        mxb = max(mxb, __float_as_uint(df));
     }
+    v[6] = (double)__uint_as_float(mxb);
 #pragma unroll
     for (int k = 0; k < 7; ++k) {
 #pragma unroll
         for (int o = 16; o; o >>= 1) {
             const double other = __hiloint2double(__shfl_xor_sync(0xFFFFFFFFu, __double2hiint(v[k]), o),
                                                   __shfl_xor_sync(0xFFFFFFFFu, __double2loint(v[k]), o));
-            v[k] = k == 6 ? fmax(v[k], other) : v[k] + other;
+            v[k] = k == 6 ? absmax(v[k], other) : v[k] + other;
         }
         if ((threadIdx.x & 31) == 0) sm[k][threadIdx.x >> 5] = v[k];
     }
     __syncthreads();
     if (threadIdx.x < 7) {
         double r = 0.0;
-        for (int w = 0; w < PS_THREADS / 32; ++w) r = threadIdx.x == 6 ? fmax(r, sm[threadIdx.x][w]) : r + sm[threadIdx.x][w];
+        for (int w = 0; w < PS_THREADS / 32; ++w) r = threadIdx.x == 6 ? absmax(r, sm[threadIdx.x][w]) : r + sm[threadIdx.x][w];
         partial[(int64_t)blockIdx.x * 8 + threadIdx.x] = r;
     }
 }
@@ -439,7 +452,7 @@ __global__ void pair_sums_final_kernel(const double* __restrict__ partial, int n
     if (k >= 8) return;
     double r = 0.0;
     if (k < 7)
-        for (int b = 0; b < nblocks; ++b) r = k == 6 ? fmax(r, partial[(int64_t)b * 8 + k]) : r + partial[(int64_t)b * 8 + k];
+        for (int b = 0; b < nblocks; ++b) r = k == 6 ? absmax(r, partial[(int64_t)b * 8 + k]) : r + partial[(int64_t)b * 8 + k];
     out[k] = r;
 }
 

@@ -230,6 +230,9 @@ __device__ __forceinline__ bool c_any(Coop& c, bool p) {
     return __any_sync(0xFFFFFFFFu, lane < (int)c.nr ? c.sh.xi[b][lane] : 0);
 }
 
+// max that keeps a nan (np.max); fmax would drop it
+__device__ __forceinline__ double dmaxnan(double a, double b) { return (a != a || b != b) ? a + b : fmax(a, b); }
+
 // deterministic cluster-wide float64 sum / max (fixed tree: lanes, warps in order, CTAs in order)
 template <bool MAX>
 __device__ __forceinline__ double c_reduce_d(Coop& c, double v) {
@@ -237,14 +240,14 @@ __device__ __forceinline__ double c_reduce_d(Coop& c, double v) {
     for (int o = 16; o; o >>= 1) {
         const double y = __hiloint2double(__shfl_xor_sync(0xFFFFFFFFu, __double2hiint(v), o),
                                           __shfl_xor_sync(0xFFFFFFFFu, __double2loint(v), o));
-        v = MAX ? fmax(v, y) : v + y;
+        v = MAX ? dmaxnan(v, y) : v + y;
     }
     if ((threadIdx.x & 31) == 0) c.sh.i64[threadIdx.x >> 5] = __double_as_longlong(v);
     __syncthreads();
     double r = __longlong_as_double(c.sh.i64[0]);
     for (int i = 1; i < NW; ++i) {
         const double y = __longlong_as_double(c.sh.i64[i]);
-        r = MAX ? fmax(r, y) : r + y;
+        r = MAX ? dmaxnan(r, y) : r + y;
     }
     __syncthreads();
     if (c.nr == 1) return r;
@@ -252,7 +255,7 @@ __device__ __forceinline__ double c_reduce_d(Coop& c, double v) {
     if (threadIdx.x < c.nr) *c.cl.map_shared_rank(&c.sh.xd[b][c.rank], threadIdx.x) = r;
     c.xarrive_wait();
     double t = c.sh.xd[b][0];
-    for (unsigned q = 1; q < c.nr; ++q) t = MAX ? fmax(t, c.sh.xd[b][q]) : t + c.sh.xd[b][q];
+    for (unsigned q = 1; q < c.nr; ++q) t = MAX ? dmaxnan(t, c.sh.xd[b][q]) : t + c.sh.xd[b][q];
     return t;
 }
 
@@ -1683,7 +1686,7 @@ __device__ __forceinline__ void greedy_chain(const double* __restrict__ table, i
     // max |x - y| of the final assignment (for the reported atol)
     c.sync();
     double amax = 0.0;
-    for (int t = c.gtid; t < nt; t += c.gth) amax = fmax(amax, table[(size_t)QA_STAT_FMT(assignment[t], 4) * nt + t]);
+    for (int t = c.gtid; t < nt; t += c.gth) amax = dmaxnan(amax, table[(size_t)QA_STAT_FMT(assignment[t], 4) * nt + t]);
     amax = c_reduce_d<true>(c, amax);
     __syncthreads();
     if (tid < QA_NFMT && sh.cnt[tid] != 0)

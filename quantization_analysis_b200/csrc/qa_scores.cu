@@ -69,6 +69,7 @@ __global__ void __launch_bounds__(SC_WARPS * 32) tile_scores_kernel(
     const int64_t row0 = tr * TILE, colb = tc * TILE;
     const int r_end = (int)min((int64_t)TILE, rows - row0);
     const int c_end = (int)min((int64_t)TILE, cols - colb);
+    uint32_t nonfinite = 0u;    // an element with exponent field 255 (inf / nan)
     for (int r = 0; r < TILE; ++r) {
         float v = 0.f;
         if (r < r_end && lane < c_end) {
@@ -77,6 +78,7 @@ __global__ void __launch_bounds__(SC_WARPS * 32) tile_scores_kernel(
             else
                 v = reinterpret_cast<const float*>(x)[(row0 + r) * ld + colb + lane];
         }
+        if (DT == QA_DT_BF16) nonfinite |= (~__float_as_uint(v) & 0x7F800000u) == 0u;
         xs[r * SCP + lane] = v;
     }
     __syncwarp();
@@ -98,12 +100,16 @@ __global__ void __launch_bounds__(SC_WARPS * 32) tile_scores_kernel(
         if (!((fmt_mask >> f) & 1u)) continue;
         if (DT == QA_DT_BF16 && f == 0) {
             // bf16 of a bf16-exact tile is the tile itself: b == a, so every intermediate of pearson_corr repeats a's
-            // (dot(a-m, b-m) = ||a-m||^2, nb = na) and mae = atol = 0; metrics.py:14-15 for a zero denominator
+            // (dot(a-m, b-m) = ||a-m||^2, nb = na) and |a - b| is 0, except at an inf or nan element, where it is nan
+            // (inf - inf): then mae and atol are nan (np.max propagates it), else 0.  A tile of finite values near FLT_MAX
+            // overflows mean_a and daa but still has mae = atol = 0, so the elements decide.  metrics.py:14-15 for a zero
+            // denominator
             const float denom = __fmul_rn(na, na);
+            const float d = __any_sync(0xFFFFFFFFu, nonfinite) ? __uint_as_float(0x7FFFFFFFu) : 0.f;
             if (lane == 0) {
                 scores[(QA_METRIC_PCC * QA_NFMT + f) * ntiles + t] = denom == 0.f ? 1.f : __fdiv_rn(daa, denom);
-                scores[(QA_METRIC_MAE * QA_NFMT + f) * ntiles + t] = 0.f;
-                scores[(QA_METRIC_ATOL * QA_NFMT + f) * ntiles + t] = 0.f;
+                scores[(QA_METRIC_MAE * QA_NFMT + f) * ntiles + t] = d;
+                scores[(QA_METRIC_ATOL * QA_NFMT + f) * ntiles + t] = d;
             }
             continue;
         }

@@ -38,6 +38,14 @@ __device__ __forceinline__ void acc_zero(TileAcc& a) {
     for (int f = 0; f < 3; ++f) { a.sy[f] = a.sy2[f] = a.sxy[f] = a.sab[f] = 0.0; a.amax[f] = 0.f; }
 }
 
+// max(m, v) that keeps a nan (one FMNMX, like fmaxf): np.max propagates the nan of |inf - inf|, which fmaxf would drop.
+// The strict kernel takes its max |x - y| with it.
+__device__ __forceinline__ float maxnan(float m, float v) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(m), "f"(v));
+    return r;
+}
+
 // Generic (any exponent, inf/nan, tiny E) fallback: integer quantizer + direct f64 accumulation.
 __device__ __noinline__ void group_slow(const uint32_t (&w)[8], uint32_t E, TileAcc& a) {
 #pragma unroll 1
@@ -55,7 +63,7 @@ __device__ __noinline__ void group_slow(const uint32_t (&w)[8], uint32_t E, Tile
             a.sy2[f] += (double)__fmul_rn(y, y);
             a.sxy[f] += (double)__fmul_rn(x, y) - (double)__fmul_rn(y, y);   // sxy holds sum (x-y)*y until the tile end
             a.sab[f] += (double)r;
-            a.amax[f] = fmaxf(a.amax[f], r);
+            a.amax[f] = fmaxf(a.amax[f], r);      // drops a nan r; the tile end restores it from sum |x-y|
         }
     }
     // 191 <= E < 255: the group's largest |x| is at least 2^64 and its reconstruction in every format has the same sign and
@@ -64,6 +72,15 @@ __device__ __noinline__ void group_slow(const uint32_t (&w)[8], uint32_t E, Tile
     if (E - 191u < 64u) {
 #pragma unroll
         for (int f = 0; f < 3; ++f) a.sxy[f] = __longlong_as_double(0x7FF0000000000000LL);
+    }
+    // E == 255 (the caller hands each group fresh accumulators): an inf x has y = inf of its sign, so x*y = +inf and the
+    // difference above is inf - inf.  The reference's sum x*y is nan when some x*y is - a nan x (then sum x^2 is nan) or a
+    // nan y (then sum y^2 is nan) - and +inf otherwise; no x*y is -inf, as y has the sign of x.
+    if (E == 255u) {
+#pragma unroll
+        for (int f = 0; f < 3; ++f)
+            a.sxy[f] = (a.sx2 != a.sx2 || a.sy2[f] != a.sy2[f]) ? __longlong_as_double(0x7FF8000000000000LL)
+                                                                 : __longlong_as_double(0x7FF0000000000000LL);
     }
 }
 
@@ -289,11 +306,14 @@ __device__ __forceinline__ void stats_fast_item(double (&part)[FAST_WARPS - 1][1
         table[QA_STAT_SX * ntiles + t] = a.sx;
         table[QA_STAT_SX2 * ntiles + t] = a.sx2;
         if (fmt_mask & 1u) {  // bf16-exact input: y == x
+            // |x - y| is 0, or nan (inf - inf) at an inf / nan element; the float64 sum x of finite bf16 values cannot
+            // overflow, so it is finite exactly when the tile has no such element
+            const double d = isfinite(a.sx) ? 0.0 : __longlong_as_double(0x7FF8000000000000LL);
             table[QA_STAT_FMT(0, 0) * ntiles + t] = a.sx;
             table[QA_STAT_FMT(0, 1) * ntiles + t] = a.sx2;
             table[QA_STAT_FMT(0, 2) * ntiles + t] = a.sx2;
-            table[QA_STAT_FMT(0, 3) * ntiles + t] = 0.0;
-            table[QA_STAT_FMT(0, 4) * ntiles + t] = 0.0;
+            table[QA_STAT_FMT(0, 3) * ntiles + t] = d;
+            table[QA_STAT_FMT(0, 4) * ntiles + t] = d;
         }
 #pragma unroll
         for (int f = 0; f < 3; ++f) {
@@ -302,7 +322,9 @@ __device__ __forceinline__ void stats_fast_item(double (&part)[FAST_WARPS - 1][1
                 table[QA_STAT_FMT(f + 1, 1) * ntiles + t] = a.sy2[f];
                 table[QA_STAT_FMT(f + 1, 2) * ntiles + t] = a.sxy[f];
                 table[QA_STAT_FMT(f + 1, 3) * ntiles + t] = a.sab[f];
-                table[QA_STAT_FMT(f + 1, 4) * ntiles + t] = (double)a.amax[f];
+                // the fmaxf maxima above drop a nan |x - y| (np.max keeps it); sum |x - y| is a sum of terms >= 0, so it is
+                // nan exactly when one of them is, and that restores it without a nan-aware max on the per-group path
+                table[QA_STAT_FMT(f + 1, 4) * ntiles + t] = a.sab[f] != a.sab[f] ? a.sab[f] : (double)a.amax[f];
             }
         }
     }
@@ -498,11 +520,11 @@ __global__ void __launch_bounds__(STRICT_WARPS * 32) stats_strict_kernel(
             const View v = views[vi];
             for (int i = lane; i < v.nr * v.nc; i += 32) {
                 const int r = v.r0 + i / v.nc, c = i % v.nc;
-                mx = fmaxf(mx, fabsf(__fsub_rn(xs[r * SP + c], ys[r * SP + c])));
+                mx = maxnan(mx, fabsf(__fsub_rn(xs[r * SP + c], ys[r * SP + c])));
             }
         }
 #pragma unroll
-        for (int o = 16; o; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, o));
+        for (int o = 16; o; o >>= 1) mx = maxnan(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, o));
         if (lane == 0) {
             table[QA_STAT_FMT(f, 0) * ntiles + t] = res[0];
             table[QA_STAT_FMT(f, 1) * ntiles + t] = res[1];

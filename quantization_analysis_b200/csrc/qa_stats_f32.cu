@@ -375,7 +375,9 @@ __global__ void __launch_bounds__(F32_WARPS * 32, 3) stats_f32_kernel(const void
                 table[QA_STAT_FMT(f, 1) * ntiles + t] = a.sy2[f];
                 table[QA_STAT_FMT(f, 2) * ntiles + t] = a.sxy[f];
                 table[QA_STAT_FMT(f, 3) * ntiles + t] = a.sab[f];
-                table[QA_STAT_FMT(f, 4) * ntiles + t] = (double)a.amax[f];
+                // the fast path's fmaxf maxima drop a nan that an earlier group of the lane left in amax; sum |x - y| is a
+                // sum of terms >= 0, nan exactly when one of them is, so it restores np.max's nan
+                table[QA_STAT_FMT(f, 4) * ntiles + t] = a.sab[f] != a.sab[f] ? a.sab[f] : (double)a.amax[f];
             }
         }
     }
